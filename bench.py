@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (sm_100a kernels through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...  # reference arm: CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed tick's results to DIR/*.npy
 
 One "step" = one lock-step tick of every instance in the batch: EKF tick (+VO correct/replay when a VO
 message is due) + MHE update(T) (kinematics, stage assembly, VO bound insertion, marginalisation, full
@@ -163,6 +164,27 @@ class ClockSampler(threading.Thread):
             s = sorted(self.samples)
             med = s[len(s) // 2]
         return {"sm_mhz": med, "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons), "samples": len(self.samples)}
+
+
+DUMP_BYTES = 60 * 10**6  # array bytes --dump-outputs writes at most, summed over ranks (with the .npy headers: under 64 MB)
+
+
+def dump_outputs(path, outs, lo, rank, world, seed=20240510):
+    """Writes what the timed dekf_run call handed its caller for the last timed tick (quat, x, v_body, contact, status) as
+    <path>/<name>.npy in float64, instances along the last axis, and the global index of every written instance as
+    instance.npy.  Above DUMP_BYTES a fixed, seeded sample of the instances is written, the same in every run."""
+    import numpy as np
+    arrs = {k: v.numpy().astype(np.float64) for k, v in outs.items()}
+    n = arrs["x"].shape[-1]
+    per_instance = 8 * (1 + sum(a.size // n for a in arrs.values()))
+    keep = min(n, DUMP_BYTES // world // per_instance)
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(seed + rank).choice(n, keep, replace=False))
+    arrs = {k: a[..., idx] for k, a in arrs.items()}
+    arrs["instance"] = (lo + idx).astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for k, a in arrs.items():
+        np.save(os.path.join(path, f"{k}{suffix}.npy"), a)
 
 
 def measured_peaks():
@@ -427,6 +449,9 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the compact objects of BASELINE configs 3/4/5 and the ragged-VO stream")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--ref-instances-per-thread", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the last timed tick to DIR/<name>.npy (float64; the inputs "
+                         "are seeded, so two builds run with the same arguments can be compared output for output)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -488,10 +513,10 @@ def main():
                 "v_body": torch.empty(kk, 3, nn, dtype=torch.float64, device=dev), "contact": torch.empty(kk, nl, nn, dtype=torch.uint8, device=dev),
                 "status": torch.empty(kk, nn, dtype=torch.int32, device=dev)}
 
-    def device_pass(rb, nn, NN, precision, over, st, vo, SS, t0, kk, profile_ticks=0, keep=False):
+    def device_pass(rb, nn, NN, precision, over, st, vo, SS, t0, kk, profile_ticks=0, keep=False, last=False):
         """kk ticks in one dekf_run call, inputs resident in HBM, every tick's results written to per-tick arrays, CUDA events
         on the launching stream, max over ranks; optionally a tick-by-tick pass of a fresh handle with an event pair around
-        every launch (per-kernel device time)."""
+        every launch (per-kernel device time).  last=True: res["last"] holds the results of the last tick on the host."""
         prm = estimator.robot_params(rb, ekf_rate=200, N=NN, **over)
         est = estimator.BatchedEstimator(prm, nn, device=local_rank, precision=precision)
         est.run(0, t0, sub(st, 0, t0, SS), vo[:t0])
@@ -516,6 +541,8 @@ def main():
             it, na = est.qp_info()
             res["factorisations_mean"] = float(it.double().mean())
             res["active_bounds_mean"] = float(na.double().mean())
+        if last:
+            res["last"] = {k: v[-1].cpu() for k, v in outs.items()}
         del outs
         if profile_ticks:
             Kp = min(kk, profile_ticks)
@@ -563,7 +590,10 @@ def main():
             o["window_solve"] = 1 if md == "incremental" else 0
         return o
 
-    est, main = device_pass(robot, n, N, args.precision, over_for(mode), stream, vo_steps, S, T0, K, profile_ticks=60 if plain else 0, keep=True)
+    est, main = device_pass(robot, n, N, args.precision, over_for(mode), stream, vo_steps, S, T0, K, profile_ticks=60 if plain else 0, keep=True,
+                            last=bool(args.dump_outputs))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, main.pop("last"), lo, rank, world)
     other = None
     if plain:
         _, other = device_pass(robot, n, N, args.precision, over_for(other_mode), stream, vo_steps, S, T0, K, profile_ticks=60)
