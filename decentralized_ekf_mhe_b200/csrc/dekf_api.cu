@@ -544,6 +544,17 @@ __global__ void k_vo_count(const Dims dm, const Buffers<T> b, int Tk, int32_t *c
   count[i] = c;
 }
 
+// smoothed window of the last update(Tk) (dekf_get_window): one thread per instance, SoA loads coalesced over instances.
+// FULL: the forward sweep from the arrival cost into the scratch ring scr [N][54][ns] runs first; otherwise the checkpoint ring
+// of the incremental solve is read (one instantiation per mode: neither carries the other's registers).
+template <typename T, bool FULL>
+__global__ void __launch_bounds__(kBlock) k_window(const MheConst<T> c, const MheConst<double> c64, const Dims dm, const Buffers<T> b,
+                                                   T *scr, int Tk, double *xout) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= dm.n) return;
+  mhe_window_smooth<T>(c, c64, dm, b, FULL ? scr : nullptr, Tk, i, xout, (size_t)dm.n);
+}
+
 }  // namespace dekf
 
 // ------------------------------------------------------------------------------------------------
@@ -594,6 +605,7 @@ struct dekf_handle {
   FootConst fc;
   FootBuffers fb = {nullptr, nullptr, nullptr};  // leg_odom_type 1
   void *ckpt_mem = nullptr;       // incremental window solve: checkpoint ring
+  void *win_scr = nullptr;        // dekf_get_window on a full re-sweep handle: filtered states [N][54][ns] (first use)
   int32_t *resweep_mem = nullptr;
   void *slab = nullptr;
   size_t slab_bytes = 0;
@@ -1168,6 +1180,7 @@ int dekf_destroy(dekf_handle *h) {
   cudaFree(h->fb.arr_M);
   cudaFree(h->fb.arr_m);
   cudaFree(h->ckpt_mem);
+  cudaFree(h->win_scr);
   cudaFree(h->resweep_mem);
   cudaFree(h->bb.fac);
   cudaFree(h->tb.prior);
@@ -2259,15 +2272,52 @@ int dekf_get_resweep_info(dekf_handle *h, int32_t *depth, int32_t *n_vo) {
   return DEKF_OK;
 }
 
+int dekf_get_window(dekf_handle *h, double *x, int32_t *len) {
+  if (!h) return DEKF_EINVAL;
+  if (!x) return fail(h, DEKF_EINVAL, "dekf_get_window: null x");
+  if (h->cfg.est_type != 0) return fail(h, DEKF_EINVAL, "dekf_get_window: est_type 1 (KF) has no window");
+  if (h->cfg.leg_odom_type != 0) return fail(h, DEKF_EINVAL, "dekf_get_window: leg_odom_type 1 (foot states) is not supported");
+  if (h->row_V != nullptr) return fail(h, DEKF_EINVAL, "dekf_get_window: not available after dekf_add_state_rows (constrained window)");
+  if (h->cfg.v_box_enable || h->cfg.x_box_mask || h->bc.enable)
+    return fail(h, DEKF_EINVAL, "dekf_get_window: not available with state bounds (v_box_enable / x_box_mask)");
+  if (h->next_T < 2) return fail(h, DEKF_ESTATE, "dekf_get_window: needs a completed update(T >= 1)");
+  CK(cudaSetDevice(h->cfg.device));
+  const int Tk = h->next_T - 1, N = h->dm.N;
+  void *scr = nullptr;
+  if (h->mc64.window_solve == 0) {
+    if (!h->win_scr) {
+      const size_t bytes = (size_t)N * 54 * h->dm.ns * (h->f32 ? sizeof(float) : sizeof(double));
+      CK(cudaMalloc(&h->win_scr, bytes));
+      h->extra_bytes += bytes;
+    }
+    scr = h->win_scr;
+  }
+  // dekf_run joins its internal streams into h->stream before returning, so this launch is ordered after every tick
+  const dim3 grid(grid_for(h->dm.n));
+  if (h->f32 && scr)
+    k_window<float, true><<<grid, kBlock, 0, h->stream>>>(h->mc32, h->mc64, h->dm, h->b32, (float *)scr, Tk, x);
+  else if (h->f32)
+    k_window<float, false><<<grid, kBlock, 0, h->stream>>>(h->mc32, h->mc64, h->dm, h->b32, nullptr, Tk, x);
+  else if (scr)
+    k_window<double, true><<<grid, kBlock, 0, h->stream>>>(h->mc64, h->mc64, h->dm, h->b64, (double *)scr, Tk, x);
+  else
+    k_window<double, false><<<grid, kBlock, 0, h->stream>>>(h->mc64, h->mc64, h->dm, h->b64, nullptr, Tk, x);
+  h->launches++;
+  CK(cudaGetLastError());
+  if (len) *len = Tk + 1 < N ? Tk + 1 : N;
+  return DEKF_OK;
+}
+
 int dekf_get_host(dekf_handle *h, int32_t what, void *host_out) {
   if (!h || !host_out) return fail(h, DEKF_EINVAL, "dekf_get_host: null argument");
   CK(cudaSetDevice(h->cfg.device));
   const size_t n = (size_t)h->dm.n;
   const size_t dsz = (size_t)h->ds;
-  const size_t rows[8] = {9, 3, dsz * dsz, dsz, 16, 1, dsz * dsz, dsz};
-  if (what < 0 || what > DEKF_GET_KF_GAIN) return fail(h, DEKF_EINVAL, "dekf_get_host: unknown selector");
+  const size_t rows[10] = {9, 3, dsz * dsz, dsz, 16, 1, dsz * dsz, dsz, 0, 9 * (size_t)h->dm.N};
+  if (what < 0 || what > DEKF_GET_WINDOW_X) return fail(h, DEKF_EINVAL, "dekf_get_host: unknown selector");
   // one scratch for the life of the handle (the 200 Hz node shells call this every tick)
-  const size_t need = (dsz * dsz + dsz + 6 * (size_t)h->nl) * n * sizeof(double);
+  size_t need = (dsz * dsz + dsz + 6 * (size_t)h->nl) * n * sizeof(double);
+  if (what == DEKF_GET_WINDOW_X && need < rows[DEKF_GET_WINDOW_X] * n * sizeof(double)) need = rows[DEKF_GET_WINDOW_X] * n * sizeof(double);
   if (h->get_scratch_bytes < need) {
     cudaFree(h->get_scratch);
     h->get_scratch = nullptr;
@@ -2318,6 +2368,12 @@ int dekf_get_host(dekf_handle *h, int32_t what, void *host_out) {
       rc = dekf_get_arrival_cov(h, d, d + dsz * dsz * n);
       src = d + dsz * dsz * n;
       break;
+    case DEKF_GET_WINDOW_X: {
+      int32_t K = 0;
+      rc = dekf_get_window(h, d, &K);
+      bytes = (size_t)K * 9 * n * sizeof(double);
+      break;
+    }
     default:
       rc = dekf_get_window_vo_count(h, (int32_t *)d);
       bytes = n * sizeof(int32_t);

@@ -2223,4 +2223,313 @@ DEKF_HD int kf_update(const MheConst<T> &c, const Dims &dm, const Buffers<T> &b,
   return status;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Smoothed window (dekf_get_window): every state block of MHEproblem::solution (MheSrb.hpp:58-112), not only x_T.
+// The window QP of update(T) holds K = min(T+1, N) states, stages T-K+1 .. T, with the arrival cost on the first.  Its
+// optimum is the Rauch-Tung-Striebel smoother of the forward sweep: x_T^s = m_T and, for k = T-1 down to T-K+1,
+//   x_k^s = m'_k + C' Sigma^-1 (x_{k+1}^s - mu)
+// where (m_k, P_k) is the filtered state of stage k (after its leg-odometry rows), mu / Sigma the prediction of x_{k+1}
+// (dynamics, then the VO row p_{k+1} - p_k = Delta_k if it is an equality: exactly the forward sweep's time update) and
+// m'_k, C' = Cov(x_k, x_{k+1}) are conditioned on that VO row.  Exact, because the leg rows of stage k+1 and everything after
+// them see x_k only through x_{k+1}.  With A the transition, L = [0, dt I, -h R] (p_{k+1} - p_k = L x_k + h a_s + w_p),
+// U = Cov(x_{k+1}, d) = A P L' + [C1; C2; 0], S = L P L' + C1 + R C_vo R' and nu = Delta - (L m + h a_s):
+//   m'_k + C' z = m_k + P_k g,   g = A' z + L' S^-1 (nu - U' z),   U' z = L P A' z + C1 z_p + C2 z_v,   z = Sigma^-1 (x^s - mu)
+// (no VO row: g = A' z).  Only Sigma is factorised (9x9 Cholesky); C' is never formed.  The arithmetic is D (double) for
+// both handle precisions; every multiply-add is an explicit fm so that the host build performs the same operations.
+// ------------------------------------------------------------------------------------------------
+template <typename D, typename T>
+DEKF_HD void load_state_as(const T *base, size_t ns, Cov9<D> &P, Vec9<D> &x) {
+#pragma unroll
+  for (int f = 0; f < 6; ++f) {
+    P.pp.a[f] = (D)base[f * ns];
+    P.vv.a[f] = (D)base[(6 + f) * ns];
+    P.bb.a[f] = (D)base[(12 + f) * ns];
+  }
+#pragma unroll
+  for (int f = 0; f < 9; ++f) {
+    P.pv.a[f] = (D)base[(18 + f) * ns];
+    P.pb.a[f] = (D)base[(27 + f) * ns];
+    P.vb.a[f] = (D)base[(36 + f) * ns];
+  }
+#pragma unroll
+  for (int f = 0; f < 3; ++f) {
+    x.p[f] = (D)base[(45 + f) * ns];
+    x.v[f] = (D)base[(48 + f) * ns];
+    x.b[f] = (D)base[(51 + f) * ns];
+  }
+}
+
+// entry (r, c) of the dense 9x9 matrix held by a Cov9 (indices are compile-time constants after unrolling)
+template <typename D>
+DEKF_HD D cov_at(const Cov9<D> &P, int r, int c) {
+  if (r > c) {
+    const int t = r;
+    r = c;
+    c = t;
+  }
+  const int br = r / 3, bc = c / 3, rr = r % 3, cc = c % 3;
+  if (br == bc) return br == 0 ? P.pp(rr, cc) : (br == 1 ? P.vv(rr, cc) : P.bb(rr, cc));
+  if (br == 0) return bc == 1 ? P.pv(rr, cc) : P.pb(rr, cc);
+  return P.vb(rr, cc);
+}
+
+// y += P a (P symmetric 9x9 in blocks)
+template <typename D>
+DEKF_HD void cov_mul_add(const Cov9<D> &P, const V3<D> &ap, const V3<D> &av, const V3<D> &ab, Vec9<D> &y) {
+#pragma unroll
+  for (int r = 0; r < 3; ++r) {
+    D sp = y.p[r], sv = y.v[r], sb = y.b[r];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      sp = fm(P.pp(r, k), ap[k], sp);
+      sp = fm(P.pv(r, k), av[k], sp);
+      sp = fm(P.pb(r, k), ab[k], sp);
+      sv = fm(P.pv(k, r), ap[k], sv);
+      sv = fm(P.vv(r, k), av[k], sv);
+      sv = fm(P.vb(r, k), ab[k], sv);
+      sb = fm(P.pb(k, r), ap[k], sb);
+      sb = fm(P.vb(k, r), av[k], sb);
+      sb = fm(P.bb(r, k), ab[k], sb);
+    }
+    y.p[r] = sp;
+    y.v[r] = sv;
+    y.b[r] = sb;
+  }
+}
+
+template <typename D, typename T>
+DEKF_HD void load_rec_dyn(const T *rec, size_t ns, M3<D> &R, V3<D> &as, V3<D> &dlt) {
+#pragma unroll
+  for (int f = 0; f < 9; ++f) R.a[f] = (D)rec[(REC_R + f) * ns];
+#pragma unroll
+  for (int f = 0; f < 3; ++f) {
+    as[f] = (D)rec[(REC_AS + f) * ns];
+    dlt[f] = (D)rec[(REC_DLT + f) * ns];
+  }
+}
+
+// One backward stage: reads x_{k+1}^s at xnext, writes x_k^s at xout (both [9] at stride n_out).  `ck` = filtered state of
+// stage k ([54] at stride ns: P 45 incl. P_pp, x 9), `rec` = stage record k (stride ns); both already offset to the instance.
+// Register budget: only z crosses from the factorisation phase to the product phase; P_k, the record and x_{k+1}^s are
+// re-read where they are needed instead of being kept live.
+template <typename D, typename T>
+DEKF_HD void window_back_stage(const MheConst<D> &c, const T *ck, const T *rec, size_t ns, const double *xnext, double *xout,
+                               size_t n_out) {
+  const bool vo = rec[REC_FLAG * ns] != T(0);
+  // z = Sigma^-1 (x^s_{k+1} - mu): (mu, Sigma) is the forward sweep's time update (+ VO row) of stage k, in D
+  D z[9];
+  {
+    Cov9<D> Sg;
+    Vec9<D> mu;
+    {
+      M3<D> R;
+      V3<D> as, dlt;
+      load_rec_dyn(rec, ns, R, as, dlt);
+      load_state_as(ck, ns, Sg, mu);
+      DefaultMath<D>::template prop<1>(c, Sg, mu, R, as, vo, dlt);
+    }
+#pragma unroll
+    for (int f = 0; f < 3; ++f) {
+      z[f] = (D)xnext[f * n_out] - mu.p[f];
+      z[3 + f] = (D)xnext[(3 + f) * n_out] - mu.v[f];
+      z[6 + f] = (D)xnext[(6 + f) * n_out] - mu.b[f];
+    }
+    D Lc[45], dinv[9];  // packed lower Cholesky factor, row r at r (r + 1) / 2; reciprocal diagonal
+#pragma unroll
+    for (int r = 0; r < 9; ++r) {
+#pragma unroll
+      for (int cc = 0; cc <= r; ++cc) {
+        D v = cov_at(Sg, r, cc);
+#pragma unroll
+        for (int k = 0; k < cc; ++k) v = fm(-Lc[r * (r + 1) / 2 + k], Lc[cc * (cc + 1) / 2 + k], v);
+        if (cc == r) {
+          const D d = sqrt(v);
+          Lc[r * (r + 1) / 2 + r] = d;
+          dinv[r] = D(1) / d;
+        } else {
+          Lc[r * (r + 1) / 2 + cc] = v * dinv[cc];
+        }
+      }
+    }
+#pragma unroll
+    for (int r = 0; r < 9; ++r) {
+      D v = z[r];
+#pragma unroll
+      for (int k = 0; k < r; ++k) v = fm(-Lc[r * (r + 1) / 2 + k], z[k], v);
+      z[r] = v * dinv[r];
+    }
+#pragma unroll
+    for (int r = 8; r >= 0; --r) {
+      D v = z[r];
+#pragma unroll
+      for (int k = r + 1; k < 9; ++k) v = fm(-Lc[k * (k + 1) / 2 + r], z[k], v);
+      z[r] = v * dinv[r];
+    }
+  }
+#if defined(__CUDA_ARCH__)
+  asm volatile("" ::: "memory");  // a real re-read: keeps the compiler from holding the first loads live across the factorisation
+#endif
+  const D dt = c.dt, h = D(0.5) * c.dt * c.dt;
+  M3<D> R;
+  V3<D> as, dlt;
+  load_rec_dyn(rec, ns, R, as, dlt);
+  Cov9<D> P;
+  Vec9<D> m;
+  load_state_as(ck, ns, P, m);
+  // a = A' z = [z_p;  dt z_p + z_v;  z_b - R' (h z_p + dt z_v)]
+  V3<D> ap, av, ab;
+  {
+    V3<D> t;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+      ap[r] = z[r];
+      av[r] = fm(dt, z[r], z[3 + r]);
+      t[r] = fm(h, z[r], dt * z[3 + r]);
+    }
+#pragma unroll
+    for (int r = 0; r < 3; ++r) ab[r] = fm(-R(2, r), t[2], fm(-R(1, r), t[1], fm(-R(0, r), t[0], z[6 + r])));
+  }
+  Vec9<D> w = m;
+  cov_mul_add(P, ap, av, ab, w);  // w = m + P A' z
+  if (vo) {
+    // rhs = nu - U' z = Delta - (L m + h a_s) - L (P A' z) - C1 z_p - C2 z_v;  L y = dt y_v - h R y_b
+    S3<D> C1, C2, Sm;
+#pragma unroll
+    for (int f = 0; f < 6; ++f) C1.a[f] = C2.a[f] = Sm.a[f] = D(0);
+    add_rot_diag(C1, R, c.n1);
+    add_rot_diag(C2, R, c.n2);
+    add_rot_diag(Sm, R, c.nvo);
+    V3<D> rhs;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+      // w - m = P A' z, so L m + L P A' z = L w
+      const D Rwb = fm(R(r, 2), w.b[2], fm(R(r, 1), w.b[1], R(r, 0) * w.b[0]));
+      D v = dlt[r] - fm(-h, Rwb, fm(h, as[r], dt * w.v[r]));
+#pragma unroll
+      for (int k = 0; k < 3; ++k) v = fm(-C2(r, k), z[3 + k], fm(-C1(r, k), z[k], v));
+      rhs[r] = v;
+    }
+    // S = L P L' + C1 + R C_vo R' = dt^2 P_vv - h dt (E + E') + h^2 R P_bb R' + C1 + R C_vo R',  E = P_vb R'
+    {
+      M3<D> E, B;
+#pragma unroll
+      for (int r = 0; r < 3; ++r)
+#pragma unroll
+        for (int cc = 0; cc < 3; ++cc) {
+          E(r, cc) = fm(P.vb(r, 2), R(cc, 2), fm(P.vb(r, 1), R(cc, 1), P.vb(r, 0) * R(cc, 0)));
+          B(r, cc) = fm(R(r, 2), P.bb(2, cc), fm(R(r, 1), P.bb(1, cc), R(r, 0) * P.bb(0, cc)));
+        }
+      const D dt2 = dt * dt, hdt = h * dt, hh = h * h;
+#pragma unroll
+      for (int r = 0; r < 3; ++r)
+#pragma unroll
+        for (int cc = r; cc < 3; ++cc) {
+          const int k = S3<D>::idx(r, cc);
+          const D BR = fm(B(r, 2), R(cc, 2), fm(B(r, 1), R(cc, 1), B(r, 0) * R(cc, 0)));
+          Sm.a[k] = fm(hh, BR, fm(-hdt, E(r, cc) + E(cc, r), fm(dt2, P.vv.a[k], Sm.a[k] + C1.a[k])));
+        }
+    }
+    // q = S^-1 rhs (3x3 Cholesky)
+    V3<D> q;
+    {
+      const D l00 = sqrt(Sm.a[0]), i0 = D(1) / l00;
+      const D l10 = Sm.a[1] * i0, l20 = Sm.a[2] * i0;
+      const D l11 = sqrt(fm(-l10, l10, Sm.a[3])), i1 = D(1) / l11;
+      const D l21 = fm(-l20, l10, Sm.a[4]) * i1;
+      const D l22 = sqrt(fm(-l21, l21, fm(-l20, l20, Sm.a[5]))), i2 = D(1) / l22;
+      const D y0 = rhs[0] * i0;
+      const D y1 = fm(-l10, y0, rhs[1]) * i1;
+      const D y2 = fm(-l21, y1, fm(-l20, y0, rhs[2])) * i2;
+      q[2] = y2 * i2;
+      q[1] = fm(-l21, q[2], y1) * i1;
+      q[0] = fm(-l20, q[2], fm(-l10, q[1], y0)) * i0;
+    }
+    // w += P L' q,  L' q = [0;  dt q;  -h R' q]
+    V3<D> e0, ev, eb;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+      e0[r] = D(0);
+      ev[r] = dt * q[r];
+      eb[r] = -h * fm(R(2, r), q[2], fm(R(1, r), q[1], R(0, r) * q[0]));
+    }
+    cov_mul_add(P, e0, ev, eb, w);
+  }
+#pragma unroll
+  for (int f = 0; f < 3; ++f) {
+    xout[f * n_out] = (double)w.p[f];
+    xout[(3 + f) * n_out] = (double)w.v[f];
+    xout[(6 + f) * n_out] = (double)w.b[f];
+  }
+}
+
+// FULL mode source of the filtered states: the forward sweep of update(T) from the arrival cost of its window (arr_P / arr_x
+// after update(T) is the prior of x_{T-N+1}; Prior_0 while T < N), with the operations of mhe_solve_incr (P_pp carried), each
+// stage's (P, x) stored into scr[k % N] ([N][54][ns]).  Bit-identical to the checkpoints of the incremental solve.
+template <typename T, typename Math = DefaultMath<T>>
+DEKF_HD void window_forward(const MheConst<T> &c, const Dims &dm, const Buffers<T> &b, int Tk, int i, T *scr) {
+  GlobalStageSource<T> src(dm, b, i);
+  Cov9<T> P;
+  Vec9<T> x;
+  mhe_solve_start(c, dm, b, Tk, i, P, x);
+  const int k0 = Tk < dm.N ? 0 : Tk - dm.N + 1;
+  const size_t ns = (size_t)dm.ns;
+  for (int k = k0;; ++k) {
+    S3<T> Lam;
+    V3<T> eta;
+    src.meas(0, k, Lam, eta);
+    Math::meas(P, x, Lam, eta);
+    T *base = scr + (size_t)(k % dm.N) * 54 * ns;
+    store_cov(base, dm.ns, i, P);
+#pragma unroll
+    for (int f = 0; f < 3; ++f) {
+      base[(45 + f) * ns + i] = x.p[f];
+      base[(48 + f) * ns + i] = x.v[f];
+      base[(51 + f) * ns + i] = x.b[f];
+    }
+    if (k == Tk) break;
+    M3<T> R;
+    V3<T> as, dlt;
+    bool vo;
+    src.rot(0, k, R);
+    src.dyn(0, k, as, dlt, vo);
+    Math::prop(c, P, x, R, as, vo, dlt);
+  }
+}
+
+// Backward pass over the filtered states of stages Tk-K+1 .. Tk held in `ring` (slot k % slots, [slots][54][ns]).
+template <typename T>
+DEKF_HD void window_backward(const MheConst<double> &c64, const Dims &dm, const Buffers<T> &b, const T *ring, int slots, int Tk,
+                             int i, double *xout, size_t n_out) {
+  const int N = dm.N, K = Tk + 1 < N ? Tk + 1 : N, k0 = Tk - K + 1;
+  const size_t ns = (size_t)dm.ns;
+  {
+    const T *top = ring + (size_t)(Tk % slots) * 54 * ns + i;  // x_T^s = m_T
+    double *o = xout + (size_t)(Tk - k0) * 9 * n_out + i;
+#pragma unroll
+    for (int f = 0; f < 9; ++f) o[f * n_out] = (double)top[(45 + f) * ns];
+  }
+  for (int k = Tk - 1; k >= k0; --k) {
+    double *o = xout + (size_t)(k - k0) * 9 * n_out + i;
+    window_back_stage<double, T>(c64, ring + (size_t)(k % slots) * 54 * ns + i, b.win + (size_t)(k % dm.NW) * REC_SIZE * ns + i, ns,
+                                 o + 9 * n_out, o, n_out);
+  }
+}
+
+// Smoothed window of update(Tk) (Tk >= 1) for instance i: xout [K][9][n_out], row j = stage Tk-K+1+j, K = min(Tk+1, N).
+// scr == nullptr: the filtered states are the checkpoint ring of the incremental solve (window_solve 1); otherwise the
+// forward sweep above writes them into scr first (window_solve 0).  c: the handle's constants, c64: the same in double.
+template <typename T>
+DEKF_HD void mhe_window_smooth(const MheConst<T> &c, const MheConst<double> &c64, const Dims &dm, const Buffers<T> &b, T *scr,
+                               int Tk, int i, double *xout, size_t n_out) {
+  if (scr == nullptr) {
+    window_backward<T>(c64, dm, b, b.ckpt, dm.NW, Tk, i, xout, n_out);
+    return;
+  }
+  window_forward<T>(c, dm, b, Tk, i, scr);
+#if defined(__CUDA_ARCH__)
+  asm volatile("" ::: "memory");  // the backward pass reads the ring back; nothing of the forward sweep stays live
+#endif
+  window_backward<T>(c64, dm, b, scr, dm.N, Tk, i, xout, n_out);
+}
+
 }  // namespace dekf

@@ -7,6 +7,7 @@ Reference (C++; /root/reference/src)                          here (Python over 
      public x_MHE_, v_MHE_b_, R_sb_, p_vo_accmulate_ :278-285     same attribute names (torch tensors [k, n])
   orien_ekf::timerCallback  orien_ekf.cpp:77-89                orien_ekf.timerCallback
   MHEproblem::M_p, n_p  MheSrb.hpp:86-87                       DecentralizedEstimation.mhe_qp_.M_p / .n_p
+  MHEproblem::solution  MheSrb.hpp:58-112 (state blocks)       DecentralizedEstimation.mhe_qp_.x_window(), BatchedEstimator.window()
 
 torch is used for device memory and streams only; all arithmetic happens in libdekf_b200.so
 (sm_100a kernels).  Nothing here falls back to PyTorch or the CPU: a missing library or device raises.
@@ -164,8 +165,17 @@ class _Handle:
             chk(quat, 4, "quaternion_") if quat is not None else None)
 
 
+def _window(h):
+    """Smoothed window of the last update(T): [K][9][n] float64 on the device (dekf_get_window)."""
+    w = torch.empty(int(h.cfg.N), 9, h.n, dtype=torch.float64, device=h.device)
+    K = C.c_int32()
+    h.check(h.L.dekf_get_window(h.h, _ptr(w), C.byref(K)), "dekf_get_window")
+    return w[:K.value]
+
+
 class _MheQpView:
-    """The two public members of ``MHEproblem`` callers read (MheSrb.hpp:86-87)."""
+    """The public members of ``MHEproblem`` callers read: M_p, n_p (MheSrb.hpp:86-87) and the state blocks of
+    ``solution`` (MheSrb.hpp:58-112)."""
 
     def __init__(self, owner):
         self._o = owner
@@ -188,6 +198,11 @@ class _MheQpView:
 
     def arrival_cov(self):
         return self._get(False)
+
+    def x_window(self):
+        """The window QP's optimum for every state of the last update(T), T >= 1: [K][9][n], K = min(T+1, N), row j =
+        stage T-K+1+j (smoothed, oldest first); row K-1 equals x_MHE_ bit for bit."""
+        return _window(self._o._hd)
 
 
 class DecentralizedEstimation:
@@ -377,6 +392,11 @@ class BatchedEstimator:
         return p
 
     K_KF_ = DecentralizedEstimation.K_KF_
+
+    def window(self):
+        """Smoothed window of the last update(T), T >= 1 (the state blocks of MHEproblem::solution): [K][9][n] float64 on the
+        device, K = min(T+1, N), row j = stage T-K+1+j; row K-1 equals x_MHE_ bit for bit.  Stream-ordered."""
+        return _window(self._hd)
 
     def step(self, T, store):
         h = self._hd

@@ -25,6 +25,8 @@
  *   dekf_outputs                public result members R_sb_, x_MHE_, v_MHE_b_ (DecentralEst.hpp:279-285) and the
  *                               imu/filter quaternion (orien_ekf.cpp:92-95)
  *   dekf_get_arrival_cost       MHEproblem::M_p, n_p               MheSrb.hpp:86-87
+ *   dekf_get_window             MHEproblem::solution (state blocks)   MheSrb.hpp:58-112 (getsolution narrows it to x_T,
+ *                               MheSrb.cpp:715-723)
  *   dekf_get_p_vo               DecentralizedEstimation::p_vo_accmulate_   DecentralEst.hpp:280
  *   dekf_reset                  DecentralizedEstimation::reset()   DecentralEst.hpp:103
  *
@@ -248,6 +250,13 @@ int dekf_get_R_sb(dekf_handle *h, double *R /*[9][n]*/);
 int dekf_get_ekf_cov(dekf_handle *h, double *P /*[16][n]*/);
 /* number of window stages whose VO row is currently an equality (LinearConstraint.equality, MheSrb.hpp:38) */
 int dekf_get_window_vo_count(dekf_handle *h, int32_t *count /*[n]*/);
+/* Smoothed window of the last update(T) (T >= 1): the state blocks of MHEproblem::solution (MheSrb.hpp:58-112) -- the exact
+ * optimum of the window QP for every state, not only x_T.  x receives [K][9][n] (device pointer, stream-ordered),
+ * K = min(T+1, N), row j = stage T-K+1+j, row K-1 equal to dekf_outputs.x of that update bit for bit.  *len (host, may be
+ * NULL) receives K.  est_type 0, leg_odom_type 0, no state bounds / rows; both window_solve modes (DEKF_SOLVE_FULL runs a
+ * forward sweep from the arrival cost into a scratch ring allocated on first use, counted in dekf_device_bytes).
+ * DEKF_EINVAL for a null x or an unsupported handle, DEKF_ESTATE before the first update(T >= 1) and after dekf_reset. */
+int dekf_get_window(dekf_handle *h, double *x, int32_t *len);
 /* Host-pointer getter for callers without a CUDA runtime of their own (the C++ facade, a ROS node): `what` selects one
  * of the arrays above, `host_out` receives it (same [rows][n] layout, double; int32 for DEKF_GET_VO_COUNT).
  * Synchronises the handle's stream. */
@@ -260,8 +269,9 @@ enum {
   DEKF_GET_VO_COUNT = 5,   /* [n] int32 */
   DEKF_GET_ARRIVAL_COV = 6,  /* [81][n] arrival covariance; est_type 1: C_KF_ (DecentralEst.hpp:288) */
   DEKF_GET_ARRIVAL_MEAN = 7, /* [9][n]  arrival mean;       est_type 1: x_KF_ */
-  DEKF_GET_KF_GAIN = 8       /* [9 * 3 * num_legs][n] K_KF_ (DecentralEst.hpp:290, DecentralEst.cpp:858), row-major 9 x 3L per
+  DEKF_GET_KF_GAIN = 8,      /* [9 * 3 * num_legs][n] K_KF_ (DecentralEst.hpp:290, DecentralEst.cpp:858), row-major 9 x 3L per
                               * instance; est_type 1, leg_odom_type 0 and cfg.kf_export_gain only */
+  DEKF_GET_WINDOW_X = 9      /* [K * 9][n] smoothed window (dekf_get_window); K <= N, so room for N * 9 rows suffices */
 };
 int dekf_get_host(dekf_handle *h, int32_t what, void *host_out);
 /* debug taps of the last step (only when cfg.debug_taps != 0): copied into caller DEVICE buffers, any may be NULL.

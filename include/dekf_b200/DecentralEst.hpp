@@ -8,6 +8,7 @@
 //        initialize(std::shared_ptr<robot_store>, std::shared_ptr<robot_params>) / update(int T) / reset()
 //        public results R_sb_, p_vo_accmulate_, x_MHE_, v_MHE_b_
 //   class MHEproblem::M_p, n_p    include/decentral_legged_est/MheSrb.hpp:86-87   dekf::DecentralizedEstimation::mhe_qp_.M_p()/n_p()
+//   MHEproblem::solution (state blocks) MheSrb.hpp:58-112                          dekf::DecentralizedEstimation::mhe_qp_.x_window()
 //
 // The reference estimates ONE robot and stores Eigen vectors; this facade steps `n_instances` robots per call and stores
 // flat SoA arrays `[rows][n_instances]` (instance fastest).  With n_instances == 1 every array has exactly the layout of the
@@ -290,6 +291,8 @@ class DecentralizedEstimation {
       detail::check(dekf_add_state_rows(h_, (int32_t)rows_lb_.size(), rows_a_.data(), rows_lb_.data(), rows_ub_.data()), h_,
                     "dekf_add_state_rows");
     n_ = cfg.n_instances;
+    N_ = cfg.N;
+    last_T_ = -1;
     nl_ = cfg.num_legs;
     nq_ = dekf_num_joints(h_);
     kf_ = cfg.est_type == 1;
@@ -316,6 +319,7 @@ class DecentralizedEstimation {
   // DecentralEst.hpp:103
   void reset() {
     if (h_) detail::check(dekf_reset(h_), h_, "dekf_reset");
+    last_T_ = -1;
   }
 
   // results (DecentralEst.hpp:278-285), `[rows][n]`
@@ -345,6 +349,15 @@ class DecentralizedEstimation {
       std::vector<double> v((size_t)o->ds_ * o->n_);
       detail::check(dekf_get_host(o->h_, DEKF_GET_ARRIVAL_N, v.data()), o->h_, "dekf_get_host");
       return v;
+    }
+    // the state blocks of MHEproblem::solution (MheSrb.hpp:58-112) of the last update(T), T >= 1: the smoothed window
+    // [K][9][n], K = min(T+1, N), row j = stage T-K+1+j, row K-1 == x_MHE_ (dekf_get_window)
+    std::vector<double> x_window() const {
+      std::vector<double> w((size_t)o->N_ * 9 * o->n_);
+      detail::check(dekf_get_host(o->h_, DEKF_GET_WINDOW_X, w.data()), o->h_, "dekf_get_host");
+      const int K = o->last_T_ + 1 < o->N_ ? o->last_T_ + 1 : o->N_;
+      w.resize((size_t)K * 9 * o->n_);
+      return w;
     }
   } mhe_qp_{this};
 
@@ -377,6 +390,7 @@ class DecentralizedEstimation {
     out.contact = st.contact_.data();
     out.status = status_.data();
     detail::check(dekf_mhe_step_host(h_, T, &in, &out), h_, "dekf_mhe_step_host");
+    last_T_ = T;
     std::fill(st.vo_new_.begin(), st.vo_new_.end(), (uint8_t)0);  // robot_sub_ptr_->vo_new_ = false (DecentralEst.cpp:891)
     detail::check(dekf_get_host(h_, DEKF_GET_R_SB, R_sb_.data()), h_, "dekf_get_host");
     detail::check(dekf_get_host(h_, DEKF_GET_P_VO, p_vo_accmulate_.data()), h_, "dekf_get_host");
@@ -388,6 +402,7 @@ class DecentralizedEstimation {
   std::vector<double> rows_a_, rows_lb_, rows_ub_;  // addStateRows()
   dekf_handle *h_ = nullptr;
   int n_ = 0, nl_ = 0, nq_ = 0;
+  int N_ = 0, last_T_ = -1;  // horizon, T of the last update (window length of mhe_qp_.x_window())
   bool kf_ = false;
   int ds_ = 9;
 };

@@ -1,0 +1,131 @@
+"""Cost of the smoothed-window getter (dekf_get_window) on a large batch.
+
+Go1, N = 20, 65,536 instances, fp64 and fp32 handles, ragged and lock-step VO arrival, both window_solve modes.  Per setup:
+64 warm-up ticks (dekf_run), then the getter timed with CUDA events over --calls calls, then a tick with and without the
+getter, alternated in the same process.  Algorithmic bytes come from the shapes, flops from the operation tally of
+tests/hostsim/window_flopcount.cpp (FLOPS below; tests/test_window_smoother.py keeps them equal); the roofline denominators are
+dekf_measure_copy_bw / dekf_measure_fma_peak of the same device, as in bench.py.  Writes one JSON file.
+
+usage: python tools/window_probe.py --out profiles/window_probe_b200.json [--n 65536] [--calls 200] [--ticks 40]
+"""
+import argparse
+import ctypes as C
+import json
+import os
+import subprocess
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+if ROOT not in sys.path:
+    sys.path.insert(0, ROOT)
+
+# operations per stage (add + mul + div + sqrt, an FMA counts 2): backward stage without / with a VO row (double arithmetic),
+# FULL-mode forward stage (leg-odometry update + time update with P_pp, handle precision) without / with a VO row
+FLOPS = {"window_back": 1165, "window_back_vo": 2331, "window_fwd": 1100, "window_fwd_vo": 1700}
+
+
+def algorithmic_bytes(N, K, esize, full):
+    """Bytes per instance: filtered states (54 words) and the record fields the backward pass reads (16 words) for N stages,
+    the double output; FULL mode adds the forward sweep's whole records (25 words) and the scratch-ring writes (54 words)."""
+    b = N * (54 + 16) * esize + 72 * K
+    if full:
+        b += N * (25 + 54) * esize
+    return b
+
+
+def algorithmic_flops(K, n_vo, full):
+    """(double flops, handle-precision flops) per instance for a window of K stages with n_vo VO rows."""
+    back = (K - 1 - n_vo) * FLOPS["window_back"] + n_vo * FLOPS["window_back_vo"]
+    fwd = ((K - n_vo) * FLOPS["window_fwd"] + n_vo * FLOPS["window_fwd_vo"]) if full else 0
+    return back, fwd
+
+
+def card():
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30).stdout.strip().splitlines()
+        return q[0] if q else "unknown"
+    except Exception as e:  # noqa: BLE001 -- the card line is informative, the run does not depend on it
+        return f"unknown ({e})"
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", required=True)
+    ap.add_argument("--n", type=int, default=65536)
+    ap.add_argument("--calls", type=int, default=200)
+    ap.add_argument("--ticks", type=int, default=40)
+    a = ap.parse_args()
+    import torch
+    from decentralized_ekf_mhe_b200 import build, estimator, synth
+    build.build()
+    if not torch.cuda.is_available():
+        raise SystemExit("window_probe needs a CUDA device")
+    peaks = estimator.measure_peaks(0)
+    N, n, warm = 20, a.n, 64
+    res = dict(card=card(), torch_device=torch.cuda.get_device_name(0), n=n, N=N, warmup_ticks=warm, calls=a.calls, peaks=peaks,
+               flops_per_stage=FLOPS, runs=[])
+    for vo_name, jitter in (("ragged", True), ("lockstep", False)):
+        d = synth.make_stream(n, warm + 2 * a.ticks + 1, vo_jitter=jitter, device="cuda")
+        vo = [bool(d["vo_flag"][s].any()) for s in range(d["gyro"].shape[0])]
+        for precision in ("fp64", "fp32"):
+            for mode, mname in ((0, "full"), (1, "incremental")):
+                prm = estimator.robot_params("go1", ekf_rate=200, N=N, window_solve=mode)
+                est = estimator.BatchedEstimator(prm, n, precision=precision)
+                est.run(0, warm, {k: v[:warm] for k, v in d.items()}, vo[:warm])
+                T = warm - 1
+                w = torch.empty(N, 9, n, dtype=torch.float64, device="cuda")
+                h = est._hd
+                K = torch.zeros(1, dtype=torch.int32)
+                call = lambda: h.check(h.L.dekf_get_window(h.h, C.c_void_p(w.data_ptr()), C.cast(K.data_ptr(), C.POINTER(C.c_int32))),
+                                       "dekf_get_window")
+                for _ in range(5):
+                    call()
+                torch.cuda.synchronize()
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record()
+                for _ in range(a.calls):
+                    call()
+                e1.record()
+                torch.cuda.synchronize()
+                ms = e0.elapsed_time(e1) / a.calls
+                n_vo = est.window_vo_count().double().mean().item()
+                Kv = int(K.item())
+                esize = 8 if precision == "fp64" else 4
+                by = algorithmic_bytes(N, Kv, esize, mode == 0)
+                fb, ff = algorithmic_flops(Kv, n_vo, mode == 0)
+                t_bw = by * n / (peaks["copy_gbs"] * 1e9) * 1e3
+                t_fl = (fb * n / (peaks["fp64_tflops"] * 1e12) + ff * n / (peaks[precision + "_tflops"] * 1e12)) * 1e3
+                # tick with and without the getter, alternated
+                tick = {"plain": [], "with_getter": []}
+                for j in range(2 * a.ticks):
+                    s = warm + j
+                    store = estimator.robot_store.from_stream(d, s)
+                    key = "with_getter" if j % 2 else "plain"
+                    e0.record()
+                    est.step(s, store)
+                    if j % 2:
+                        call()
+                    e1.record()
+                    torch.cuda.synchronize()
+                    tick[key].append(e0.elapsed_time(e1))
+                tick = {k: sorted(v)[len(v) // 2] for k, v in tick.items()}
+                r = dict(vo=vo_name, precision=precision, window_solve=mname, T=T, K=Kv, mean_vo_rows=n_vo, ms_per_call=ms,
+                         bytes_per_instance=by, double_flops_per_instance=fb, handle_flops_per_instance=ff,
+                         hbm_bound_ms=t_bw, flop_bound_ms=t_fl, bound="hbm" if t_bw >= t_fl else "fma",
+                         roof_fraction=max(t_bw, t_fl) / ms, tick_ms_median=tick,
+                         device_bytes=est.device_bytes())
+                print(json.dumps(r), flush=True)
+                res["runs"].append(r)
+                est.close()
+                del est
+        del d
+        torch.cuda.empty_cache()
+    os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+    with open(a.out, "w") as f:
+        json.dump(res, f, indent=1)
+    print("card:", res["card"])
+
+
+if __name__ == "__main__":
+    main()
