@@ -555,6 +555,19 @@ __global__ void __launch_bounds__(kBlock) k_window(const MheConst<T> c, const Mh
   mhe_window_smooth<T>(c, c64, dm, b, FULL ? scr : nullptr, Tk, i, xout, (size_t)dm.n);
 }
 
+// smoothed covariances of the window (dekf_get_window_cov): one thread per instance like k_window, which already sits at
+// 250-255 registers; the 9x9 gain G and Sigma - P_{k+1}^s of each thread (126 doubles) live in shared memory instead, one
+// column per thread so that a warp's accesses are conflict-free.  One-warp CTAs keep that area within the static limit.
+constexpr int kCovBlock = 32;
+template <typename T, bool FULL>
+__global__ void __launch_bounds__(kCovBlock) k_window_cov(const MheConst<T> c, const MheConst<double> c64, const Dims dm,
+                                                          const Buffers<T> b, T *scr, int Tk, double *pout) {
+  __shared__ double sh[126 * kCovBlock];
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= dm.n) return;
+  mhe_window_cov<T>(c, c64, dm, b, FULL ? scr : nullptr, Tk, i, pout, (size_t)dm.n, sh + threadIdx.x, kCovBlock);
+}
+
 }  // namespace dekf
 
 // ------------------------------------------------------------------------------------------------
@@ -2308,16 +2321,53 @@ int dekf_get_window(dekf_handle *h, double *x, int32_t *len) {
   return DEKF_OK;
 }
 
+int dekf_get_window_cov(dekf_handle *h, double *P, int32_t *len) {
+  if (!h) return DEKF_EINVAL;
+  if (!P) return fail(h, DEKF_EINVAL, "dekf_get_window_cov: null P");
+  if (h->cfg.est_type != 0) return fail(h, DEKF_EINVAL, "dekf_get_window_cov: est_type 1 (KF) has no window");
+  if (h->cfg.leg_odom_type != 0) return fail(h, DEKF_EINVAL, "dekf_get_window_cov: leg_odom_type 1 (foot states) is not supported");
+  if (h->row_V != nullptr)
+    return fail(h, DEKF_EINVAL, "dekf_get_window_cov: not available after dekf_add_state_rows (constrained window)");
+  if (h->cfg.v_box_enable || h->cfg.x_box_mask || h->bc.enable)
+    return fail(h, DEKF_EINVAL, "dekf_get_window_cov: not available with state bounds (v_box_enable / x_box_mask)");
+  if (h->next_T < 2) return fail(h, DEKF_ESTATE, "dekf_get_window_cov: needs a completed update(T >= 1)");
+  CK(cudaSetDevice(h->cfg.device));
+  const int Tk = h->next_T - 1, N = h->dm.N;
+  void *scr = nullptr;
+  if (h->mc64.window_solve == 0) {  // the same scratch ring as dekf_get_window: each call rewrites it before reading it
+    if (!h->win_scr) {
+      const size_t bytes = (size_t)N * 54 * h->dm.ns * (h->f32 ? sizeof(float) : sizeof(double));
+      CK(cudaMalloc(&h->win_scr, bytes));
+      h->extra_bytes += bytes;
+    }
+    scr = h->win_scr;
+  }
+  const dim3 grid((h->dm.n + kCovBlock - 1) / kCovBlock);
+  if (h->f32 && scr)
+    k_window_cov<float, true><<<grid, kCovBlock, 0, h->stream>>>(h->mc32, h->mc64, h->dm, h->b32, (float *)scr, Tk, P);
+  else if (h->f32)
+    k_window_cov<float, false><<<grid, kCovBlock, 0, h->stream>>>(h->mc32, h->mc64, h->dm, h->b32, nullptr, Tk, P);
+  else if (scr)
+    k_window_cov<double, true><<<grid, kCovBlock, 0, h->stream>>>(h->mc64, h->mc64, h->dm, h->b64, (double *)scr, Tk, P);
+  else
+    k_window_cov<double, false><<<grid, kCovBlock, 0, h->stream>>>(h->mc64, h->mc64, h->dm, h->b64, nullptr, Tk, P);
+  h->launches++;
+  CK(cudaGetLastError());
+  if (len) *len = Tk + 1 < N ? Tk + 1 : N;
+  return DEKF_OK;
+}
+
 int dekf_get_host(dekf_handle *h, int32_t what, void *host_out) {
   if (!h || !host_out) return fail(h, DEKF_EINVAL, "dekf_get_host: null argument");
   CK(cudaSetDevice(h->cfg.device));
   const size_t n = (size_t)h->dm.n;
   const size_t dsz = (size_t)h->ds;
-  const size_t rows[10] = {9, 3, dsz * dsz, dsz, 16, 1, dsz * dsz, dsz, 0, 9 * (size_t)h->dm.N};
-  if (what < 0 || what > DEKF_GET_WINDOW_X) return fail(h, DEKF_EINVAL, "dekf_get_host: unknown selector");
+  const size_t rows[11] = {9, 3, dsz * dsz, dsz, 16, 1, dsz * dsz, dsz, 0, 9 * (size_t)h->dm.N, 81 * (size_t)h->dm.N};
+  if (what < 0 || what > DEKF_GET_WINDOW_P) return fail(h, DEKF_EINVAL, "dekf_get_host: unknown selector");
   // one scratch for the life of the handle (the 200 Hz node shells call this every tick)
   size_t need = (dsz * dsz + dsz + 6 * (size_t)h->nl) * n * sizeof(double);
   if (what == DEKF_GET_WINDOW_X && need < rows[DEKF_GET_WINDOW_X] * n * sizeof(double)) need = rows[DEKF_GET_WINDOW_X] * n * sizeof(double);
+  if (what == DEKF_GET_WINDOW_P && need < rows[DEKF_GET_WINDOW_P] * n * sizeof(double)) need = rows[DEKF_GET_WINDOW_P] * n * sizeof(double);
   if (h->get_scratch_bytes < need) {
     cudaFree(h->get_scratch);
     h->get_scratch = nullptr;
@@ -2372,6 +2422,12 @@ int dekf_get_host(dekf_handle *h, int32_t what, void *host_out) {
       int32_t K = 0;
       rc = dekf_get_window(h, d, &K);
       bytes = (size_t)K * 9 * n * sizeof(double);
+      break;
+    }
+    case DEKF_GET_WINDOW_P: {
+      int32_t K = 0;
+      rc = dekf_get_window_cov(h, d, &K);
+      bytes = (size_t)K * 81 * n * sizeof(double);
       break;
     }
     default:

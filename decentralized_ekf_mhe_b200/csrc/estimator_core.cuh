@@ -2532,4 +2532,252 @@ DEKF_HD void mhe_window_smooth(const MheConst<T> &c, const MheConst<double> &c64
   window_backward<T>(c64, dm, b, scr, dm.N, Tk, i, xout, n_out);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Smoothed covariances (dekf_get_window_cov): for every window state the 9x9 block of the window QP's posterior covariance
+// (the x_k block of the inverse of its KKT matrix over the equality rows, in the 1/2 z'Hz scaling under which M_p = P^-1).
+// The covariance half of the RTS pass above, with its notation (P = P_k filtered, (mu, Sigma) the time update of stage k
+// incl. the VO row when it is an equality, L = [0, dt I, -h R], S = L P L' + C1 + R C_vo R'):
+//   P'_k = P - P L' S^-1 L P                        x_k conditioned on the VO row
+//   C'   = P (A' - L' S^-1 U') = P'_k A' - P L' S^-1 [C1 C2 0]    Cov(x_k, x_{k+1}) conditioned on the VO row
+//   G    = C' Sigma^-1,    P_k^s = P'_k - G (Sigma - P_{k+1}^s) G'
+// (no VO row: P' = P, C' = P A'), P_T^s = P_T.  Row r of P' needs P L' S^-1 only through its own row q_r = S^-1 (L P)_{:,r},
+// so P' is formed one row at a time and C' row r right after it.  Arithmetic in double, every multiply-add an explicit fm.
+// Each output entry is written to (r, c) and (c, r) from one value, so every block is exactly symmetric.
+// ------------------------------------------------------------------------------------------------
+// packed upper triangle of a symmetric 9x9, row-major: (r, c), r <= c
+DEKF_HD constexpr int sym9(int r, int c) { return r <= c ? r * (17 - r) / 2 + c : c * (17 - c) / 2 + r; }
+
+// field of entry (r, c) of the dense 9x9 matrix in the stored layout of a Cov9 (store_cov: pp, vv, bb, pv, pb, vb)
+DEKF_HD constexpr int cov_slot(int r, int c) {
+  return r > c ? cov_slot(c, r)
+               : (r / 3 == c / 3 ? 6 * (r / 3) + (r % 3 == 0 ? c % 3 : (r % 3 == 1 ? 2 + c % 3 : 5))
+                                 : 18 + 9 * (r / 3 + c / 3 - 1) + 3 * (r % 3) + c % 3);
+}
+
+// One backward covariance stage: reads P_{k+1}^s at pnext, writes P_k^s at pout (both [81] row-major at stride n_out).  `ck`,
+// `rec` as in window_back_stage.  `sh`: per-thread work area of 126 doubles at stride ss, G (row-major, [81]) then
+// Sigma - P_{k+1}^s (sym9, [45]).  P'_k is parked in the upper triangle of pout between the first and the last phase.
+template <typename D, typename T>
+DEKF_HD void window_cov_stage(const MheConst<D> &c, const T *ck, const T *rec, size_t ns, const double *pnext, double *pout,
+                              size_t n_out, double *sh, size_t ss) {
+  const bool vo = rec[REC_FLAG * ns] != T(0);
+  const D dt = c.dt, h = D(0.5) * c.dt * c.dt;
+  double *Gs = sh, *Ds = sh + 81 * ss;
+  // phase 1: P' (upper triangle into pout) and C' (into G), one row at a time; P is read row by row from ck, the finished
+  // entries left of the diagonal back from pout.  With a VO row, P L' is staged first in the Sigma - P^s area (free until
+  // phase 2): PLs[(m * 3 + j) * ss] = dt P(m, v_j) - h (P_{m,b} R')_j
+  {
+    M3<D> R;
+#pragma unroll
+    for (int f = 0; f < 9; ++f) R.a[f] = (D)rec[(REC_R + f) * ns];
+    S3<D> C1, C2;
+#pragma unroll
+    for (int f = 0; f < 6; ++f) C1.a[f] = C2.a[f] = D(0);
+    double *PLs = Ds;
+    D l00 = D(0), l10 = D(0), l20 = D(0), l11 = D(0), l21 = D(0), l22 = D(0), i0 = D(0), i1 = D(0), i2 = D(0);
+    if (vo) {
+      add_rot_diag(C1, R, c.n1);
+      add_rot_diag(C2, R, c.n2);
+#pragma unroll
+      for (int r = 0; r < 9; ++r) {
+        D pb[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) pb[k] = (D)ck[cov_slot(r, 6 + k) * ns];
+#pragma unroll
+        for (int j = 0; j < 3; ++j)
+          PLs[(r * 3 + j) * ss] = (double)fm(-h, fm(pb[2], R(j, 2), fm(pb[1], R(j, 1), pb[0] * R(j, 0))), dt * (D)ck[cov_slot(r, 3 + j) * ns]);
+      }
+      // S = L (P L') + C1 + R C_vo R',  (L y)_r = dt y_{v,r} - h (R y_b)_r
+      S3<D> Sm;
+#pragma unroll
+      for (int f = 0; f < 6; ++f) Sm.a[f] = D(0);
+      add_rot_diag(Sm, R, c.nvo);
+#pragma unroll
+      for (int r = 0; r < 3; ++r)
+#pragma unroll
+        for (int j = r; j < 3; ++j) {
+          const D RPb = fm(R(r, 2), (D)PLs[(8 * 3 + j) * ss], fm(R(r, 1), (D)PLs[(7 * 3 + j) * ss], R(r, 0) * (D)PLs[(6 * 3 + j) * ss]));
+          const int k = S3<D>::idx(r, j);
+          Sm.a[k] = fm(-h, RPb, fm(dt, (D)PLs[((3 + r) * 3 + j) * ss], Sm.a[k] + C1.a[k]));
+        }
+      l00 = sqrt(Sm.a[0]);
+      i0 = D(1) / l00;
+      l10 = Sm.a[1] * i0;
+      l20 = Sm.a[2] * i0;
+      l11 = sqrt(fm(-l10, l10, Sm.a[3]));
+      i1 = D(1) / l11;
+      l21 = fm(-l20, l10, Sm.a[4]) * i1;
+      l22 = sqrt(fm(-l21, l21, fm(-l20, l20, Sm.a[5])));
+      i2 = D(1) / l22;
+    }
+#pragma unroll
+    for (int r = 0; r < 9; ++r) {
+#if defined(__CUDA_ARCH__)
+      asm volatile("" ::: "memory");  // the entries of the earlier rows are re-read from pout, not kept in registers
+#endif
+      D y[9];  // row r of P'
+#pragma unroll
+      for (int cc = r; cc < 9; ++cc) y[cc] = (D)ck[cov_slot(r, cc) * ns];
+      D q[3] = {D(0), D(0), D(0)};  // S^-1 (L P)_{:,r}
+      if (vo) {
+        const D y0 = (D)PLs[(r * 3 + 0) * ss] * i0;
+        const D y1 = fm(-l10, y0, (D)PLs[(r * 3 + 1) * ss]) * i1;
+        const D y2 = fm(-l21, y1, fm(-l20, y0, (D)PLs[(r * 3 + 2) * ss])) * i2;
+        q[2] = y2 * i2;
+        q[1] = fm(-l21, q[2], y1) * i1;
+        q[0] = fm(-l20, q[2], fm(-l10, q[1], y0)) * i0;
+#pragma unroll
+        for (int cc = r; cc < 9; ++cc)
+          y[cc] = fm(-q[2], (D)PLs[(cc * 3 + 2) * ss], fm(-q[1], (D)PLs[(cc * 3 + 1) * ss], fm(-q[0], (D)PLs[(cc * 3 + 0) * ss], y[cc])));
+      }
+#pragma unroll
+      for (int cc = r; cc < 9; ++cc) pout[(r * 9 + cc) * n_out] = (double)y[cc];
+#pragma unroll
+      for (int cc = 0; cc < r; ++cc) y[cc] = (D)pout[(cc * 9 + r) * n_out];
+      // C' row r = A P'_{:,r} - [C1 q; C2 q; 0],  A y = [y_p + dt y_v - h R y_b;  y_v - dt R y_b;  y_b]
+#pragma unroll
+      for (int j = 0; j < 3; ++j) {
+        const D Rb = fm(R(j, 2), y[8], fm(R(j, 1), y[7], R(j, 0) * y[6]));
+        D cp = fm(-h, Rb, fm(dt, y[3 + j], y[j]));
+        D cv = fm(-dt, Rb, y[3 + j]);
+        if (vo) {
+          cp = fm(-C1(j, 2), q[2], fm(-C1(j, 1), q[1], fm(-C1(j, 0), q[0], cp)));
+          cv = fm(-C2(j, 2), q[2], fm(-C2(j, 1), q[1], fm(-C2(j, 0), q[0], cv)));
+        }
+        Gs[(r * 9 + j) * ss] = (double)cp;
+        Gs[(r * 9 + 3 + j) * ss] = (double)cv;
+        Gs[(r * 9 + 6 + j) * ss] = (double)y[6 + j];
+      }
+    }
+  }
+#if defined(__CUDA_ARCH__)
+  asm volatile("" ::: "memory");  // P' and C' are in memory; nothing of phase 1 stays live across the factorisation
+#endif
+  // phase 2: Sigma (the forward time update of stage k, in D), Sigma - P_{k+1}^s into Ds, Cholesky of Sigma in registers
+  D Lc[45], dinv[9];  // packed lower factor, row r at r (r + 1) / 2; reciprocal diagonal
+  {
+    Cov9<D> Sg;
+    Vec9<D> mu;
+    {
+      M3<D> R;
+      V3<D> as, dlt;
+      load_rec_dyn(rec, ns, R, as, dlt);
+      load_state_as(ck, ns, Sg, mu);
+      DefaultMath<D>::template prop<1>(c, Sg, mu, R, as, vo, dlt);
+    }
+#pragma unroll
+    for (int r = 0; r < 9; ++r)
+#pragma unroll
+      for (int cc = r; cc < 9; ++cc) Ds[sym9(r, cc) * ss] = (double)(cov_at(Sg, r, cc) - (D)pnext[(r * 9 + cc) * n_out]);
+#pragma unroll
+    for (int r = 0; r < 9; ++r) {
+#pragma unroll
+      for (int cc = 0; cc <= r; ++cc) {
+        D v = cov_at(Sg, r, cc);
+#pragma unroll
+        for (int k = 0; k < cc; ++k) v = fm(-Lc[r * (r + 1) / 2 + k], Lc[cc * (cc + 1) / 2 + k], v);
+        if (cc == r) {
+          const D d = sqrt(v);
+          Lc[r * (r + 1) / 2 + r] = d;
+          dinv[r] = D(1) / d;
+        } else {
+          Lc[r * (r + 1) / 2 + cc] = v * dinv[cc];
+        }
+      }
+    }
+  }
+  // phase 3: G row j = Sigma^-1 C'_{j,:}' (Sigma symmetric), in place
+#pragma unroll 1
+  for (int j = 0; j < 9; ++j) {
+    double *g = Gs + (size_t)j * 9 * ss;
+    D z[9];
+#pragma unroll
+    for (int r = 0; r < 9; ++r) {
+      D v = (D)g[r * ss];
+#pragma unroll
+      for (int k = 0; k < r; ++k) v = fm(-Lc[r * (r + 1) / 2 + k], z[k], v);
+      z[r] = v * dinv[r];
+    }
+#pragma unroll
+    for (int r = 8; r >= 0; --r) {
+      D v = z[r];
+#pragma unroll
+      for (int k = r + 1; k < 9; ++k) v = fm(-Lc[k * (k + 1) / 2 + r], z[k], v);
+      z[r] = v * dinv[r];
+    }
+#pragma unroll
+    for (int r = 0; r < 9; ++r) g[r * ss] = (double)z[r];
+  }
+#if defined(__CUDA_ARCH__)
+  asm volatile("" ::: "memory");
+#endif
+  // phase 4: P_k^s = P' - G (Sigma - P_{k+1}^s) G', one row of G (Sigma - P^s) at a time, upper triangle mirrored
+  D Dm[45];
+#pragma unroll
+  for (int f = 0; f < 45; ++f) Dm[f] = (D)Ds[f * ss];
+#pragma unroll 1
+  for (int r = 0; r < 9; ++r) {
+    D u[9];
+    {
+      D g[9];
+#pragma unroll
+      for (int l = 0; l < 9; ++l) g[l] = (D)Gs[(r * 9 + l) * ss];
+#pragma unroll
+      for (int mm = 0; mm < 9; ++mm) {
+        D v = Dm[sym9(mm, 0)] * g[0];
+#pragma unroll
+        for (int l = 1; l < 9; ++l) v = fm(Dm[sym9(mm, l)], g[l], v);
+        u[mm] = v;
+      }
+    }
+#pragma unroll 1
+    for (int cc = r; cc < 9; ++cc) {
+      D v = (D)pout[(r * 9 + cc) * n_out];
+#pragma unroll
+      for (int l = 0; l < 9; ++l) v = fm(-(D)Gs[(cc * 9 + l) * ss], u[l], v);
+      pout[(r * 9 + cc) * n_out] = (double)v;
+      pout[(cc * 9 + r) * n_out] = (double)v;
+    }
+  }
+}
+
+// Backward covariance pass over the filtered states of stages Tk-K+1 .. Tk in `ring` (as window_backward); pout [K][81][n_out].
+template <typename T>
+DEKF_HD void window_cov_backward(const MheConst<double> &c64, const Dims &dm, const Buffers<T> &b, const T *ring, int slots, int Tk,
+                                 int i, double *pout, size_t n_out, double *sh, size_t ss) {
+  const int N = dm.N, K = Tk + 1 < N ? Tk + 1 : N, k0 = Tk - K + 1;
+  const size_t ns = (size_t)dm.ns;
+  {
+    Cov9<double> P;  // P_T^s = P_T, widened
+    Vec9<double> x;
+    load_state_as(ring + (size_t)(Tk % slots) * 54 * ns + i, ns, P, x);
+    double *o = pout + (size_t)(Tk - k0) * 81 * n_out + i;
+#pragma unroll
+    for (int r = 0; r < 9; ++r)
+#pragma unroll
+      for (int cc = 0; cc < 9; ++cc) o[(r * 9 + cc) * n_out] = cov_at(P, r, cc);
+  }
+  for (int k = Tk - 1; k >= k0; --k) {
+    double *o = pout + (size_t)(k - k0) * 81 * n_out + i;
+    window_cov_stage<double, T>(c64, ring + (size_t)(k % slots) * 54 * ns + i, b.win + (size_t)(k % dm.NW) * REC_SIZE * ns + i, ns,
+                                o + 81 * n_out, o, n_out, sh, ss);
+  }
+}
+
+// Smoothed covariances of update(Tk) (Tk >= 1) for instance i: pout [K][81][n_out], block j = stage Tk-K+1+j, row-major over
+// (p_s, v_s, accel bias).  Sources of the filtered states as in mhe_window_smooth; sh / ss: see window_cov_stage.
+template <typename T>
+DEKF_HD void mhe_window_cov(const MheConst<T> &c, const MheConst<double> &c64, const Dims &dm, const Buffers<T> &b, T *scr, int Tk,
+                            int i, double *pout, size_t n_out, double *sh, size_t ss) {
+  if (scr == nullptr) {
+    window_cov_backward<T>(c64, dm, b, b.ckpt, dm.NW, Tk, i, pout, n_out, sh, ss);
+    return;
+  }
+  window_forward<T>(c, dm, b, Tk, i, scr);
+#if defined(__CUDA_ARCH__)
+  asm volatile("" ::: "memory");
+#endif
+  window_cov_backward<T>(c64, dm, b, scr, dm.N, Tk, i, pout, n_out, sh, ss);
+}
+
 }  // namespace dekf

@@ -8,6 +8,7 @@ Reference (C++; /root/reference/src)                          here (Python over 
   orien_ekf::timerCallback  orien_ekf.cpp:77-89                orien_ekf.timerCallback
   MHEproblem::M_p, n_p  MheSrb.hpp:86-87                       DecentralizedEstimation.mhe_qp_.M_p / .n_p
   MHEproblem::solution  MheSrb.hpp:58-112 (state blocks)       DecentralizedEstimation.mhe_qp_.x_window(), BatchedEstimator.window()
+  (posterior covariance of each state block; not in the reference)  DecentralizedEstimation.mhe_qp_.P_window(), BatchedEstimator.window_cov()
 
 torch is used for device memory and streams only; all arithmetic happens in libdekf_b200.so
 (sm_100a kernels).  Nothing here falls back to PyTorch or the CPU: a missing library or device raises.
@@ -173,6 +174,14 @@ def _window(h):
     return w[:K.value]
 
 
+def _window_cov(h):
+    """Smoothed covariances of the last update(T): [K][9][9][n] float64 on the device (dekf_get_window_cov)."""
+    P = torch.empty(int(h.cfg.N), 9, 9, h.n, dtype=torch.float64, device=h.device)
+    K = C.c_int32()
+    h.check(h.L.dekf_get_window_cov(h.h, _ptr(P), C.byref(K)), "dekf_get_window_cov")
+    return P[:K.value]
+
+
 class _MheQpView:
     """The public members of ``MHEproblem`` callers read: M_p, n_p (MheSrb.hpp:86-87) and the state blocks of
     ``solution`` (MheSrb.hpp:58-112)."""
@@ -203,6 +212,11 @@ class _MheQpView:
         """The window QP's optimum for every state of the last update(T), T >= 1: [K][9][n], K = min(T+1, N), row j =
         stage T-K+1+j (smoothed, oldest first); row K-1 equals x_MHE_ bit for bit."""
         return _window(self._o._hd)
+
+    def P_window(self):
+        """Posterior covariance of every state of the same window: [K][9][9][n], block j = stage T-K+1+j, over (p_s, v_s,
+        accel bias), exactly symmetric; block K-1 is the filtered covariance of x_T."""
+        return _window_cov(self._o._hd)
 
 
 class DecentralizedEstimation:
@@ -397,6 +411,11 @@ class BatchedEstimator:
         """Smoothed window of the last update(T), T >= 1 (the state blocks of MHEproblem::solution): [K][9][n] float64 on the
         device, K = min(T+1, N), row j = stage T-K+1+j; row K-1 equals x_MHE_ bit for bit.  Stream-ordered."""
         return _window(self._hd)
+
+    def window_cov(self):
+        """Smoothed covariances of the same window: [K][9][9][n] float64 on the device, block j = stage T-K+1+j, row-major
+        over (p_s, v_s, accel bias), exactly symmetric; block K-1 is the filtered covariance of x_T.  Stream-ordered."""
+        return _window_cov(self._hd)
 
     def step(self, T, store):
         h = self._hd

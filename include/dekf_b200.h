@@ -27,6 +27,7 @@
  *   dekf_get_arrival_cost       MHEproblem::M_p, n_p               MheSrb.hpp:86-87
  *   dekf_get_window             MHEproblem::solution (state blocks)   MheSrb.hpp:58-112 (getsolution narrows it to x_T,
  *                               MheSrb.cpp:715-723)
+ *   dekf_get_window_cov         posterior covariance of each state of MHEproblem::solution (not exported by the reference)
  *   dekf_get_p_vo               DecentralizedEstimation::p_vo_accmulate_   DecentralEst.hpp:280
  *   dekf_reset                  DecentralizedEstimation::reset()   DecentralEst.hpp:103
  *
@@ -257,6 +258,12 @@ int dekf_get_window_vo_count(dekf_handle *h, int32_t *count /*[n]*/);
  * forward sweep from the arrival cost into a scratch ring allocated on first use, counted in dekf_device_bytes).
  * DEKF_EINVAL for a null x or an unsupported handle, DEKF_ESTATE before the first update(T >= 1) and after dekf_reset. */
 int dekf_get_window(dekf_handle *h, double *x, int32_t *len);
+/* Smoothed covariances of the same window: for every state its 9x9 block of the window QP's posterior covariance (the x_k
+ * block of the inverse of the QP's KKT matrix over its equality rows; the scaling of dekf_get_arrival_cov, M_p = P^-1).
+ * P receives [K][81][n] (device pointer, stream-ordered), block j = stage T-K+1+j, each block row-major over (p_s, v_s,
+ * accel bias) and exactly symmetric; block K-1 is the filtered covariance of x_T.  *len (host, may be NULL) receives K.  Same
+ * handles, modes, scratch ring and errors as dekf_get_window (DEKF_EINVAL for a null P). */
+int dekf_get_window_cov(dekf_handle *h, double *P, int32_t *len);
 /* Host-pointer getter for callers without a CUDA runtime of their own (the C++ facade, a ROS node): `what` selects one
  * of the arrays above, `host_out` receives it (same [rows][n] layout, double; int32 for DEKF_GET_VO_COUNT).
  * Synchronises the handle's stream. */
@@ -271,7 +278,8 @@ enum {
   DEKF_GET_ARRIVAL_MEAN = 7, /* [9][n]  arrival mean;       est_type 1: x_KF_ */
   DEKF_GET_KF_GAIN = 8,      /* [9 * 3 * num_legs][n] K_KF_ (DecentralEst.hpp:290, DecentralEst.cpp:858), row-major 9 x 3L per
                               * instance; est_type 1, leg_odom_type 0 and cfg.kf_export_gain only */
-  DEKF_GET_WINDOW_X = 9      /* [K * 9][n] smoothed window (dekf_get_window); K <= N, so room for N * 9 rows suffices */
+  DEKF_GET_WINDOW_X = 9,     /* [K * 9][n] smoothed window (dekf_get_window); K <= N, so room for N * 9 rows suffices */
+  DEKF_GET_WINDOW_P = 10     /* [K * 81][n] smoothed covariances (dekf_get_window_cov); room for N * 81 rows suffices */
 };
 int dekf_get_host(dekf_handle *h, int32_t what, void *host_out);
 /* debug taps of the last step (only when cfg.debug_taps != 0): copied into caller DEVICE buffers, any may be NULL.

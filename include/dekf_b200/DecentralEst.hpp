@@ -9,6 +9,7 @@
 //        public results R_sb_, p_vo_accmulate_, x_MHE_, v_MHE_b_
 //   class MHEproblem::M_p, n_p    include/decentral_legged_est/MheSrb.hpp:86-87   dekf::DecentralizedEstimation::mhe_qp_.M_p()/n_p()
 //   MHEproblem::solution (state blocks) MheSrb.hpp:58-112                          dekf::DecentralizedEstimation::mhe_qp_.x_window()
+//   (posterior covariance of each state block, not in the reference)               dekf::DecentralizedEstimation::mhe_qp_.P_window()
 //
 // The reference estimates ONE robot and stores Eigen vectors; this facade steps `n_instances` robots per call and stores
 // flat SoA arrays `[rows][n_instances]` (instance fastest).  With n_instances == 1 every array has exactly the layout of the
@@ -358,6 +359,15 @@ class DecentralizedEstimation {
       const int K = o->last_T_ + 1 < o->N_ ? o->last_T_ + 1 : o->N_;
       w.resize((size_t)K * 9 * o->n_);
       return w;
+    }
+    // posterior covariance of each state of that window (dekf_get_window_cov): [K][81][n], block j = stage T-K+1+j, row-major
+    // over (p_s, v_s, accel bias); block K-1 is the filtered covariance of x_T
+    std::vector<double> P_window() const {
+      std::vector<double> P((size_t)o->N_ * 81 * o->n_);
+      detail::check(dekf_get_host(o->h_, DEKF_GET_WINDOW_P, P.data()), o->h_, "dekf_get_host");
+      const int K = o->last_T_ + 1 < o->N_ ? o->last_T_ + 1 : o->N_;
+      P.resize((size_t)K * 81 * o->n_);
+      return P;
     }
   } mhe_qp_{this};
 

@@ -1,4 +1,4 @@
-"""Cost of the smoothed-window getter (dekf_get_window) on a large batch.
+"""Cost of the smoothed-window getters (dekf_get_window, and dekf_get_window_cov in the cov_* fields) on a large batch.
 
 Go1, N = 20, 65,536 instances, fp64 and fp32 handles, ragged and lock-step VO arrival, both window_solve modes.  Per setup:
 64 warm-up ticks (dekf_run), then the getter timed with CUDA events over --calls calls, then a tick with and without the
@@ -22,6 +22,9 @@ if ROOT not in sys.path:
 # operations per stage (add + mul + div + sqrt, an FMA counts 2): backward stage without / with a VO row (double arithmetic),
 # FULL-mode forward stage (leg-odometry update + time update with P_pp, handle precision) without / with a VO row
 FLOPS = {"window_back": 1165, "window_back_vo": 2331, "window_fwd": 1100, "window_fwd_vo": 1700}
+# one backward stage of the covariance getter (dekf_get_window_cov, double arithmetic) without / with a VO row
+# (tests/hostsim/window_cov_flopcount.cpp; tests/test_window_covariance.py keeps them equal)
+FLOPS_COV = {"window_cov": 4786, "window_cov_vo": 6543}
 
 
 def algorithmic_bytes(N, K, esize, full):
@@ -31,6 +34,23 @@ def algorithmic_bytes(N, K, esize, full):
     if full:
         b += N * (25 + 54) * esize
     return b
+
+
+def cov_algorithmic_bytes(N, K, esize, full):
+    """Bytes per instance of dekf_get_window_cov: filtered covariances (45 words) and the record fields the backward pass reads
+    (16 words) for N stages, the double output [K][81]; FULL mode adds the forward sweep as in algorithmic_bytes.  Re-reading
+    P_{k+1}^s from the block just written is an L2 hit and not counted."""
+    b = N * (45 + 16) * esize + 648 * K
+    if full:
+        b += N * (25 + 54) * esize
+    return b
+
+
+def cov_algorithmic_flops(K, n_vo, full):
+    """(double flops, handle-precision flops) per instance of dekf_get_window_cov."""
+    back = (K - 1 - n_vo) * FLOPS_COV["window_cov"] + n_vo * FLOPS_COV["window_cov_vo"]
+    fwd = ((K - n_vo) * FLOPS["window_fwd"] + n_vo * FLOPS["window_fwd_vo"]) if full else 0
+    return back, fwd
 
 
 def algorithmic_flops(K, n_vo, full):
@@ -64,7 +84,7 @@ def main():
     peaks = estimator.measure_peaks(0)
     N, n, warm = 20, a.n, 64
     res = dict(card=card(), torch_device=torch.cuda.get_device_name(0), n=n, N=N, warmup_ticks=warm, calls=a.calls, peaks=peaks,
-               flops_per_stage=FLOPS, runs=[])
+               flops_per_stage=FLOPS, cov_flops_per_stage=FLOPS_COV, runs=[])
     for vo_name, jitter in (("ragged", True), ("lockstep", False)):
         d = synth.make_stream(n, warm + 2 * a.ticks + 1, vo_jitter=jitter, device="cuda")
         vo = [bool(d["vo_flag"][s].any()) for s in range(d["gyro"].shape[0])]
@@ -110,11 +130,34 @@ def main():
                     torch.cuda.synchronize()
                     tick[key].append(e0.elapsed_time(e1))
                 tick = {k: sorted(v)[len(v) // 2] for k, v in tick.items()}
+                # covariance getter: [K][81][n] doubles
+                P = torch.empty(N, 81, n, dtype=torch.float64, device="cuda")
+                cov = lambda: h.check(h.L.dekf_get_window_cov(h.h, C.c_void_p(P.data_ptr()), C.cast(K.data_ptr(), C.POINTER(C.c_int32))),
+                                      "dekf_get_window_cov")
+                for _ in range(5):
+                    cov()
+                torch.cuda.synchronize()
+                e0.record()
+                for _ in range(a.calls):
+                    cov()
+                e1.record()
+                torch.cuda.synchronize()
+                cov_ms = e0.elapsed_time(e1) / a.calls
+                n_vo_c = est.window_vo_count().double().mean().item()
+                Kc = int(K.item())
+                cby = cov_algorithmic_bytes(N, Kc, esize, mode == 0)
+                cfb, cff = cov_algorithmic_flops(Kc, n_vo_c, mode == 0)
+                c_bw = cby * n / (peaks["copy_gbs"] * 1e9) * 1e3
+                c_fl = (cfb * n / (peaks["fp64_tflops"] * 1e12) + cff * n / (peaks[precision + "_tflops"] * 1e12)) * 1e3
+                del P
                 r = dict(vo=vo_name, precision=precision, window_solve=mname, T=T, K=Kv, mean_vo_rows=n_vo, ms_per_call=ms,
                          bytes_per_instance=by, double_flops_per_instance=fb, handle_flops_per_instance=ff,
                          hbm_bound_ms=t_bw, flop_bound_ms=t_fl, bound="hbm" if t_bw >= t_fl else "fma",
                          roof_fraction=max(t_bw, t_fl) / ms, tick_ms_median=tick,
-                         device_bytes=est.device_bytes())
+                         device_bytes=est.device_bytes(), cov_K=Kc, cov_mean_vo_rows=n_vo_c, cov_ms_per_call=cov_ms,
+                         cov_bytes_per_instance=cby, cov_double_flops_per_instance=cfb, cov_handle_flops_per_instance=cff,
+                         cov_hbm_bound_ms=c_bw, cov_flop_bound_ms=c_fl, cov_bound="hbm" if c_bw >= c_fl else "fma",
+                         cov_roof_fraction=max(c_bw, c_fl) / cov_ms)
                 print(json.dumps(r), flush=True)
                 res["runs"].append(r)
                 est.close()
