@@ -15,6 +15,7 @@
 #include "host_setup.hpp"
 #include "box_team.cuh"
 #include "foot_team.cuh"
+#include "foot_window.cuh"
 
 namespace dekf {
 
@@ -231,6 +232,29 @@ __global__ void __launch_bounds__(kTeamBlock) k_foot_team(const FootConst fc, co
     tick_status(dm, b, Tk, i) = st;
     if (status_out != nullptr) status_out[i] = st;
   }
+}
+// smoothed window of the foot-state model (dekf_get_foot_window, foot_window.cuh): one warp per instance, two warps per CTA
+// with the stage record, P_{k+1} and the transpose buffer of each warp in shared memory
+constexpr int kFootWinBlock = 64;
+template <int L, bool WX, bool WP>
+__global__ void __launch_bounds__(kFootWinBlock) k_foot_window(const FootConst fc, const Dims dm, const Buffers<double> b,
+                                                               const FootBuffers fb, double *ring, int Tk, double *xout, double *Pout) {
+  __shared__ double sh[kFootWinBlock / 32][foot_win_smem_words<L>()];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int i = (int)((size_t)blockIdx.x * (kFootWinBlock / 32) + w);
+  if (i >= dm.n) return;  // whole warps only: no block-wide barrier follows
+  foot_window_team<L, WX, WP>(fc, dm, b, fb, ring, Tk, i, lane, sh[w], xout, Pout);
+}
+template <int L>
+void launch_foot_window(const FootConst &fc, const Dims &dm, const Buffers<double> &b, const FootBuffers &fb, double *ring, int Tk,
+                        double *x, double *P, cudaStream_t stream) {
+  const dim3 grid((dm.n + kFootWinBlock / 32 - 1) / (kFootWinBlock / 32));
+  if (x && P)
+    k_foot_window<L, true, true><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P);
+  else if (x)
+    k_foot_window<L, true, false><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P);
+  else
+    k_foot_window<L, false, true><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P);
 }
 // arrival cost of the foot-state model: (M_p, n_p) as the reference holds them (MheSrb.hpp:86-87)
 __global__ void k_get_arrival_foot(const Dims dm, const FootBuffers fb, int ds, double *Mout, double *nout) {
@@ -619,6 +643,7 @@ struct dekf_handle {
   FootBuffers fb = {nullptr, nullptr, nullptr};  // leg_odom_type 1
   void *ckpt_mem = nullptr;       // incremental window solve: checkpoint ring
   void *win_scr = nullptr;        // dekf_get_window on a full re-sweep handle: filtered states [N][54][ns] (first use)
+  double *foot_win_ring = nullptr;  // dekf_get_foot_window: stage factors [N-1][ns][FootWin<L>::W] (first use)
   int32_t *resweep_mem = nullptr;
   void *slab = nullptr;
   size_t slab_bytes = 0;
@@ -1194,6 +1219,7 @@ int dekf_destroy(dekf_handle *h) {
   cudaFree(h->fb.arr_m);
   cudaFree(h->ckpt_mem);
   cudaFree(h->win_scr);
+  cudaFree(h->foot_win_ring);
   cudaFree(h->resweep_mem);
   cudaFree(h->bb.fac);
   cudaFree(h->tb.prior);
@@ -2357,17 +2383,47 @@ int dekf_get_window_cov(dekf_handle *h, double *P, int32_t *len) {
   return DEKF_OK;
 }
 
+int dekf_get_foot_window(dekf_handle *h, double *x, double *P, int32_t *len) {
+  if (!h) return DEKF_EINVAL;
+  if (!x && !P) return fail(h, DEKF_EINVAL, "dekf_get_foot_window: x and P are both null");
+  if (h->cfg.est_type != 0) return fail(h, DEKF_EINVAL, "dekf_get_foot_window: est_type 1 (KF) has no window");
+  if (h->cfg.leg_odom_type != 1)
+    return fail(h, DEKF_EINVAL, "dekf_get_foot_window: leg_odom_type 0 handle; use dekf_get_window / dekf_get_window_cov");
+  if (h->next_T < 2) return fail(h, DEKF_ESTATE, "dekf_get_foot_window: needs a completed update(T >= 1)");
+  CK(cudaSetDevice(h->cfg.device));
+  const int Tk = h->next_T - 1, N = h->dm.N;
+  if (!h->foot_win_ring) {  // every call rewrites the stages it reads
+    const int W = h->nl == 4 ? FootWin<4>::W : (h->nl == 2 ? FootWin<2>::W : FootWin<1>::W);
+    const size_t bytes = (size_t)(N > 1 ? N - 1 : 1) * h->dm.ns * W * sizeof(double);
+    CK(cudaMalloc((void **)&h->foot_win_ring, bytes));
+    h->extra_bytes += bytes;
+  }
+  // dekf_run joins its internal streams into h->stream before returning, so this launch is ordered after every tick
+  if (h->nl == 4)
+    launch_foot_window<4>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, x, P, h->stream);
+  else if (h->nl == 2)
+    launch_foot_window<2>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, x, P, h->stream);
+  else
+    launch_foot_window<1>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, x, P, h->stream);
+  h->launches++;
+  CK(cudaGetLastError());
+  if (len) *len = Tk + 1 < N ? Tk + 1 : N;
+  return DEKF_OK;
+}
+
 int dekf_get_host(dekf_handle *h, int32_t what, void *host_out) {
   if (!h || !host_out) return fail(h, DEKF_EINVAL, "dekf_get_host: null argument");
   CK(cudaSetDevice(h->cfg.device));
   const size_t n = (size_t)h->dm.n;
   const size_t dsz = (size_t)h->ds;
-  const size_t rows[11] = {9, 3, dsz * dsz, dsz, 16, 1, dsz * dsz, dsz, 0, 9 * (size_t)h->dm.N, 81 * (size_t)h->dm.N};
-  if (what < 0 || what > DEKF_GET_WINDOW_P) return fail(h, DEKF_EINVAL, "dekf_get_host: unknown selector");
+  const size_t rows[13] = {9, 3, dsz * dsz, dsz, 16, 1, dsz * dsz, dsz, 0, 9 * (size_t)h->dm.N, 81 * (size_t)h->dm.N,
+                           dsz * (size_t)h->dm.N, dsz * dsz * (size_t)h->dm.N};
+  if (what < 0 || what > DEKF_GET_FOOT_WINDOW_P) return fail(h, DEKF_EINVAL, "dekf_get_host: unknown selector");
   // one scratch for the life of the handle (the 200 Hz node shells call this every tick)
   size_t need = (dsz * dsz + dsz + 6 * (size_t)h->nl) * n * sizeof(double);
   if (what == DEKF_GET_WINDOW_X && need < rows[DEKF_GET_WINDOW_X] * n * sizeof(double)) need = rows[DEKF_GET_WINDOW_X] * n * sizeof(double);
   if (what == DEKF_GET_WINDOW_P && need < rows[DEKF_GET_WINDOW_P] * n * sizeof(double)) need = rows[DEKF_GET_WINDOW_P] * n * sizeof(double);
+  if (what >= DEKF_GET_FOOT_WINDOW_X && need < rows[what] * n * sizeof(double)) need = rows[what] * n * sizeof(double);
   if (h->get_scratch_bytes < need) {
     cudaFree(h->get_scratch);
     h->get_scratch = nullptr;
@@ -2428,6 +2484,18 @@ int dekf_get_host(dekf_handle *h, int32_t what, void *host_out) {
       int32_t K = 0;
       rc = dekf_get_window_cov(h, d, &K);
       bytes = (size_t)K * 81 * n * sizeof(double);
+      break;
+    }
+    case DEKF_GET_FOOT_WINDOW_X: {
+      int32_t K = 0;
+      rc = dekf_get_foot_window(h, d, nullptr, &K);
+      bytes = (size_t)K * dsz * n * sizeof(double);
+      break;
+    }
+    case DEKF_GET_FOOT_WINDOW_P: {
+      int32_t K = 0;
+      rc = dekf_get_foot_window(h, nullptr, d, &K);
+      bytes = (size_t)K * dsz * dsz * n * sizeof(double);
       break;
     }
     default:

@@ -17,13 +17,16 @@ namespace dekf {
 
 #if defined(__CUDACC__)
 
-template <int DS, int K>
+template <int DS, int K, bool REC = false>
 struct FtFactor {
   // column K of the fused elimination (see header).  M: row r of Hxx (becomes L, inverse diagonal), X: row r of Hxp
   // (becomes Y), Mp: row r of M+ (starts as Hpp), m: rhs entry r (becomes y_r), gp: entry r of m+ (starts as gp).
-  static __device__ __forceinline__ void run(double (&M)[DS], double (&X)[DS], double (&Mp)[DS], double &m, double &gp, bool &ok, int r) {
+  // REC: *rinv receives this lane's 1 / L_rr (for the window getter's stage record).
+  static __device__ __forceinline__ void run(double (&M)[DS], double (&X)[DS], double (&Mp)[DS], double &m, double &gp, bool &ok, int r,
+                                             double *rinv = nullptr) {
     const double inv = bt_shfl(rsqrt(M[K]), K);
     if (!(inv > 0.0) || !(inv - inv == 0.0)) ok = false;
+    if (REC && r == K) *rinv = inv;
     const double Lrk = M[K] * inv;  // meaningful for r > K
     const double yk = bt_shfl(m * inv, K);
     if (r == K) m = yk;
@@ -48,12 +51,12 @@ struct FtFactor {
       const double Lck = bt_shfl(Lrk, c);
       if (r >= c) M[c] -= Lrk * Lck;
     }
-    FtFactor<DS, K + 1>::run(M, X, Mp, m, gp, ok, r);
+    FtFactor<DS, K + 1, REC>::run(M, X, Mp, m, gp, ok, r, rinv);
   }
 };
-template <int DS>
-struct FtFactor<DS, DS> {
-  static __device__ __forceinline__ void run(double (&)[DS], double (&)[DS], double (&)[DS], double &, double &, bool &, int) {}
+template <int DS, bool REC>
+struct FtFactor<DS, DS, REC> {
+  static __device__ __forceinline__ void run(double (&)[DS], double (&)[DS], double (&)[DS], double &, double &, bool &, int, double *) {}
 };
 
 // x = M^-1 m by Cholesky + forward substitution (column loop) + backward substitution (row K broadcasts L[K][c] x_K)
@@ -175,8 +178,12 @@ struct FootTeam {
       m += sf * qb;  // p rows: -Q b, foot rows: +Q b
     }
   }
-  // eliminate x_k (see header); R, as, dlt, vo: the common stage record; contact_mask: bit l = leg l in stance
-  __device__ __forceinline__ void propagate(const FootConst &fc, const double *R, const double *as, int contact_mask, bool vo, const double *dlt) {
+  // eliminate x_k (see header); R, as, dlt, vo: the common stage record; contact_mask: bit l = leg l in stance.
+  // REC: also write row r of the stage's factors L, Y, y into rec (FootWin<L> layout, footstate.cuh; rec null: this lane
+  // takes part in the shuffles only)
+  template <bool REC = false>
+  __device__ __forceinline__ void propagate(const FootConst &fc, const double *R, const double *as, int contact_mask, bool vo, const double *dlt,
+                                            double *rec = nullptr) {
     const BoxConst &bc = fc.bc;
     const double dt = bc.dt, h = 0.5 * bc.dt * bc.dt;
     double X[DS], Mp[DS], gp = 0.0;
@@ -263,10 +270,31 @@ struct FootTeam {
         }
       }
     }
-    FtFactor<DS, 0>::run(M, X, Mp, m, gp, ok, r);
+    if constexpr (REC) {
+      double inv = 0.0;
+      FtFactor<DS, 0, true>::run(M, X, Mp, m, gp, ok, r, &inv);
+      record(X, inv, rec);
+    } else {
+      FtFactor<DS, 0>::run(M, X, Mp, m, gp, ok, r);
+    }
 #pragma unroll
     for (int c = 0; c < DS; ++c) M[c] = Mp[c];
     m = gp;
+  }
+  // after FtFactor: M[c < r] is L(r, c) L_cc, M[r] is L_rr^2, X is row r of Hxp with the rows above eliminated (Y(r, :) L_rr) and
+  // m is y_r; inv is 1 / L_rr as FtFactor broadcast it.  The stores of one column cover consecutive words.
+  __device__ __forceinline__ void record(const double (&X)[DS], double inv, double *rec) const {
+    using FW = FootWin<L>;
+#pragma unroll
+    for (int c = 0; c < DS; ++c) {
+      const double ic = bt_shfl(inv, c);
+      if (rec != nullptr && r >= c) rec[FW::li(r, c)] = r == c ? inv : M[c] * ic;
+    }
+    if (rec == nullptr) return;
+#pragma unroll
+    for (int c = 0; c < DS; ++c)
+      if (r >= fw_rs(c)) rec[FW::yi(r, c)] = X[c] * inv;
+    rec[FW::vi(r)] = m;
   }
   // x = M^-1 m; returns x_r (M is destroyed)
   __device__ __forceinline__ double solve() {

@@ -56,6 +56,126 @@ DEKF_HD bool foot_chol(double *S, int n) {
   return true;
 }
 
+// ---- smoothed window of the foot-state model (dekf_get_foot_window) ----
+// After its leg rows, stage k of the sweep eliminates x_k from the joint quadratic in (x_k, x_{k+1}) with Hxx = L L',
+// Y = L^-1 Hxp, y = L^-1 g_x.  Conditioned on x_{k+1}, x_k is Gaussian with information Hxx and mean Hxx^-1 (g_x - Hxp x_{k+1}),
+// so the window's optimum and posterior covariance follow backwards from x_T = M_T^-1 m_T, P_T = M_T^-1:
+//   x_k = L^-T (y - Y x_{k+1}),      P_k = L^-T (I + Y P_{k+1} Y') L^-1.
+// The stage record holds (L, Y, y) in FootWin<L>::W doubles, packed by column so that the lanes of a warp (lane r = row r,
+// foot_window.cuh) touch consecutive words for every column:
+//   L(r, c), r >= c          at fw_li(r, c) = lcol(c) + r - c, the diagonal as 1 / L_cc                  NL = DS (DS + 1) / 2
+//   Y(r, c), r >= fw_rs(c)   at NL + ycol(c) + r - fw_rs(c); Hxp is block diagonal (base 9 x 9, one 3 x 3 block per foot)
+//                            and L^-1 lower triangular, so Y(r, c) = 0 above the block of c                    NY
+//   y_r                      at NL + NY + r                                                                     DS
+// Go1 (DS = 21): 231 + 279 + 21 = 531 doubles per stage.
+DEKF_HD constexpr int fw_rs(int c) { return c < 9 ? 0 : 9 + 3 * ((c - 9) / 3); }      // first row of Y's column c that can be nonzero
+DEKF_HD constexpr int fw_ce(int r) { return r < 9 ? 9 : 9 + 3 * ((r - 9) / 3 + 1); }  // Y(r, c) = 0 for c >= fw_ce(r)
+DEKF_HD constexpr int fw_lcol(int DS, int c) { return c * DS - c * (c - 1) / 2; }
+DEKF_HD constexpr int fw_ycol(int DS, int c) {
+  int o = 0;
+  for (int k = 0; k < c; ++k) o += DS - fw_rs(k);
+  return o;
+}
+template <int L>
+struct FootWin {
+  static constexpr int DS = 9 + 3 * L;
+  static constexpr int NL = DS * (DS + 1) / 2;
+  static constexpr int NY = fw_ycol(DS, DS);
+  static constexpr int W = NL + NY + DS;  // doubles per stage
+  DEKF_HD static constexpr int li(int r, int c) { return fw_lcol(DS, c) + r - c; }
+  DEKF_HD static constexpr int yi(int r, int c) { return NL + fw_ycol(DS, c) + r - fw_rs(c); }
+  DEKF_HD static constexpr int vi(int r) { return NL + NY + r; }
+};
+
+// stage record from the serial factors: Lm row-major lower Cholesky factor (L_rr on the diagonal), Y row-major, y
+template <int L>
+DEKF_HD void foot_win_record(const double *Lm, const double *Y, const double *y, double *rec) {
+  using FW = FootWin<L>;
+  constexpr int DS = FW::DS;
+  for (int c = 0; c < DS; ++c) {
+    rec[FW::li(c, c)] = 1.0 / Lm[c * DS + c];
+    for (int r = c + 1; r < DS; ++r) rec[FW::li(r, c)] = Lm[r * DS + c];
+    for (int r = fw_rs(c); r < DS; ++r) rec[FW::yi(r, c)] = Y[r * DS + c];
+  }
+  for (int r = 0; r < DS; ++r) rec[FW::vi(r)] = y[r];
+}
+
+// z = L^-T z (back substitution with the L of one stage record)
+template <typename S, int L>
+DEKF_HD void fw_back(const S *rec, S *z) {
+  using FW = FootWin<L>;
+  constexpr int DS = FW::DS;
+#pragma unroll
+  for (int r = DS - 1; r >= 0; --r) {
+    S v = z[r];
+#pragma unroll
+    for (int k = r + 1; k < DS; ++k) v -= rec[FW::li(k, r)] * z[k];
+    z[r] = v * rec[FW::li(r, r)];
+  }
+}
+
+// backward mean stage: x = L^-T (y - Y xn), xn = x_{k+1}
+template <typename S, int L>
+DEKF_HD void fw_mean_stage(const S *rec, const S *xn, S *x) {
+  using FW = FootWin<L>;
+  constexpr int DS = FW::DS;
+#pragma unroll
+  for (int r = 0; r < DS; ++r) {
+    S v = rec[FW::vi(r)];
+#pragma unroll
+    for (int c = 0; c < fw_ce(r); ++c) v -= rec[FW::yi(r, c)] * xn[c];
+    x[r] = v;
+  }
+  fw_back<S, L>(rec, x);
+}
+
+// column j of G = L^-T (I + Y P Y'), P = P_{k+1} (full, row stride sp); P null: G = L^-T (for P_T = L^-T L^-1)
+template <typename S, int L>
+DEKF_HD void fw_cov_col(const S *rec, const S *P, int sp, int j, S *g) {
+  using FW = FootWin<L>;
+  constexpr int DS = FW::DS;
+  if (P != nullptr) {
+    S v[DS], w[DS];
+#pragma unroll
+    for (int c = 0; c < DS; ++c) v[c] = j >= fw_rs(c) ? rec[FW::yi(j, c)] : S(0.0);  // row j of Y
+#pragma unroll
+    for (int a = 0; a < DS; ++a) {  // w = P v
+      S t = P[a * sp] * v[0];
+#pragma unroll
+      for (int c = 1; c < DS; ++c) t += P[a * sp + c] * v[c];
+      w[a] = t;
+    }
+#pragma unroll
+    for (int r = 0; r < DS; ++r) {  // e_j + Y w
+      S t = r == j ? S(1.0) : S(0.0);
+#pragma unroll
+      for (int c = 0; c < fw_ce(r); ++c) t += rec[FW::yi(r, c)] * w[c];
+      g[r] = t;
+    }
+  } else {
+#pragma unroll
+    for (int r = 0; r < DS; ++r) g[r] = r == j ? S(1.0) : S(0.0);
+  }
+  fw_back<S, L>(rec, g);
+}
+
+// serial backward covariance stage: Pk = L^-T (I + Y Pn Y') L^-1 = L^-T G' (Pn null: L^-T L^-1), DS x DS row-major; Pk is
+// written from its lower triangle, so every block is exactly symmetric
+template <typename S, int L>
+DEKF_HD void fw_cov_stage(const S *rec, const S *Pn, S *Pk) {
+  constexpr int DS = 9 + 3 * L;
+  S G[DS * DS], g[DS];
+  for (int j = 0; j < DS; ++j) {
+    fw_cov_col<S, L>(rec, Pn, DS, j, g);
+    for (int r = 0; r < DS; ++r) G[r * DS + j] = g[r];
+  }
+  for (int c = 0; c < DS; ++c) {
+    for (int r = 0; r < DS; ++r) g[r] = G[c * DS + r];
+    fw_back<S, L>(rec, g);  // column c of Pk
+    for (int r = c; r < DS; ++r) Pk[r * DS + c] = Pk[c * DS + r] = g[r];
+  }
+}
+
 template <int L>
 struct FootFilter {
   static constexpr int DS = 9 + 3 * L;
@@ -135,7 +255,10 @@ struct FootFilter {
 
   // Eliminate x_k from  1/2 x'Mx - m'x + 1/2 |A x - x+ + c|^2_Q (+ 1/2 |p - p+ + Delta|^2_Qc): (M, m) becomes the
   // information of x_{k+1} (DecentralEst.cpp:387-484; marginalizeQP's Schur complement, MheSrb.cpp:475-713).
-  DEKF_HD void propagate(const FootConst &fc, const double *R, const double *as, int contact_mask, bool vo, const double *dlt) {
+  // REC: also write the stage's factors L, Y, y into rec (FootWin<L> layout) for the window getter's backward passes.
+  template <bool REC = false>
+  DEKF_HD void propagate(const FootConst &fc, const double *R, const double *as, int contact_mask, bool vo, const double *dlt,
+                         double *rec = nullptr) {
     BoxStage s;
     for (int f = 0; f < 9; ++f) s.R[f] = R[f];
     for (int f = 0; f < 3; ++f) {
@@ -185,6 +308,7 @@ struct FootFilter {
       for (int k = 0; k < r; ++k) v -= M[r * DS + k] * m[k];
       m[r] = v / M[r * DS + r];
     }
+    if constexpr (REC) foot_win_record<L>(M, Hxp, m, rec);
     // M+ = Hpp - Y'Y,  m+ = gp - Y'y
     for (int r = 0; r < DS; ++r) {
       double v = gp[r];
@@ -275,6 +399,66 @@ DEKF_HD int foot_solve(const FootConst &fc, const Dims &dm, const Buffers<T> &b,
   if (out.v_body != nullptr)
     for (int r = 0; r < 3; ++r) out.v_body[(size_t)r * n + i] = R[r * 3 + 0] * u[0] + R[r * 3 + 1] * u[1] + R[r * 3 + 2] * u[2];
   return status;
+}
+
+// Smoothed window of update(Tk) (est_type 0), serial form of dekf_get_foot_window: the K = min(Tk+1, N) states
+// Tk-K+1 .. Tk.  The forward sweep of foot_solve from the arrival cost written by that update (the prior of x_{Tk-N+1};
+// Prior_0 while Tk < N) records every stage into rec ([K][FootWin<L>::W], the last slot takes L_T); then the backward
+// mean and covariance passes.  x: [K][DS] and P: [K][DS * DS] at element stride os (either may be null).  Row K-1 of x is
+// foot_solve's x_T bit for bit.
+template <typename T, int L>
+DEKF_HD void foot_window_smooth(const FootConst &fc, const Dims &dm, const Buffers<T> &b, const FootBuffers &fb, int Tk, int i,
+                                double *rec, double *x, double *P, size_t os) {
+  using FW = FootWin<L>;
+  constexpr int DS = FW::DS, W = FW::W;
+  const size_t ns = (size_t)dm.ns;
+  const int N = dm.N, RS = foot_rec_size(L);
+  const int K = Tk + 1 < N ? Tk + 1 : N, k0 = Tk - K + 1;
+  FootFilter<L> f;
+  auto leg = [&](int k) { return fb.leg + (size_t)(k % dm.NW) * RS * ns + i; };
+  double R[9], as[3], dlt[3], xv[DS], xn[DS];
+  bool vo;
+  if (Tk >= N)
+    f.load(fb, ns, i);
+  else
+    f.set_prior(fc, leg(0), ns);
+  for (int k = k0;; ++k) {
+    f.meas_update(leg(k), ns);
+    if (k == Tk) break;
+    foot_common(dm, b, k, i, R, as, dlt, vo);
+    f.template propagate<true>(fc, R, as, (int)leg(k)[(size_t)(9 * L) * ns], vo, dlt, rec + (size_t)(k - k0) * W);
+  }
+  double Lc[DS * DS];  // the factor solve() forms, kept for P_T
+  for (int e = 0; e < DS * DS; ++e) Lc[e] = f.M[e];
+  foot_chol(Lc, DS);
+  f.solve(xv);
+  double *rT = rec + (size_t)(K - 1) * W;
+  for (int c = 0; c < DS; ++c) {
+    rT[FW::li(c, c)] = 1.0 / Lc[c * DS + c];
+    for (int r = c + 1; r < DS; ++r) rT[FW::li(r, c)] = Lc[r * DS + c];
+  }
+  double Pn[DS * DS], Pk[DS * DS];
+  if (x != nullptr)
+    for (int c = 0; c < DS; ++c) x[((size_t)(K - 1) * DS + c) * os] = xv[c];
+  if (P != nullptr) {
+    fw_cov_stage<double, L>(rT, nullptr, Pn);
+    for (int e = 0; e < DS * DS; ++e) P[((size_t)(K - 1) * DS * DS + e) * os] = Pn[e];
+  }
+  for (int j = K - 2; j >= 0; --j) {
+    const double *rj = rec + (size_t)j * W;
+    if (x != nullptr) {
+      for (int c = 0; c < DS; ++c) xn[c] = xv[c];
+      fw_mean_stage<double, L>(rj, xn, xv);
+      for (int c = 0; c < DS; ++c) x[((size_t)j * DS + c) * os] = xv[c];
+    }
+    if (P != nullptr) {
+      fw_cov_stage<double, L>(rj, Pn, Pk);
+      for (int e = 0; e < DS * DS; ++e) {
+        P[((size_t)j * DS * DS + e) * os] = Pk[e];
+        Pn[e] = Pk[e];
+      }
+    }
+  }
 }
 
 }  // namespace dekf

@@ -9,6 +9,7 @@ Reference (C++; /root/reference/src)                          here (Python over 
   MHEproblem::M_p, n_p  MheSrb.hpp:86-87                       DecentralizedEstimation.mhe_qp_.M_p / .n_p
   MHEproblem::solution  MheSrb.hpp:58-112 (state blocks)       DecentralizedEstimation.mhe_qp_.x_window(), BatchedEstimator.window()
   (posterior covariance of each state block; not in the reference)  DecentralizedEstimation.mhe_qp_.P_window(), BatchedEstimator.window_cov()
+  (leg_odom_type 1: the same with 9 + 3L rows per state block)    the same methods, through dekf_get_foot_window
 
 torch is used for device memory and streams only; all arithmetic happens in libdekf_b200.so
 (sm_100a kernels).  Nothing here falls back to PyTorch or the CPU: a missing library or device raises.
@@ -166,8 +167,22 @@ class _Handle:
             chk(quat, 4, "quaternion_") if quat is not None else None)
 
 
+def _foot_window(h, want_x, want_P):
+    """Smoothed window of a foot-state handle: ([K][ds][n], [K][ds][ds][n]) float64 on the device (dekf_get_foot_window)."""
+    N, ds = int(h.cfg.N), h.ds
+    x = torch.empty(N, ds, h.n, dtype=torch.float64, device=h.device) if want_x else None
+    P = torch.empty(N, ds, ds, h.n, dtype=torch.float64, device=h.device) if want_P else None
+    K = C.c_int32()
+    h.check(h.L.dekf_get_foot_window(h.h, _ptr(x) if want_x else None, _ptr(P) if want_P else None, C.byref(K)),
+            "dekf_get_foot_window")
+    return (x[:K.value] if want_x else None), (P[:K.value] if want_P else None)
+
+
 def _window(h):
-    """Smoothed window of the last update(T): [K][9][n] float64 on the device (dekf_get_window)."""
+    """Smoothed window of the last update(T): [K][9][n] float64 on the device (dekf_get_window); foot-state handles
+    (leg_odom_type 1): [K][ds][n] (dekf_get_foot_window)."""
+    if h.cfg.leg_odom_type == 1:
+        return _foot_window(h, True, False)[0]
     w = torch.empty(int(h.cfg.N), 9, h.n, dtype=torch.float64, device=h.device)
     K = C.c_int32()
     h.check(h.L.dekf_get_window(h.h, _ptr(w), C.byref(K)), "dekf_get_window")
@@ -175,7 +190,10 @@ def _window(h):
 
 
 def _window_cov(h):
-    """Smoothed covariances of the last update(T): [K][9][9][n] float64 on the device (dekf_get_window_cov)."""
+    """Smoothed covariances of the last update(T): [K][9][9][n] float64 on the device (dekf_get_window_cov); foot-state
+    handles (leg_odom_type 1): [K][ds][ds][n] (dekf_get_foot_window)."""
+    if h.cfg.leg_odom_type == 1:
+        return _foot_window(h, False, True)[1]
     P = torch.empty(int(h.cfg.N), 9, 9, h.n, dtype=torch.float64, device=h.device)
     K = C.c_int32()
     h.check(h.L.dekf_get_window_cov(h.h, _ptr(P), C.byref(K)), "dekf_get_window_cov")

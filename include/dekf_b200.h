@@ -28,6 +28,7 @@
  *   dekf_get_window             MHEproblem::solution (state blocks)   MheSrb.hpp:58-112 (getsolution narrows it to x_T,
  *                               MheSrb.cpp:715-723)
  *   dekf_get_window_cov         posterior covariance of each state of MHEproblem::solution (not exported by the reference)
+ *   dekf_get_foot_window        MHEproblem::solution and its covariances for leg_odom_type 1 (9 + 3 num_legs rows per state)
  *   dekf_get_p_vo               DecentralizedEstimation::p_vo_accmulate_   DecentralEst.hpp:280
  *   dekf_reset                  DecentralizedEstimation::reset()   DecentralEst.hpp:103
  *
@@ -264,6 +265,15 @@ int dekf_get_window(dekf_handle *h, double *x, int32_t *len);
  * accel bias) and exactly symmetric; block K-1 is the filtered covariance of x_T.  *len (host, may be NULL) receives K.  Same
  * handles, modes, scratch ring and errors as dekf_get_window (DEKF_EINVAL for a null P). */
 int dekf_get_window_cov(dekf_handle *h, double *P, int32_t *len);
+/* Smoothed window of a foot-state handle (leg_odom_type 1, est_type 0): for every state of the last update's window its QP
+ * optimum over all ds = dekf_state_dim(h) = 9 + 3 num_legs components (p_s, v_s, accel bias, p_foot_1 .. p_foot_L) and,
+ * optionally, its ds x ds posterior covariance (the x_k block of the inverse of the window's normal matrix, in the scaling
+ * where M_p is the information; row-major, exactly symmetric).  x receives [K][ds][n], P receives [K][ds * ds][n] (device
+ * pointers, stream-ordered; either may be NULL, not both), row / block j = stage T-K+1+j, K = min(T+1, N); row K-1 equals
+ * dekf_outputs.x of that update.  *len (host, may be NULL) receives K.  A device ring of the stage factors is allocated on
+ * first use and counted in dekf_device_bytes.  DEKF_EINVAL for null x and P, est_type 1 and leg_odom_type 0 handles (those
+ * use dekf_get_window / dekf_get_window_cov); DEKF_ESTATE before the first update(T >= 1) and after dekf_reset. */
+int dekf_get_foot_window(dekf_handle *h, double *x, double *P, int32_t *len);
 /* Host-pointer getter for callers without a CUDA runtime of their own (the C++ facade, a ROS node): `what` selects one
  * of the arrays above, `host_out` receives it (same [rows][n] layout, double; int32 for DEKF_GET_VO_COUNT).
  * Synchronises the handle's stream. */
@@ -279,7 +289,9 @@ enum {
   DEKF_GET_KF_GAIN = 8,      /* [9 * 3 * num_legs][n] K_KF_ (DecentralEst.hpp:290, DecentralEst.cpp:858), row-major 9 x 3L per
                               * instance; est_type 1, leg_odom_type 0 and cfg.kf_export_gain only */
   DEKF_GET_WINDOW_X = 9,     /* [K * 9][n] smoothed window (dekf_get_window); K <= N, so room for N * 9 rows suffices */
-  DEKF_GET_WINDOW_P = 10     /* [K * 81][n] smoothed covariances (dekf_get_window_cov); room for N * 81 rows suffices */
+  DEKF_GET_WINDOW_P = 10,    /* [K * 81][n] smoothed covariances (dekf_get_window_cov); room for N * 81 rows suffices */
+  DEKF_GET_FOOT_WINDOW_X = 11, /* [K * ds][n] smoothed window of a foot-state handle (dekf_get_foot_window); room for N * ds rows */
+  DEKF_GET_FOOT_WINDOW_P = 12  /* [K * ds * ds][n] its covariances (dekf_get_foot_window); room for N * ds * ds rows */
 };
 int dekf_get_host(dekf_handle *h, int32_t what, void *host_out);
 /* debug taps of the last step (only when cfg.debug_taps != 0): copied into caller DEVICE buffers, any may be NULL.

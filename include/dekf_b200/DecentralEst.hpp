@@ -10,6 +10,7 @@
 //   class MHEproblem::M_p, n_p    include/decentral_legged_est/MheSrb.hpp:86-87   dekf::DecentralizedEstimation::mhe_qp_.M_p()/n_p()
 //   MHEproblem::solution (state blocks) MheSrb.hpp:58-112                          dekf::DecentralizedEstimation::mhe_qp_.x_window()
 //   (posterior covariance of each state block, not in the reference)               dekf::DecentralizedEstimation::mhe_qp_.P_window()
+//   (both for leg_odom_type 1: 9 + 3 num_legs rows per state block)                 the same, through dekf_get_foot_window
 //
 // The reference estimates ONE robot and stores Eigen vectors; this facade steps `n_instances` robots per call and stores
 // flat SoA arrays `[rows][n_instances]` (instance fastest).  With n_instances == 1 every array has exactly the layout of the
@@ -352,21 +353,24 @@ class DecentralizedEstimation {
       return v;
     }
     // the state blocks of MHEproblem::solution (MheSrb.hpp:58-112) of the last update(T), T >= 1: the smoothed window
-    // [K][9][n], K = min(T+1, N), row j = stage T-K+1+j, row K-1 == x_MHE_ (dekf_get_window)
+    // [K][ds][n], K = min(T+1, N), row j = stage T-K+1+j, row K-1 == x_MHE_ (dekf_get_window; foot-state handles, ds = 9 + 3L:
+    // dekf_get_foot_window)
     std::vector<double> x_window() const {
-      std::vector<double> w((size_t)o->N_ * 9 * o->n_);
-      detail::check(dekf_get_host(o->h_, DEKF_GET_WINDOW_X, w.data()), o->h_, "dekf_get_host");
+      const size_t ds = (size_t)o->ds_;
+      std::vector<double> w((size_t)o->N_ * ds * o->n_);
+      detail::check(dekf_get_host(o->h_, ds != 9 ? DEKF_GET_FOOT_WINDOW_X : DEKF_GET_WINDOW_X, w.data()), o->h_, "dekf_get_host");
       const int K = o->last_T_ + 1 < o->N_ ? o->last_T_ + 1 : o->N_;
-      w.resize((size_t)K * 9 * o->n_);
+      w.resize((size_t)K * ds * o->n_);
       return w;
     }
-    // posterior covariance of each state of that window (dekf_get_window_cov): [K][81][n], block j = stage T-K+1+j, row-major
-    // over (p_s, v_s, accel bias); block K-1 is the filtered covariance of x_T
+    // posterior covariance of each state of that window (dekf_get_window_cov; foot-state handles: dekf_get_foot_window):
+    // [K][ds * ds][n], block j = stage T-K+1+j, row-major over the state components; block K-1 is the covariance of x_T
     std::vector<double> P_window() const {
-      std::vector<double> P((size_t)o->N_ * 81 * o->n_);
-      detail::check(dekf_get_host(o->h_, DEKF_GET_WINDOW_P, P.data()), o->h_, "dekf_get_host");
+      const size_t ds = (size_t)o->ds_;
+      std::vector<double> P((size_t)o->N_ * ds * ds * o->n_);
+      detail::check(dekf_get_host(o->h_, ds != 9 ? DEKF_GET_FOOT_WINDOW_P : DEKF_GET_WINDOW_P, P.data()), o->h_, "dekf_get_host");
       const int K = o->last_T_ + 1 < o->N_ ? o->last_T_ + 1 : o->N_;
-      P.resize((size_t)K * 81 * o->n_);
+      P.resize((size_t)K * ds * ds * o->n_);
       return P;
     }
   } mhe_qp_{this};

@@ -1,4 +1,5 @@
-"""Cost of the smoothed-window getters (dekf_get_window, and dekf_get_window_cov in the cov_* fields) on a large batch.
+"""Cost of the smoothed-window getters (dekf_get_window, and dekf_get_window_cov in the cov_* fields) on a large batch;
+with --foot, of dekf_get_foot_window on Go1 foot-state handles (x-only, P-only, x+P and one step, at each --foot-n).
 
 Go1, N = 20, 65,536 instances, fp64 and fp32 handles, ragged and lock-step VO arrival, both window_solve modes.  Per setup:
 64 warm-up ticks (dekf_run), then the getter timed with CUDA events over --calls calls, then a tick with and without the
@@ -7,6 +8,7 @@ tests/hostsim/window_flopcount.cpp (FLOPS below; tests/test_window_smoother.py k
 dekf_measure_copy_bw / dekf_measure_fma_peak of the same device, as in bench.py.  Writes one JSON file.
 
 usage: python tools/window_probe.py --out profiles/window_probe_b200.json [--n 65536] [--calls 200] [--ticks 40]
+       python tools/window_probe.py --foot --out profiles/foot_window_probe_b200.json [--foot-n 16384 65536] [--calls 20]
 """
 import argparse
 import ctypes as C
@@ -60,6 +62,97 @@ def algorithmic_flops(K, n_vo, full):
     return back, fwd
 
 
+
+def foot_stage_flops(L):
+    """Operations of the backward passes of dekf_get_foot_window per stage (double; tests/hostsim/foot_window_flopcount.cpp,
+    tests/test_foot_window.py keeps them equal): mean x_k = L^-T (y - Y x_{k+1}); covariance P_k = L^-T (I + Y P Y') L^-1
+    (ds columns of G, each P v, Y w and a back substitution, then ds back substitutions); cov_T = L_T^-T L_T^-1."""
+    ds = 9 + 3 * L
+    ny = 9 * ds + sum(ds - (9 + 3 * ((c - 9) // 3)) for c in range(9, ds))   # nonzeros of Y
+    back = ds * ds
+    return {"mean": 2 * ny + back, "cov": ds * (ds * (2 * ds - 1) + 2 * ny + back) + ds * back, "cov_T": 2 * ds * back}
+
+
+def foot_words(L):
+    """(stage record words W, nonzeros of L, nonzeros of Y) of the dekf_get_foot_window ring."""
+    ds = 9 + 3 * L
+    nl = ds * (ds + 1) // 2
+    ny = 9 * ds + sum(ds - (9 + 3 * ((c - 9) // 3)) for c in range(9, ds))
+    return nl + ny + ds, nl, ny
+
+
+def foot_algorithmic(L, K, want_x, want_P):
+    """(bytes, backward-pass double flops) per instance of one dekf_get_foot_window call over K states.  Bytes: the forward
+    sweep's inputs (arrival cost, K leg records of 9L+1 words and K common records of 16 words), the ring written and read
+    back ((K-1) W words each way), the outputs.  The forward sweep's flops (the step's own sweep, repeated) are not in the
+    tally; the flop bound below is the backward passes only."""
+    ds = 9 + 3 * L
+    W, nl, _ = foot_words(L)
+    words = nl + ds + K * (9 * L + 1 + 16) + 2 * (K - 1) * W + (K * ds if want_x else 0) + (K * ds * ds if want_P else 0)
+    f = foot_stage_flops(L)
+    flops = ((K - 1) * f["mean"] if want_x else 0) + (((K - 1) * f["cov"] + f["cov_T"]) if want_P else 0)
+    return 8 * words, flops
+
+
+def foot_main(a, torch, estimator, synth, peaks):
+    """Go1 foot-state handles (leg_odom_type 1), N = 20, ragged VO, warm-up to K = N; x-only, P-only and x+P calls and one
+    k_foot_team tick, per instance count."""
+    N, warm, L = 20, 40, 4
+    res = dict(card=card(), torch_device=torch.cuda.get_device_name(0), N=N, warmup_ticks=warm, calls=a.calls, peaks=peaks,
+               foot_stage_flops=foot_stage_flops(L), ring_words_per_stage=foot_words(L)[0], runs=[])
+    for n in a.foot_n:
+        d = synth.make_stream(n, warm + 2 * a.ticks + 1, vo_jitter=True, device="cuda")
+        vo = [bool(d["vo_flag"][s].any()) for s in range(d["gyro"].shape[0])]
+        est = estimator.BatchedEstimator(estimator.robot_params("go1", ekf_rate=200, N=N, leg_odom_type=1), n, precision="fp64")
+        est.run(0, warm, {k: v[:warm] for k, v in d.items()}, vo[:warm])
+        h = est._hd
+        ds = h.ds
+        x = torch.empty(N, ds, n, dtype=torch.float64, device="cuda")
+        P = torch.empty(N, ds * ds, n, dtype=torch.float64, device="cuda")
+        K = torch.zeros(1, dtype=torch.int32)
+        kp = C.cast(K.data_ptr(), C.POINTER(C.c_int32))
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        r = dict(n=n, T=warm - 1)
+        for name, px, pP in (("x", x, None), ("P", None, P), ("xP", x, P)):
+            call = lambda: h.check(h.L.dekf_get_foot_window(h.h, C.c_void_p(px.data_ptr()) if px is not None else None,
+                                                            C.c_void_p(pP.data_ptr()) if pP is not None else None, kp),
+                                   "dekf_get_foot_window")
+            for _ in range(3):
+                call()
+            torch.cuda.synchronize()
+            e0.record()
+            for _ in range(a.calls):
+                call()
+            e1.record()
+            torch.cuda.synchronize()
+            ms = e0.elapsed_time(e1) / a.calls
+            Kv = int(K.item())
+            by, fl = foot_algorithmic(L, Kv, px is not None, pP is not None)
+            t_bw = by * n / (peaks["copy_gbs"] * 1e9) * 1e3
+            t_fl = fl * n / (peaks["fp64_tflops"] * 1e12) * 1e3
+            r[name] = dict(K=Kv, ms_per_call=ms, bytes_per_instance=by, backward_double_flops_per_instance=fl, hbm_bound_ms=t_bw,
+                           flop_bound_ms=t_fl, bound="hbm" if t_bw >= t_fl else "fma", roof_fraction=max(t_bw, t_fl) / ms)
+        ticks = []
+        for j in range(a.ticks):   # k_foot_team tick (the whole step) in the same process, for scale
+            s = warm + j
+            store = estimator.robot_store.from_stream(d, s)
+            e0.record()
+            est.step(s, store)
+            e1.record()
+            torch.cuda.synchronize()
+            ticks.append(e0.elapsed_time(e1))
+        r["tick_ms_median"] = sorted(ticks)[len(ticks) // 2]
+        r["x_over_tick"] = r["x"]["ms_per_call"] / r["tick_ms_median"]
+        r["device_bytes"] = est.device_bytes()
+        print(json.dumps(r), flush=True)
+        res["runs"].append(r)
+        est.close()
+        del est, x, P, d
+        torch.cuda.empty_cache()
+    res["card_after"] = card()
+    return res
+
+
 def card():
     try:
         q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
@@ -75,6 +168,8 @@ def main():
     ap.add_argument("--n", type=int, default=65536)
     ap.add_argument("--calls", type=int, default=200)
     ap.add_argument("--ticks", type=int, default=40)
+    ap.add_argument("--foot", action="store_true", help="foot-state handles (dekf_get_foot_window) instead of the 9-state getters")
+    ap.add_argument("--foot-n", type=int, nargs="+", default=[16384, 65536])
     a = ap.parse_args()
     import torch
     from decentralized_ekf_mhe_b200 import build, estimator, synth
@@ -82,6 +177,13 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("window_probe needs a CUDA device")
     peaks = estimator.measure_peaks(0)
+    if a.foot:
+        res = foot_main(a, torch, estimator, synth, peaks)
+        os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+        with open(a.out, "w") as f:
+            json.dump(res, f, indent=1)
+        print("card:", res["card"])
+        return
     N, n, warm = 20, a.n, 64
     res = dict(card=card(), torch_device=torch.cuda.get_device_name(0), n=n, N=N, warmup_ticks=warm, calls=a.calls, peaks=peaks,
                flops_per_stage=FLOPS, cov_flops_per_stage=FLOPS_COV, runs=[])
