@@ -6,7 +6,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libdekf_b200.so")
 SOURCES = ["dekf_api.cu"]
-DEPS = ["dekf_api.cu", "solve_tma.cuh", "box_solve.cuh", "box_team.cuh", "foot_team.cuh", "foot_window.cuh", "footstate.cuh", "estimator_core.cuh", "smallmat.cuh", "kinematics.cuh", "host_setup.hpp"]
+DEPS = ["dekf_api.cu", "solve_tma.cuh", "box_solve.cuh", "box_team.cuh", "foot_team.cuh", "foot_window.cuh", "box_window.cuh", "footstate.cuh", "estimator_core.cuh", "smallmat.cuh", "kinematics.cuh", "host_setup.hpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-shared",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 

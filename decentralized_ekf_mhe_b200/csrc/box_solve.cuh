@@ -53,6 +53,9 @@ struct BoxBuffers {
   int32_t *nactive;  // [ns] active bounds of the last solve
   uint32_t *act32;   // [NW][ns]  general bounds only: bits 0-8 lower bound active on component a, bits 9-17 upper bound
   const double *V;   // [81] W^-1 of the row basis (general linear rows only, else nullptr)
+  // [ns] how the last solve ended, for dekf_get_constrained_window: 0 converged, 1 iteration cap (x = the last minimiser),
+  // 2 iteration cap inside the finite method (x = its feasible iterate, slot 135).  Null in builds that do not export the window.
+  uint8_t *capped = nullptr;
 };
 
 // Active-set encodings.  GEN = false: the velocity box (uint8 masks, components 3..5 -- the layout k_box_team shares);
@@ -271,6 +274,13 @@ DEKF_HD void box_stage_rows(const BoxConst &bc, const BoxStage &s, const double 
   }
   box_congruence(V, Ds);
   box_tvec(V, rs);
+}
+
+// component a of x = V y (general linear rows: back from the row basis; x_T and the exported window use this one loop)
+DEKF_HD double box_row_V(const double *V, const double *y, int a) {
+  double v = 0.0;
+  for (int k = 0; k < 9; ++k) v += V[a * 9 + k] * y[k];
+  return v;
 }
 
 // Constrained solve over the window states k0 .. Tk (K = Tk - k0 + 1 <= N) with the Gaussian prior
@@ -685,15 +695,12 @@ DEKF_HD int box_solve(const BoxConst &bc, const Dims &dm, const Buffers<T> &b, c
   }
   if (rows) {  // x_T = V y_T
     double xv[9];
-    for (int a = 0; a < 9; ++a) {
-      double v = 0.0;
-      for (int k = 0; k < 9; ++k) v += Vm[a * 9 + k] * xT[k];
-      xv[a] = v;
-    }
+    for (int a = 0; a < 9; ++a) xv[a] = box_row_V(Vm, xT, a);
     for (int a = 0; a < 9; ++a) xT[a] = xv[a];
   }
   bb.iters[i] = iters;
   bb.nactive[i] = nact;
+  if (bb.capped != nullptr) bb.capped[i] = (status & ST_QP_MAXITER) ? (GEN && have_xc ? 2 : 1) : 0;
   return status;
 }
 

@@ -16,6 +16,7 @@
 #include "box_team.cuh"
 #include "foot_team.cuh"
 #include "foot_window.cuh"
+#include "box_window.cuh"
 
 namespace dekf {
 
@@ -200,6 +201,7 @@ __global__ void __launch_bounds__(kTeamBlock, DEKF_MINB_BOXTEAM) k_box_team(cons
     }
   }
   if (valid && r == 0) {
+    if (Tk >= 1) bb.capped[i] = (st & ST_QP_MAXITER) ? 1 : 0;  // only box_team_solve sets ST_QP_MAXITER in st
     st |= tick_status(dm, b, Tk, i);
     tick_status(dm, b, Tk, i) = st;
     if (status_out != nullptr) status_out[i] = st;
@@ -255,6 +257,22 @@ void launch_foot_window(const FootConst &fc, const Dims &dm, const Buffers<doubl
     k_foot_window<L, true, false><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P);
   else
     k_foot_window<L, false, true><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P);
+}
+// window of a state-constrained handle (dekf_get_constrained_window, box_window.cuh): 9 lanes per instance, 3 instances per
+// warp as in k_box_team; SOA: the serial solve's scratch [N][BOX_FAC][ns], else the team solve's [ns][N][BOX_TFAC]
+template <bool SOA>
+__global__ void __launch_bounds__(kTeamBlock) k_box_window(const BoxConst bc, const Dims dm, const BoxBuffers bb, const double *fac,
+                                                           int Tk, double *x, double *P, uint32_t *act) {
+  __shared__ double sh[kTeamBlock / 32 * 4][BW_TEAM_WORDS];  // per team (3 + the idle lanes' slot per warp)
+  const int lane = threadIdx.x & 31;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int team = lane / 9;
+  const int r = lane - 9 * team;
+  int i = warp * kTeamsPerWarp + team;
+  const bool valid = team < kTeamsPerWarp && i < dm.n;
+  if (i > dm.n - 1) i = dm.n - 1;  // idle teams shadow a real instance (loads only)
+  const BwLayout<SOA> lay = {fac, (size_t)dm.ns, dm.N};
+  box_window_team<SOA>(bc, dm, bb, lay, Tk, i, valid, r, sh[(threadIdx.x >> 5) * 4 + team], x, P, act);
 }
 // arrival cost of the foot-state model: (M_p, n_p) as the reference holds them (MheSrb.hpp:86-87)
 __global__ void k_get_arrival_foot(const Dims dm, const FootBuffers fb, int ds, double *Mout, double *nout) {
@@ -634,7 +652,7 @@ struct dekf_handle {
   Buffers<double> b64;
   Buffers<float> b32;
   BoxConst bc;
-  BoxBuffers bb = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  BoxBuffers bb = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   double *row_V = nullptr;  // device copy of W^-1 (dekf_add_state_rows)
   BoxTeamBuffers tb = {nullptr, nullptr};
   bool box_team = true;           // team form of the constrained solve (DEKF_BOX_SERIAL=1 selects one thread per instance)
@@ -1176,7 +1194,8 @@ int dekf_create(const dekf_config *cfg, dekf_handle **out) {
     if ((ce = cudaMalloc((void **)&h->bb.act, act)) != cudaSuccess) return bail(DEKF_ENOMEM, "cudaMalloc", ce);
     if ((ce = cudaMalloc((void **)&h->bb.iters, ns * sizeof(int32_t))) != cudaSuccess) return bail(DEKF_ENOMEM, "cudaMalloc", ce);
     if ((ce = cudaMalloc((void **)&h->bb.nactive, ns * sizeof(int32_t))) != cudaSuccess) return bail(DEKF_ENOMEM, "cudaMalloc", ce);
-    h->extra_bytes += fac + act + 2 * ns * sizeof(int32_t);
+    if ((ce = cudaMalloc((void **)&h->bb.capped, ns)) != cudaSuccess) return bail(DEKF_ENOMEM, "cudaMalloc", ce);
+    h->extra_bytes += fac + act + 2 * ns * sizeof(int32_t) + ns;
     if (const char *e = std::getenv("DEKF_BOX_SERIAL")) h->box_team = h->box_team && std::atoi(e) == 0;
     if (h->box_team) {
       const size_t tfac = (size_t)h->dm.N * BOX_TFAC * ns * sizeof(double);
@@ -1228,6 +1247,7 @@ int dekf_destroy(dekf_handle *h) {
   cudaFree(h->bb.act32);
   cudaFree(h->bb.iters);
   cudaFree(h->bb.nactive);
+  cudaFree(h->bb.capped);
   cudaFree(h->row_V);
   free_stage_set(h->stage[0]);
   free_stage_set(h->stage[1]);
@@ -1295,6 +1315,7 @@ int dekf_reset(dekf_handle *h) {
     if (h->bb.act32) CK(cudaMemsetAsync(h->bb.act32, 0, (size_t)h->dm.NW * h->dm.ns * sizeof(uint32_t), h->stream));
     CK(cudaMemsetAsync(h->bb.iters, 0, (size_t)h->dm.ns * sizeof(int32_t), h->stream));
     CK(cudaMemsetAsync(h->bb.nactive, 0, (size_t)h->dm.ns * sizeof(int32_t), h->stream));
+    CK(cudaMemsetAsync(h->bb.capped, 0, (size_t)h->dm.ns, h->stream));
   }
   if (h->f32)
     k_init_state<float><<<grid_for(h->dm.n), kBlock, 0, h->stream>>>(h->ec32, h->mc32, h->dm, h->b32);
@@ -2411,14 +2432,37 @@ int dekf_get_foot_window(dekf_handle *h, double *x, double *P, int32_t *len) {
   return DEKF_OK;
 }
 
+int dekf_get_constrained_window(dekf_handle *h, double *x, double *P, uint32_t *active, int32_t *len) {
+  if (!h) return DEKF_EINVAL;
+  if (!x && !P && !active) return fail(h, DEKF_EINVAL, "dekf_get_constrained_window: x, P and active are all null");
+  if (!h->bc.enable)
+    return fail(h, DEKF_EINVAL, "dekf_get_constrained_window: handle without state constraints; use dekf_get_window / dekf_get_window_cov");
+  if (h->next_T < 2) return fail(h, DEKF_ESTATE, "dekf_get_constrained_window: needs a completed update(T >= 1)");
+  CK(cudaSetDevice(h->cfg.device));
+  const int Tk = h->next_T - 1, N = h->dm.N;
+  const int warps = (h->dm.n + kTeamsPerWarp - 1) / kTeamsPerWarp, wpb = kTeamBlock / 32;
+  const dim3 grid((warps + wpb - 1) / wpb);
+  // dekf_run joins its internal streams into h->stream before returning, so this launch is ordered after every tick
+  if (h->box_team)
+    k_box_window<false><<<grid, kTeamBlock, 0, h->stream>>>(h->bc, h->dm, h->bb, h->tb.fac, Tk, x, P, active);
+  else
+    k_box_window<true><<<grid, kTeamBlock, 0, h->stream>>>(h->bc, h->dm, h->bb, h->bb.fac, Tk, x, P, active);
+  h->launches++;
+  CK(cudaGetLastError());
+  if (len) *len = Tk + 1 < N ? Tk + 1 : N;
+  return DEKF_OK;
+}
+
 int dekf_get_host(dekf_handle *h, int32_t what, void *host_out) {
   if (!h || !host_out) return fail(h, DEKF_EINVAL, "dekf_get_host: null argument");
   CK(cudaSetDevice(h->cfg.device));
   const size_t n = (size_t)h->dm.n;
   const size_t dsz = (size_t)h->ds;
-  const size_t rows[13] = {9, 3, dsz * dsz, dsz, 16, 1, dsz * dsz, dsz, 0, 9 * (size_t)h->dm.N, 81 * (size_t)h->dm.N,
-                           dsz * (size_t)h->dm.N, dsz * dsz * (size_t)h->dm.N};
-  if (what < 0 || what > DEKF_GET_FOOT_WINDOW_P) return fail(h, DEKF_EINVAL, "dekf_get_host: unknown selector");
+  // DEKF_GET_BOX_WINDOW_ACTIVE: [N][n] uint32, half a double row each
+  const size_t rows[16] = {9, 3, dsz * dsz, dsz, 16, 1, dsz * dsz, dsz, 0, 9 * (size_t)h->dm.N, 81 * (size_t)h->dm.N,
+                           dsz * (size_t)h->dm.N, dsz * dsz * (size_t)h->dm.N, 9 * (size_t)h->dm.N, 81 * (size_t)h->dm.N,
+                           ((size_t)h->dm.N + 1) / 2};
+  if (what < 0 || what > DEKF_GET_BOX_WINDOW_ACTIVE) return fail(h, DEKF_EINVAL, "dekf_get_host: unknown selector");
   // one scratch for the life of the handle (the 200 Hz node shells call this every tick)
   size_t need = (dsz * dsz + dsz + 6 * (size_t)h->nl) * n * sizeof(double);
   if (what == DEKF_GET_WINDOW_X && need < rows[DEKF_GET_WINDOW_X] * n * sizeof(double)) need = rows[DEKF_GET_WINDOW_X] * n * sizeof(double);
@@ -2498,6 +2542,24 @@ int dekf_get_host(dekf_handle *h, int32_t what, void *host_out) {
       bytes = (size_t)K * dsz * dsz * n * sizeof(double);
       break;
     }
+    case DEKF_GET_BOX_WINDOW_X: {
+      int32_t K = 0;
+      rc = dekf_get_constrained_window(h, d, nullptr, nullptr, &K);
+      bytes = (size_t)K * 9 * n * sizeof(double);
+      break;
+    }
+    case DEKF_GET_BOX_WINDOW_P: {
+      int32_t K = 0;
+      rc = dekf_get_constrained_window(h, nullptr, d, nullptr, &K);
+      bytes = (size_t)K * 81 * n * sizeof(double);
+      break;
+    }
+    case DEKF_GET_BOX_WINDOW_ACTIVE: {
+      int32_t K = 0;
+      rc = dekf_get_constrained_window(h, nullptr, nullptr, (uint32_t *)d, &K);
+      bytes = (size_t)K * n * sizeof(uint32_t);
+      break;
+    }
     default:
       rc = dekf_get_window_vo_count(h, (int32_t *)d);
       bytes = n * sizeof(int32_t);
@@ -2524,7 +2586,8 @@ int dekf_add_state_rows(dekf_handle *h, int32_t count, const double *a, const do
     CK(cudaMalloc((void **)&h->bb.act, act));
     CK(cudaMalloc((void **)&h->bb.iters, ns * sizeof(int32_t)));
     CK(cudaMalloc((void **)&h->bb.nactive, ns * sizeof(int32_t)));
-    h->extra_bytes += fac + act + 2 * ns * sizeof(int32_t);
+    CK(cudaMalloc((void **)&h->bb.capped, ns));
+    h->extra_bytes += fac + act + 2 * ns * sizeof(int32_t) + ns;
   }
   if (!h->bb.act32) {
     CK(cudaMalloc((void **)&h->bb.act32, act * sizeof(uint32_t)));
@@ -2536,6 +2599,7 @@ int dekf_add_state_rows(dekf_handle *h, int32_t count, const double *a, const do
   CK(cudaMemsetAsync(h->bb.act32, 0, act * sizeof(uint32_t), h->stream));
   CK(cudaMemsetAsync(h->bb.iters, 0, ns * sizeof(int32_t), h->stream));
   CK(cudaMemsetAsync(h->bb.nactive, 0, ns * sizeof(int32_t), h->stream));
+  CK(cudaMemsetAsync(h->bb.capped, 0, ns, h->stream));
   CK(cudaStreamSynchronize(h->stream));  // V is a stack array
   h->bb.V = h->row_V;
   if (!h->bc.enable) h->bc = make_box_const(h->cfg);  // model constants of the information form (dt, noise weights, lever arm)

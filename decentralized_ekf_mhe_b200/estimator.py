@@ -10,6 +10,8 @@ Reference (C++; /root/reference/src)                          here (Python over 
   MHEproblem::solution  MheSrb.hpp:58-112 (state blocks)       DecentralizedEstimation.mhe_qp_.x_window(), BatchedEstimator.window()
   (posterior covariance of each state block; not in the reference)  DecentralizedEstimation.mhe_qp_.P_window(), BatchedEstimator.window_cov()
   (leg_odom_type 1: the same with 9 + 3L rows per state block)    the same methods, through dekf_get_foot_window
+  (state-constrained handles: the same, with the active bounds)   the same methods, through dekf_get_constrained_window;
+                                                                  BatchedEstimator.window_active(), mhe_qp_.active_window()
 
 torch is used for device memory and streams only; all arithmetic happens in libdekf_b200.so
 (sm_100a kernels).  Nothing here falls back to PyTorch or the CPU: a missing library or device raises.
@@ -178,11 +180,31 @@ def _foot_window(h, want_x, want_P):
     return (x[:K.value] if want_x else None), (P[:K.value] if want_P else None)
 
 
+def _constrained(h):
+    return bool(h.cfg.v_box_enable or h.cfg.x_box_mask or getattr(h, "has_rows", False))
+
+
+def _box_window(h, want_x, want_P, want_act):
+    """Window of a state-constrained handle: ([K][9][n], [K][9][9][n] float64, [K][n] int64 active-set words) on the device
+    (dekf_get_constrained_window)."""
+    N = int(h.cfg.N)
+    x = torch.empty(N, 9, h.n, dtype=torch.float64, device=h.device) if want_x else None
+    P = torch.empty(N, 9, 9, h.n, dtype=torch.float64, device=h.device) if want_P else None
+    a = torch.empty(N, h.n, dtype=torch.int32, device=h.device) if want_act else None
+    K = C.c_int32()
+    h.check(h.L.dekf_get_constrained_window(h.h, _ptr(x), _ptr(P), _ptr(a), C.byref(K)), "dekf_get_constrained_window")
+    k = K.value
+    return (x[:k] if want_x else None), (P[:k] if want_P else None), (a[:k].to(torch.int64) & 0xFFFFFFFF if want_act else None)
+
+
 def _window(h):
     """Smoothed window of the last update(T): [K][9][n] float64 on the device (dekf_get_window); foot-state handles
-    (leg_odom_type 1): [K][ds][n] (dekf_get_foot_window)."""
+    (leg_odom_type 1): [K][ds][n] (dekf_get_foot_window); state-constrained handles: the window QP's optimum
+    (dekf_get_constrained_window)."""
     if h.cfg.leg_odom_type == 1:
         return _foot_window(h, True, False)[0]
+    if _constrained(h):
+        return _box_window(h, True, False, False)[0]
     w = torch.empty(int(h.cfg.N), 9, h.n, dtype=torch.float64, device=h.device)
     K = C.c_int32()
     h.check(h.L.dekf_get_window(h.h, _ptr(w), C.byref(K)), "dekf_get_window")
@@ -194,6 +216,8 @@ def _window_cov(h):
     handles (leg_odom_type 1): [K][ds][ds][n] (dekf_get_foot_window)."""
     if h.cfg.leg_odom_type == 1:
         return _foot_window(h, False, True)[1]
+    if _constrained(h):
+        return _box_window(h, False, True, False)[1]
     P = torch.empty(int(h.cfg.N), 9, 9, h.n, dtype=torch.float64, device=h.device)
     K = C.c_int32()
     h.check(h.L.dekf_get_window_cov(h.h, _ptr(P), C.byref(K)), "dekf_get_window_cov")
@@ -235,6 +259,11 @@ class _MheQpView:
         """Posterior covariance of every state of the same window: [K][9][9][n], block j = stage T-K+1+j, over (p_s, v_s,
         accel bias), exactly symmetric; block K-1 is the filtered covariance of x_T."""
         return _window_cov(self._o._hd)
+
+    def active_window(self):
+        """Active bounds of every state of the same window of a state-constrained handle: [K][n] int64, bit a = lower bound of
+        row a active, bit 9 + a = upper bound (dekf_get_constrained_window)."""
+        return _box_window(self._o._hd, False, False, True)[2]
 
 
 class DecentralizedEstimation:
@@ -435,6 +464,12 @@ class BatchedEstimator:
         over (p_s, v_s, accel bias), exactly symmetric; block K-1 is the filtered covariance of x_T.  Stream-ordered."""
         return _window_cov(self._hd)
 
+    def window_active(self):
+        """Active bounds of every state of the same window of a state-constrained handle (v_box_enable, x_box_mask,
+        add_state_rows): [K][n] int64, bit a = lower bound of row a active, bit 9 + a = upper bound; rows are the state
+        components, or the add_state_rows rows in order followed by the config's component bounds.  Stream-ordered."""
+        return _box_window(self._hd, False, False, True)[2]
+
     def step(self, T, store):
         h = self._hd
         inp = h.inputs(store)
@@ -556,6 +591,7 @@ class BatchedEstimator:
         dp = C.POINTER(C.c_double)
         h.check(h.L.dekf_add_state_rows(h.h, a.shape[0], a.ctypes.data_as(dp), lb.ctypes.data_as(dp), ub.ctypes.data_as(dp)),
                 "dekf_add_state_rows")
+        h.has_rows = True
 
     def qp_info(self):
         """(factorisations, active bounds) [n] int32 of the last state-constrained solve (params.v_box_enable)."""

@@ -29,6 +29,7 @@
  *                               MheSrb.cpp:715-723)
  *   dekf_get_window_cov         posterior covariance of each state of MHEproblem::solution (not exported by the reference)
  *   dekf_get_foot_window        MHEproblem::solution and its covariances for leg_odom_type 1 (9 + 3 num_legs rows per state)
+ *   dekf_get_constrained_window MHEproblem::solution, its covariances and active bounds with addConstraints rows (MheSrb.cpp:58-68)
  *   dekf_get_p_vo               DecentralizedEstimation::p_vo_accmulate_   DecentralEst.hpp:280
  *   dekf_reset                  DecentralizedEstimation::reset()   DecentralEst.hpp:103
  *
@@ -274,6 +275,19 @@ int dekf_get_window_cov(dekf_handle *h, double *P, int32_t *len);
  * first use and counted in dekf_device_bytes.  DEKF_EINVAL for null x and P, est_type 1 and leg_odom_type 0 handles (those
  * use dekf_get_window / dekf_get_window_cov); DEKF_ESTATE before the first update(T >= 1) and after dekf_reset. */
 int dekf_get_foot_window(dekf_handle *h, double *x, double *P, int32_t *len);
+/* Window of a state-constrained handle (v_box_enable, x_box_mask or dekf_add_state_rows; est_type 0, leg_odom_type 0) after
+ * the last update(T): for every state of the window QP (with its inequality rows) the optimum x (p_s, v_s, accel bias; on
+ * rows handles V y), its 9x9 posterior covariance P -- the x_k block of the inverse KKT matrix with the equality rows and the
+ * bounds active at the optimum as equalities, scaling M_p = P^-1, row-major, exactly symmetric, zero rows and columns for a
+ * component fixed at a bound (rows handles: a_i P = 0 for every active row i) -- and the active set: bit a = lower bound of
+ * row a active, bit 9 + a = upper bound (rows a = the components 0..8, or on dekf_add_state_rows handles the rows of that
+ * call in order followed by the config's component bounds in ascending component order).  x receives [K][9][n], P [K][81][n],
+ * active [K][n] (device pointers, stream-ordered; any may be NULL, not all three), row / block j = stage T-K+1+j,
+ * K = min(T+1, N); row K-1 of x equals dekf_outputs.x of that update.  An instance whose last solve hit the iteration cap
+ * (DEKF_ST_QP_MAXITER) returns the iterate the step reported in x, all-NaN P blocks and the active set as it stands.
+ * *len (host, may be NULL) receives K.  DEKF_EINVAL for all-null outputs and for handles without state constraints (those
+ * use dekf_get_window / dekf_get_window_cov); DEKF_ESTATE before the first update(T >= 1) and after dekf_reset. */
+int dekf_get_constrained_window(dekf_handle *h, double *x, double *P, uint32_t *active, int32_t *len);
 /* Host-pointer getter for callers without a CUDA runtime of their own (the C++ facade, a ROS node): `what` selects one
  * of the arrays above, `host_out` receives it (same [rows][n] layout, double; int32 for DEKF_GET_VO_COUNT).
  * Synchronises the handle's stream. */
@@ -291,7 +305,10 @@ enum {
   DEKF_GET_WINDOW_X = 9,     /* [K * 9][n] smoothed window (dekf_get_window); K <= N, so room for N * 9 rows suffices */
   DEKF_GET_WINDOW_P = 10,    /* [K * 81][n] smoothed covariances (dekf_get_window_cov); room for N * 81 rows suffices */
   DEKF_GET_FOOT_WINDOW_X = 11, /* [K * ds][n] smoothed window of a foot-state handle (dekf_get_foot_window); room for N * ds rows */
-  DEKF_GET_FOOT_WINDOW_P = 12  /* [K * ds * ds][n] its covariances (dekf_get_foot_window); room for N * ds * ds rows */
+  DEKF_GET_FOOT_WINDOW_P = 12, /* [K * ds * ds][n] its covariances (dekf_get_foot_window); room for N * ds * ds rows */
+  DEKF_GET_BOX_WINDOW_X = 13,  /* [K * 9][n] window of a state-constrained handle (dekf_get_constrained_window); room for N * 9 rows */
+  DEKF_GET_BOX_WINDOW_P = 14,  /* [K * 81][n] its covariances (dekf_get_constrained_window); room for N * 81 rows */
+  DEKF_GET_BOX_WINDOW_ACTIVE = 15 /* [K][n] uint32 its active sets (dekf_get_constrained_window); room for N rows */
 };
 int dekf_get_host(dekf_handle *h, int32_t what, void *host_out);
 /* debug taps of the last step (only when cfg.debug_taps != 0): copied into caller DEVICE buffers, any may be NULL.

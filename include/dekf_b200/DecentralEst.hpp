@@ -11,6 +11,8 @@
 //   MHEproblem::solution (state blocks) MheSrb.hpp:58-112                          dekf::DecentralizedEstimation::mhe_qp_.x_window()
 //   (posterior covariance of each state block, not in the reference)               dekf::DecentralizedEstimation::mhe_qp_.P_window()
 //   (both for leg_odom_type 1: 9 + 3 num_legs rows per state block)                 the same, through dekf_get_foot_window
+//   (both with state constraints, and the active bounds)                            the same and mhe_qp_.active_window(),
+//                                                                                   through dekf_get_constrained_window
 //
 // The reference estimates ONE robot and stores Eigen vectors; this facade steps `n_instances` robots per call and stores
 // flat SoA arrays `[rows][n_instances]` (instance fastest).  With n_instances == 1 every array has exactly the layout of the
@@ -298,6 +300,7 @@ class DecentralizedEstimation {
     nl_ = cfg.num_legs;
     nq_ = dekf_num_joints(h_);
     kf_ = cfg.est_type == 1;
+    constrained_ = cfg.v_box_enable || cfg.x_box_mask || !rows_lb_.empty();
     ds_ = dekf_state_dim(h_);
     x_MHE_.assign(kf_ ? 0 : ds_ * (size_t)n_, 0.0);
     v_MHE_b_.assign(kf_ ? 0 : 3 * (size_t)n_, 0.0);
@@ -354,24 +357,36 @@ class DecentralizedEstimation {
     }
     // the state blocks of MHEproblem::solution (MheSrb.hpp:58-112) of the last update(T), T >= 1: the smoothed window
     // [K][ds][n], K = min(T+1, N), row j = stage T-K+1+j, row K-1 == x_MHE_ (dekf_get_window; foot-state handles, ds = 9 + 3L:
-    // dekf_get_foot_window)
+    // dekf_get_foot_window; handles with state constraints: the window QP's optimum, dekf_get_constrained_window)
     std::vector<double> x_window() const {
       const size_t ds = (size_t)o->ds_;
       std::vector<double> w((size_t)o->N_ * ds * o->n_);
-      detail::check(dekf_get_host(o->h_, ds != 9 ? DEKF_GET_FOOT_WINDOW_X : DEKF_GET_WINDOW_X, w.data()), o->h_, "dekf_get_host");
+      const int32_t sel = o->constrained_ ? DEKF_GET_BOX_WINDOW_X : (ds != 9 ? DEKF_GET_FOOT_WINDOW_X : DEKF_GET_WINDOW_X);
+      detail::check(dekf_get_host(o->h_, sel, w.data()), o->h_, "dekf_get_host");
       const int K = o->last_T_ + 1 < o->N_ ? o->last_T_ + 1 : o->N_;
       w.resize((size_t)K * ds * o->n_);
       return w;
     }
-    // posterior covariance of each state of that window (dekf_get_window_cov; foot-state handles: dekf_get_foot_window):
-    // [K][ds * ds][n], block j = stage T-K+1+j, row-major over the state components; block K-1 is the covariance of x_T
+    // posterior covariance of each state of that window (dekf_get_window_cov; foot-state handles: dekf_get_foot_window; handles
+    // with state constraints: active bounds as equalities, dekf_get_constrained_window): [K][ds * ds][n], block j = stage
+    // T-K+1+j, row-major over the state components
     std::vector<double> P_window() const {
       const size_t ds = (size_t)o->ds_;
       std::vector<double> P((size_t)o->N_ * ds * ds * o->n_);
-      detail::check(dekf_get_host(o->h_, ds != 9 ? DEKF_GET_FOOT_WINDOW_P : DEKF_GET_WINDOW_P, P.data()), o->h_, "dekf_get_host");
+      const int32_t sel = o->constrained_ ? DEKF_GET_BOX_WINDOW_P : (ds != 9 ? DEKF_GET_FOOT_WINDOW_P : DEKF_GET_WINDOW_P);
+      detail::check(dekf_get_host(o->h_, sel, P.data()), o->h_, "dekf_get_host");
       const int K = o->last_T_ + 1 < o->N_ ? o->last_T_ + 1 : o->N_;
       P.resize((size_t)K * ds * ds * o->n_);
       return P;
+    }
+    // active bounds of each state of that window (handles with state constraints, dekf_get_constrained_window): [K][n], bit a =
+    // lower bound of row a active, bit 9 + a = upper bound
+    std::vector<uint32_t> active_window() const {
+      std::vector<uint32_t> a((size_t)o->N_ * o->n_);
+      detail::check(dekf_get_host(o->h_, DEKF_GET_BOX_WINDOW_ACTIVE, a.data()), o->h_, "dekf_get_host");
+      const int K = o->last_T_ + 1 < o->N_ ? o->last_T_ + 1 : o->N_;
+      a.resize((size_t)K * o->n_);
+      return a;
     }
   } mhe_qp_{this};
 
@@ -418,6 +433,7 @@ class DecentralizedEstimation {
   int n_ = 0, nl_ = 0, nq_ = 0;
   int N_ = 0, last_T_ = -1;  // horizon, T of the last update (window length of mhe_qp_.x_window())
   bool kf_ = false;
+  bool constrained_ = false;  // v_box_enable, x_box_mask or addStateRows: the window comes from dekf_get_constrained_window
   int ds_ = 9;
 };
 

@@ -1,5 +1,7 @@
 """Cost of the smoothed-window getters (dekf_get_window, and dekf_get_window_cov in the cov_* fields) on a large batch;
-with --foot, of dekf_get_foot_window on Go1 foot-state handles (x-only, P-only, x+P and one step, at each --foot-n).
+with --foot, of dekf_get_foot_window on Go1 foot-state handles (x-only, P-only, x+P and one step, at each --foot-n); with --box,
+of dekf_get_constrained_window on state-constrained handles (PogoX config 4 and Go1 with a velocity box on the team layout, general
+rows on the serial layout).
 
 Go1, N = 20, 65,536 instances, fp64 and fp32 handles, ragged and lock-step VO arrival, both window_solve modes.  Per setup:
 64 warm-up ticks (dekf_run), then the getter timed with CUDA events over --calls calls, then a tick with and without the
@@ -9,6 +11,7 @@ dekf_measure_copy_bw / dekf_measure_fma_peak of the same device, as in bench.py.
 
 usage: python tools/window_probe.py --out profiles/window_probe_b200.json [--n 65536] [--calls 200] [--ticks 40]
        python tools/window_probe.py --foot --out profiles/foot_window_probe_b200.json [--foot-n 16384 65536] [--calls 20]
+       python tools/window_probe.py --box --out profiles/box_window_probe_b200.json [--calls 50] [--ticks 20]
 """
 import argparse
 import ctypes as C
@@ -152,6 +155,97 @@ def foot_main(a, torch, estimator, synth, peaks):
     res["card_after"] = card()
     return res
 
+# covariance pass of dekf_get_constrained_window per stage (double): S_j = L^-T (I + F' S F) L^-1, S_{K-1} = L^-T L^-1, and
+# P = V S V' on rows handles (tests/hostsim/box_window_flopcount.cpp; tests/test_constrained_window.py keeps them equal).  The
+# mean x = V y of rows handles costs 9 x (9 mul + 9 add) = 162 per stage (box_row_V, double only: not in the tally).
+BOX_STAGE_FLOPS = {"cov": 4374, "cov_T": 1458, "rows_vsvt": 2268}
+BOX_MEAN_ROWS_FLOPS = 162
+
+
+def box_algorithmic(K, want_x, want_P, rows, act_bytes):
+    """(bytes, double flops) per instance of one dekf_get_constrained_window call over K states.  Bytes: the capped byte; x: the
+    iterate (9 words) read and written per stage; P: the stage factor (L and F, 126 words) and the active word read, 81 words
+    written per stage."""
+    words = (18 * K if want_x else 0) + (207 * K if want_P else 0)
+    by = 8 * words + 1 + (act_bytes * K if want_P else 0)
+    fl = (BOX_MEAN_ROWS_FLOPS * K if (want_x and rows) else 0)
+    if want_P:
+        fl += (K - 1) * BOX_STAGE_FLOPS["cov"] + BOX_STAGE_FLOPS["cov_T"] + (K * BOX_STAGE_FLOPS["rows_vsvt"] if rows else 0)
+    return by, fl
+
+
+def box_main(a, torch, estimator, synth, peaks):
+    """Constrained handles, N = 20, warm-up to K = N: x-only, P-only and x+P calls against the constrained tick's own time."""
+    import numpy as np
+    N, warm = 20, 40
+    rows = np.zeros((3, 9))
+    rows[0, 3], rows[0, 5] = 1.0, 0.5
+    rows[1, 6], rows[1, 7] = 1.0, -1.0
+    rows[2, 2], rows[2, 8] = 1.0, 0.02
+    cases = [("pogox_vbox_team", "pogox", 16384, dict(v_box_enable=1, v_box_lo=(-0.45, -0.03, -0.015), v_box_hi=(0.55, 0.03, 0.015)), None),
+             ("go1_vbox_team", "go1", 65536, dict(v_box_enable=1, v_box_lo=(-0.3, -0.1, -0.05), v_box_hi=(0.6, 0.1, 0.05)), None),
+             ("pogox_rows_serial", "pogox", 16384, dict(x_box_mask=1 << 4, x_box_lo=(0.0, 0.0, 0.0, 0.0, -0.02, 0.0, 0.0, 0.0, 0.0),
+                                                        x_box_hi=(0.0, 0.0, 0.0, 0.0, 0.02, 0.0, 0.0, 0.0, 0.0)),
+              (rows, np.array([0.47, -0.003, -2e-4]), np.array([0.52, 0.003, 2e-4])))]
+    res = dict(card=card(), torch_device=torch.cuda.get_device_name(0), N=N, warmup_ticks=warm, calls=a.calls, peaks=peaks,
+               box_stage_flops=BOX_STAGE_FLOPS, box_mean_rows_flops=BOX_MEAN_ROWS_FLOPS, runs=[])
+    for name, robot, n, kw, rws in cases:
+        d = synth.make_stream(n, warm + a.ticks + 1, robot=robot, vo_jitter=True, device="cuda")
+        est = estimator.BatchedEstimator(estimator.robot_params(robot, ekf_rate=200, N=N, **kw), n, precision="fp64")
+        if rws is not None:
+            est.add_state_rows(*rws)
+        bind = []
+        for s in range(warm):
+            est.step(s, estimator.robot_store.from_stream(d, s))
+            if s >= 1:
+                bind.append(float((est.window_active()[-1] != 0).double().mean()))
+        h = est._hd
+        x = torch.empty(N, 9, n, dtype=torch.float64, device="cuda")
+        P = torch.empty(N, 81, n, dtype=torch.float64, device="cuda")
+        K = torch.zeros(1, dtype=torch.int32)
+        kp = C.cast(K.data_ptr(), C.POINTER(C.c_int32))
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        r = dict(case=name, robot=robot, n=n, layout="team" if h.cfg.x_box_mask == 0 and rws is None else "serial", T=warm - 1,
+                 steps_with_a_bound_active=float(np.mean([b > 0 for b in bind])), mean_fraction_of_instances_bound=float(np.mean(bind)))
+        for cname, px, pP in (("x", x, None), ("P", None, P), ("xP", x, P)):
+            call = lambda: h.check(h.L.dekf_get_constrained_window(h.h, C.c_void_p(px.data_ptr()) if px is not None else None,
+                                                                   C.c_void_p(pP.data_ptr()) if pP is not None else None, None, kp),
+                                   "dekf_get_constrained_window")
+            for _ in range(3):
+                call()
+            torch.cuda.synchronize()
+            e0.record()
+            for _ in range(a.calls):
+                call()
+            e1.record()
+            torch.cuda.synchronize()
+            ms = e0.elapsed_time(e1) / a.calls
+            Kv = int(K.item())
+            by, fl = box_algorithmic(Kv, px is not None, pP is not None, rws is not None, 4 if h.cfg.x_box_mask or rws is not None else 1)
+            t_bw = by * n / (peaks["copy_gbs"] * 1e9) * 1e3
+            t_fl = fl * n / (peaks["fp64_tflops"] * 1e12) * 1e3
+            r[cname] = dict(K=Kv, ms_per_call=ms, bytes_per_instance=by, double_flops_per_instance=fl, hbm_bound_ms=t_bw,
+                            flop_bound_ms=t_fl, bound="hbm" if t_bw >= t_fl else "fma", roof_fraction=max(t_bw, t_fl) / ms)
+        ticks = []
+        for j in range(a.ticks):   # the constrained tick itself (the whole step), for scale
+            s = warm + j
+            store = estimator.robot_store.from_stream(d, s)
+            e0.record()
+            est.step(s, store)
+            e1.record()
+            torch.cuda.synchronize()
+            ticks.append(e0.elapsed_time(e1))
+        r["tick_ms_median"] = sorted(ticks)[len(ticks) // 2]
+        r["xP_over_tick"] = r["xP"]["ms_per_call"] / r["tick_ms_median"]
+        r["device_bytes"] = est.device_bytes()
+        print(json.dumps(r), flush=True)
+        res["runs"].append(r)
+        est.close()
+        del est, x, P, d
+        torch.cuda.empty_cache()
+    res["card_after"] = card()
+    return res
+
 
 def card():
     try:
@@ -170,6 +264,7 @@ def main():
     ap.add_argument("--ticks", type=int, default=40)
     ap.add_argument("--foot", action="store_true", help="foot-state handles (dekf_get_foot_window) instead of the 9-state getters")
     ap.add_argument("--foot-n", type=int, nargs="+", default=[16384, 65536])
+    ap.add_argument("--box", action="store_true", help="state-constrained handles (dekf_get_constrained_window)")
     a = ap.parse_args()
     import torch
     from decentralized_ekf_mhe_b200 import build, estimator, synth
@@ -177,8 +272,8 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("window_probe needs a CUDA device")
     peaks = estimator.measure_peaks(0)
-    if a.foot:
-        res = foot_main(a, torch, estimator, synth, peaks)
+    if a.foot or a.box:
+        res = (box_main if a.box else foot_main)(a, torch, estimator, synth, peaks)
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
         with open(a.out, "w") as f:
             json.dump(res, f, indent=1)
