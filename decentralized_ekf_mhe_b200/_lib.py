@@ -17,7 +17,7 @@ SYMBOLS = [
     "dekf_destroy", "dekf_reset", "dekf_set_stream", "dekf_get_stream", "dekf_last_error", "dekf_num_joints", "dekf_state_dim",
     "dekf_ekf_step", "dekf_mhe_step", "dekf_step", "dekf_step_host", "dekf_mhe_step_host", "dekf_ekf_step_host",
     "dekf_run", "dekf_run_host", "dekf_run_host_f32", "dekf_run_host_f32io", "dekf_synchronize", "dekf_get_arrival_cost",
-    "dekf_get_arrival_cov", "dekf_get_p_vo", "dekf_get_R_sb", "dekf_get_ekf_cov", "dekf_get_window_vo_count", "dekf_get_window", "dekf_get_window_cov", "dekf_get_foot_window", "dekf_get_constrained_window", "dekf_get_host", "dekf_debug_taps", "dekf_get_qp_info", "dekf_get_resweep_info", "dekf_add_state_rows",
+    "dekf_get_arrival_cov", "dekf_get_p_vo", "dekf_get_R_sb", "dekf_get_ekf_cov", "dekf_get_window_vo_count", "dekf_get_window", "dekf_get_window_cov", "dekf_get_foot_window", "dekf_get_constrained_window", "dekf_get_window_cross_cov", "dekf_get_host", "dekf_debug_taps", "dekf_get_qp_info", "dekf_get_resweep_info", "dekf_add_state_rows",
     "dekf_launch_count", "dekf_device_bytes", "dekf_profile_enable", "dekf_profile_read", "dekf_measure_fma_peak",
     "dekf_measure_copy_bw",
 ]
@@ -89,6 +89,7 @@ def load():
     L.dekf_get_window_cov.argtypes = [hp, C.c_void_p, ip]
     L.dekf_get_foot_window.argtypes = [hp, C.c_void_p, C.c_void_p, ip]
     L.dekf_get_constrained_window.argtypes = [hp, C.c_void_p, C.c_void_p, C.c_void_p, ip]
+    L.dekf_get_window_cross_cov.argtypes = [hp, C.c_void_p, C.c_void_p, ip]
     L.dekf_get_host.argtypes = [hp, C.c_int32, C.c_void_p]
     L.dekf_debug_taps.argtypes = [hp, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.dekf_get_qp_info.argtypes = [hp, C.c_void_p, C.c_void_p]

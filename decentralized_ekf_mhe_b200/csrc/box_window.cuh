@@ -69,17 +69,42 @@ DEKF_HD void bw_cov_col(const S *rec, const S *Sn, int sp, int j, S *g) {
   bw_back<S>(rec, g);
 }
 
-// row r of V Sz (Sz: S with the rows and columns of the fixed coordinates fx zeroed); P(r, c) = bw_dot9(t, row c of V) for
-// c <= r, written to (r, c) and (c, r) from one value
+// column j of the lag-one block C_j = Cov(x_j, x_{j+1}) = -L_j^-T F_j' S_{j+1}, the block (j, j+1) of H^-1 = L^-T L^-1 for
+// L_{j+1,j} = F_j; Sn = S_{j+1} (row stride sp), rows of C over x_j
 template <typename S>
-DEKF_HD void bw_vs_row(const double *V, const S *Sm, int sp, int fx, int r, S *t) {
+DEKF_HD void bw_cross_col(const S *rec, const S *Sn, int sp, int j, S *g) {
+  S w[9];
+#pragma unroll
+  for (int a = 0; a < 9; ++a) w[a] = Sn[a * sp + j];  // S_{j+1} e_j
+#pragma unroll
+  for (int r = 0; r < 9; ++r) {  // F' w
+    S t = S(0.0);
+#pragma unroll
+    for (int a = 0; a < 9; ++a) t = fm<S>(rec[BW_F + a * 9 + r], w[a], t);
+    g[r] = t;
+  }
+  bw_back<S>(rec, g);
+#pragma unroll
+  for (int r = 0; r < 9; ++r) g[r] = -g[r];
+}
+
+// row r of V Sz (Sz: S with the rows of the fixed coordinates fx and the columns of those of fxc zeroed: fx of stage j and
+// fxc of stage j + 1 for the lag-one block C_j)
+template <typename S>
+DEKF_HD void bw_vs_row(const double *V, const S *Sm, int sp, int fx, int fxc, int r, S *t) {
 #pragma unroll
   for (int k = 0; k < 9; ++k) {
     S v = S(0.0);
 #pragma unroll
-    for (int b = 0; b < 9; ++b) v = fm<S>(S(V[r * 9 + b]), (((fx >> b) | (fx >> k)) & 1) ? S(0.0) : Sm[b * sp + k], v);
+    for (int b = 0; b < 9; ++b) v = fm<S>(S(V[r * 9 + b]), (((fx >> b) | (fxc >> k)) & 1) ? S(0.0) : Sm[b * sp + k], v);
     t[k] = v;
   }
+}
+// row r of V Sz for a covariance block (rows and columns of the fixed coordinates fx zeroed); P(r, c) = bw_dot9(t, row c
+// of V) for c <= r, written to (r, c) and (c, r) from one value
+template <typename S>
+DEKF_HD void bw_vs_row(const double *V, const S *Sm, int sp, int fx, int r, S *t) {
+  bw_vs_row<S>(V, Sm, sp, fx, fx, r, t);
 }
 template <typename S>
 DEKF_HD S bw_dot9(const S *t, const double *v) {
@@ -137,10 +162,12 @@ DEKF_HD uint32_t bw_load_active(const BoxConst &bc, const BoxBuffers &bb, const 
 }
 
 // Serial form (host build; the device runs box_window_team with the same per-column functions): window of update(Tk) for
-// instance i.  x [K][9], P [K][81], act [K] at element stride os (any may be null).
+// instance i.  x [K][9], P [K][81], act [K], C [K-1][81] (the lag-one blocks, rows of the components fixed at stage j and
+// columns of those fixed at j+1 zeroed; rows handles: V C_y V' with the same zeroing in y) at element stride os (any may be
+// null).
 template <bool SOA>
 DEKF_HD void box_window_serial(const BoxConst &bc, const Dims &dm, const BoxBuffers &bb, const BwLayout<SOA> &lay, int Tk, int i,
-                               double *x, double *P, uint32_t *act, size_t os) {
+                               double *x, double *P, uint32_t *act, size_t os, double *C = nullptr) {
   const int N = dm.N, K = Tk + 1 < N ? Tk + 1 : N, k0 = Tk - K + 1;
   const int cap = bb.capped[i];
   const bool rows = bc.general && bc.nrows > 0;
@@ -154,13 +181,31 @@ DEKF_HD void box_window_serial(const BoxConst &bc, const Dims &dm, const BoxBuff
       for (int a = 0; a < 9; ++a) x[((size_t)j * 9 + a) * os] = rows ? box_row_V(bb.V, y, a) : y[a];
     }
   }
-  if (P == nullptr) return;
-  double rec[BW_REC], Sn[81], Sk[81], t[9];
+  if (P == nullptr && C == nullptr) return;
+  double rec[BW_REC], Sn[81], Sk[81], t[9], Cz[81], g[9];
+  int fxn = 0;  // fixed components of stage j + 1
   for (int j = K - 1; j >= 0; --j) {
     const double *f = lay.stage(j, i);
     for (int e = 0; e < BW_REC; ++e) rec[e] = lay.rec(f, e);
-    bw_cov_stage<double>(rec, j == K - 1 ? nullptr : Sn, Sk);
     const int fx = bw_fixed(bw_load_active(bc, bb, dm, k0 + j, i));
+    if (C != nullptr && j < K - 1) {
+      for (int c = 0; c < 9; ++c) {
+        bw_cross_col<double>(rec, Sn, 9, c, g);
+        for (int r = 0; r < 9; ++r) Cz[r * 9 + c] = g[r];
+      }
+      double *Cj = C + (size_t)j * 81 * os;
+      for (int r = 0; r < 9; ++r) {
+        if (rows) bw_vs_row<double>(bb.V, Cz, 9, fx, fxn, r, t);
+        for (int c = 0; c < 9; ++c)
+          Cj[(size_t)(r * 9 + c) * os] = cap ? NAN
+                                        : rows ? bw_dot9<double>(t, bb.V + c * 9)
+                                               : ((((fx >> r) | (fxn >> c)) & 1) ? 0.0 : Cz[r * 9 + c]);
+      }
+    }
+    bw_cov_stage<double>(rec, j == K - 1 ? nullptr : Sn, Sk);
+    fxn = fx;
+    for (int e = 0; e < 81; ++e) Sn[e] = Sk[e];
+    if (P == nullptr) continue;
     double *Pj = P + (size_t)j * 81 * os;
     for (int r = 0; r < 9; ++r) {
       if (rows) {
@@ -172,7 +217,6 @@ DEKF_HD void box_window_serial(const BoxConst &bc, const Dims &dm, const BoxBuff
     }
     if (cap)
       for (int e = 0; e < 81; ++e) Pj[(size_t)e * os] = NAN;
-    for (int e = 0; e < 81; ++e) Sn[e] = Sk[e];
   }
 }
 
@@ -182,9 +226,11 @@ enum { BW_SP = 9, BW_TEAM_WORDS = BW_REC + 2 * 81 };  // shared memory per team:
 
 // Team form: lane r (0..8) of the team of instance i; valid: the team owns a real instance (stores are predicated on it).
 // sh: the team's BW_TEAM_WORDS doubles of shared memory.  Every lane of the warp runs the same instruction stream.
-template <bool SOA>
+// CROSS: also the lag-one blocks into C [K-1][81] as in box_window_serial (P may then be null); lane r forms column r of
+// C_j from S_{j+1} before the stage overwrites it, and rows handles pass it through the G area to form V C_y V'.
+template <bool SOA, bool CROSS = false>
 __device__ void box_window_team(const BoxConst &bc, const Dims &dm, const BoxBuffers &bb, const BwLayout<SOA> &lay, int Tk, int i,
-                                bool valid, int r, double *sh, double *x, double *P, uint32_t *act) {
+                                bool valid, int r, double *sh, double *x, double *P, uint32_t *act, double *C = nullptr) {
   const int N = dm.N, K = Tk + 1 < N ? Tk + 1 : N, k0 = Tk - K + 1;
   const size_t n = (size_t)dm.n;
   const int cap = bb.capped[i];
@@ -206,15 +252,18 @@ __device__ void box_window_team(const BoxConst &bc, const Dims &dm, const BoxBuf
       if (valid) x[((size_t)j * 9 + r) * n + i] = xr;
     }
   }
-  if (P == nullptr) return;
+  if (!CROSS && P == nullptr) return;
+  const bool wp = !CROSS || P != nullptr;
   double *srec = sh, *sS = sh + BW_REC, *sG = sS + 81;
+  int fxn = 0;  // fixed components of stage j + 1
   for (int j = K - 1; j >= 0; --j) {
     const double *f = lay.stage(j, i);
     __syncwarp();  // every lane is done with the previous record and with G
     for (int e = r; e < BW_REC; e += 9) srec[e] = lay.rec(f, e);
     __syncwarp();
-    double g[9];
-    bw_cov_col<double>(srec, j == K - 1 ? nullptr : sS, BW_SP, r, g);  // column r of G
+    double g[9], cg[9];
+    if (CROSS && j < K - 1) bw_cross_col<double>(srec, sS, BW_SP, r, cg);  // column r of C_j
+    bw_cov_col<double>(srec, j == K - 1 ? nullptr : sS, BW_SP, r, g);     // column r of G
 #pragma unroll
     for (int a = 0; a < 9; ++a) sG[a * BW_SP + r] = g[a];
     __syncwarp();  // every lane has read S_{j+1} and written its column of G
@@ -227,17 +276,38 @@ __device__ void box_window_team(const BoxConst &bc, const Dims &dm, const BoxBuf
     __syncwarp();
     const int fx = bw_fixed(bw_load_active(bc, bb, dm, k0 + j, i));
     double *Pj = P + (size_t)j * 81 * n + i;
-    if (rows) {
+    if (wp && rows) {
       double t[9];
       bw_vs_row<double>(bb.V, sS, BW_SP, fx, r, t);
       for (int c = 0; c <= r; ++c) {
         const double v = bw_dot9<double>(t, bb.V + c * 9);
         if (valid) Pj[(size_t)(r * 9 + c) * n] = Pj[(size_t)(c * 9 + r) * n] = cap ? NAN : v;
       }
-    } else if (valid) {
+    } else if (wp && valid) {
 #pragma unroll
       for (int c = 0; c < 9; ++c)
         Pj[(size_t)(r * 9 + c) * n] = cap ? NAN : ((((fx >> r) | (fx >> c)) & 1) ? 0.0 : sS[r * BW_SP + c]);
+    }
+    if constexpr (CROSS) {
+      if (j < K - 1) {
+        double *Cj = C + (size_t)j * 81 * n + i;
+        if (rows) {  // G is consumed: its area takes C_y
+#pragma unroll
+          for (int a = 0; a < 9; ++a) sG[a * BW_SP + r] = cg[a];
+          __syncwarp();
+          double t[9];
+          bw_vs_row<double>(bb.V, sG, BW_SP, fx, fxn, r, t);
+#pragma unroll
+          for (int c = 0; c < 9; ++c) {
+            const double v = bw_dot9<double>(t, bb.V + c * 9);
+            if (valid) Cj[(size_t)(r * 9 + c) * n] = cap ? NAN : v;
+          }
+        } else if (valid) {
+#pragma unroll
+          for (int a = 0; a < 9; ++a) Cj[(size_t)(a * 9 + r) * n] = cap ? NAN : ((((fx >> a) | (fxn >> r)) & 1) ? 0.0 : cg[a]);
+        }
+      }
+      fxn = fx;
     }
   }
 }

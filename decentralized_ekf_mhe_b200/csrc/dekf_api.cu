@@ -238,31 +238,38 @@ __global__ void __launch_bounds__(kTeamBlock) k_foot_team(const FootConst fc, co
 // smoothed window of the foot-state model (dekf_get_foot_window, foot_window.cuh): one warp per instance, two warps per CTA
 // with the stage record, P_{k+1} and the transpose buffer of each warp in shared memory
 constexpr int kFootWinBlock = 64;
-template <int L, bool WX, bool WP>
+template <int L, bool WX, bool WP, bool WC = false>
 __global__ void __launch_bounds__(kFootWinBlock) k_foot_window(const FootConst fc, const Dims dm, const Buffers<double> b,
-                                                               const FootBuffers fb, double *ring, int Tk, double *xout, double *Pout) {
+                                                               const FootBuffers fb, double *ring, int Tk, double *xout, double *Pout,
+                                                               double *Cout) {
   __shared__ double sh[kFootWinBlock / 32][foot_win_smem_words<L>()];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int i = (int)((size_t)blockIdx.x * (kFootWinBlock / 32) + w);
   if (i >= dm.n) return;  // whole warps only: no block-wide barrier follows
-  foot_window_team<L, WX, WP>(fc, dm, b, fb, ring, Tk, i, lane, sh[w], xout, Pout);
+  foot_window_team<L, WX, WP, WC>(fc, dm, b, fb, ring, Tk, i, lane, sh[w], xout, Pout, Cout);
 }
+// C non-null (dekf_get_window_cross_cov): the lag-one blocks into C and, when P is non-null, the covariances into P (x unused)
 template <int L>
 void launch_foot_window(const FootConst &fc, const Dims &dm, const Buffers<double> &b, const FootBuffers &fb, double *ring, int Tk,
-                        double *x, double *P, cudaStream_t stream) {
+                        double *x, double *P, double *C, cudaStream_t stream) {
   const dim3 grid((dm.n + kFootWinBlock / 32 - 1) / (kFootWinBlock / 32));
-  if (x && P)
-    k_foot_window<L, true, true><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P);
+  if (C && P)
+    k_foot_window<L, false, true, true><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P, C);
+  else if (C)
+    k_foot_window<L, false, false, true><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P, C);
+  else if (x && P)
+    k_foot_window<L, true, true><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P, nullptr);
   else if (x)
-    k_foot_window<L, true, false><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P);
+    k_foot_window<L, true, false><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P, nullptr);
   else
-    k_foot_window<L, false, true><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P);
+    k_foot_window<L, false, true><<<grid, kFootWinBlock, 0, stream>>>(fc, dm, b, fb, ring, Tk, x, P, nullptr);
 }
 // window of a state-constrained handle (dekf_get_constrained_window, box_window.cuh): 9 lanes per instance, 3 instances per
 // warp as in k_box_team; SOA: the serial solve's scratch [N][BOX_FAC][ns], else the team solve's [ns][N][BOX_TFAC]
-template <bool SOA>
+// CROSS (dekf_get_window_cross_cov): the lag-one blocks into C and, when P is non-null, the covariances into P
+template <bool SOA, bool CROSS = false>
 __global__ void __launch_bounds__(kTeamBlock) k_box_window(const BoxConst bc, const Dims dm, const BoxBuffers bb, const double *fac,
-                                                           int Tk, double *x, double *P, uint32_t *act) {
+                                                           int Tk, double *x, double *P, uint32_t *act, double *C) {
   __shared__ double sh[kTeamBlock / 32 * 4][BW_TEAM_WORDS];  // per team (3 + the idle lanes' slot per warp)
   const int lane = threadIdx.x & 31;
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -272,7 +279,7 @@ __global__ void __launch_bounds__(kTeamBlock) k_box_window(const BoxConst bc, co
   const bool valid = team < kTeamsPerWarp && i < dm.n;
   if (i > dm.n - 1) i = dm.n - 1;  // idle teams shadow a real instance (loads only)
   const BwLayout<SOA> lay = {fac, (size_t)dm.ns, dm.N};
-  box_window_team<SOA>(bc, dm, bb, lay, Tk, i, valid, r, sh[(threadIdx.x >> 5) * 4 + team], x, P, act);
+  box_window_team<SOA, CROSS>(bc, dm, bb, lay, Tk, i, valid, r, sh[(threadIdx.x >> 5) * 4 + team], x, P, act, C);
 }
 // arrival cost of the foot-state model: (M_p, n_p) as the reference holds them (MheSrb.hpp:86-87)
 __global__ void k_get_arrival_foot(const Dims dm, const FootBuffers fb, int ds, double *Mout, double *nout) {
@@ -600,14 +607,17 @@ __global__ void __launch_bounds__(kBlock) k_window(const MheConst<T> c, const Mh
 // smoothed covariances of the window (dekf_get_window_cov): one thread per instance like k_window, which already sits at
 // 250-255 registers; the 9x9 gain G and Sigma - P_{k+1}^s of each thread (126 doubles) live in shared memory instead, one
 // column per thread so that a warp's accesses are conflict-free.  One-warp CTAs keep that area within the static limit.
+// CROSS (dekf_get_window_cross_cov): also the lag-one blocks into cout, pout holding pslots blocks (window_cov_backward).
 constexpr int kCovBlock = 32;
-template <typename T, bool FULL>
+template <typename T, bool FULL, bool CROSS = false>
 __global__ void __launch_bounds__(kCovBlock) k_window_cov(const MheConst<T> c, const MheConst<double> c64, const Dims dm,
-                                                          const Buffers<T> b, T *scr, int Tk, double *pout) {
+                                                          const Buffers<T> b, T *scr, int Tk, double *pout, double *cout,
+                                                          int pslots) {
   __shared__ double sh[126 * kCovBlock];
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= dm.n) return;
-  mhe_window_cov<T>(c, c64, dm, b, FULL ? scr : nullptr, Tk, i, pout, (size_t)dm.n, sh + threadIdx.x, kCovBlock);
+  mhe_window_cov<T, CROSS>(c, c64, dm, b, FULL ? scr : nullptr, Tk, i, pout, (size_t)dm.n, sh + threadIdx.x, kCovBlock, cout,
+                           pslots);
 }
 
 }  // namespace dekf
@@ -662,6 +672,7 @@ struct dekf_handle {
   void *ckpt_mem = nullptr;       // incremental window solve: checkpoint ring
   void *win_scr = nullptr;        // dekf_get_window on a full re-sweep handle: filtered states [N][54][ns] (first use)
   double *foot_win_ring = nullptr;  // dekf_get_foot_window: stage factors [N-1][ns][FootWin<L>::W] (first use)
+  double *cross_ring = nullptr;     // dekf_get_window_cross_cov without P on a 9-state handle: P_k^s, P_{k+1}^s [2][81][n]
   int32_t *resweep_mem = nullptr;
   void *slab = nullptr;
   size_t slab_bytes = 0;
@@ -1239,6 +1250,7 @@ int dekf_destroy(dekf_handle *h) {
   cudaFree(h->ckpt_mem);
   cudaFree(h->win_scr);
   cudaFree(h->foot_win_ring);
+  cudaFree(h->cross_ring);
   cudaFree(h->resweep_mem);
   cudaFree(h->bb.fac);
   cudaFree(h->tb.prior);
@@ -2391,13 +2403,13 @@ int dekf_get_window_cov(dekf_handle *h, double *P, int32_t *len) {
   }
   const dim3 grid((h->dm.n + kCovBlock - 1) / kCovBlock);
   if (h->f32 && scr)
-    k_window_cov<float, true><<<grid, kCovBlock, 0, h->stream>>>(h->mc32, h->mc64, h->dm, h->b32, (float *)scr, Tk, P);
+    k_window_cov<float, true><<<grid, kCovBlock, 0, h->stream>>>(h->mc32, h->mc64, h->dm, h->b32, (float *)scr, Tk, P, nullptr, 0);
   else if (h->f32)
-    k_window_cov<float, false><<<grid, kCovBlock, 0, h->stream>>>(h->mc32, h->mc64, h->dm, h->b32, nullptr, Tk, P);
+    k_window_cov<float, false><<<grid, kCovBlock, 0, h->stream>>>(h->mc32, h->mc64, h->dm, h->b32, nullptr, Tk, P, nullptr, 0);
   else if (scr)
-    k_window_cov<double, true><<<grid, kCovBlock, 0, h->stream>>>(h->mc64, h->mc64, h->dm, h->b64, (double *)scr, Tk, P);
+    k_window_cov<double, true><<<grid, kCovBlock, 0, h->stream>>>(h->mc64, h->mc64, h->dm, h->b64, (double *)scr, Tk, P, nullptr, 0);
   else
-    k_window_cov<double, false><<<grid, kCovBlock, 0, h->stream>>>(h->mc64, h->mc64, h->dm, h->b64, nullptr, Tk, P);
+    k_window_cov<double, false><<<grid, kCovBlock, 0, h->stream>>>(h->mc64, h->mc64, h->dm, h->b64, nullptr, Tk, P, nullptr, 0);
   h->launches++;
   CK(cudaGetLastError());
   if (len) *len = Tk + 1 < N ? Tk + 1 : N;
@@ -2421,11 +2433,11 @@ int dekf_get_foot_window(dekf_handle *h, double *x, double *P, int32_t *len) {
   }
   // dekf_run joins its internal streams into h->stream before returning, so this launch is ordered after every tick
   if (h->nl == 4)
-    launch_foot_window<4>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, x, P, h->stream);
+    launch_foot_window<4>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, x, P, nullptr, h->stream);
   else if (h->nl == 2)
-    launch_foot_window<2>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, x, P, h->stream);
+    launch_foot_window<2>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, x, P, nullptr, h->stream);
   else
-    launch_foot_window<1>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, x, P, h->stream);
+    launch_foot_window<1>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, x, P, nullptr, h->stream);
   h->launches++;
   CK(cudaGetLastError());
   if (len) *len = Tk + 1 < N ? Tk + 1 : N;
@@ -2444,9 +2456,73 @@ int dekf_get_constrained_window(dekf_handle *h, double *x, double *P, uint32_t *
   const dim3 grid((warps + wpb - 1) / wpb);
   // dekf_run joins its internal streams into h->stream before returning, so this launch is ordered after every tick
   if (h->box_team)
-    k_box_window<false><<<grid, kTeamBlock, 0, h->stream>>>(h->bc, h->dm, h->bb, h->tb.fac, Tk, x, P, active);
+    k_box_window<false><<<grid, kTeamBlock, 0, h->stream>>>(h->bc, h->dm, h->bb, h->tb.fac, Tk, x, P, active, nullptr);
   else
-    k_box_window<true><<<grid, kTeamBlock, 0, h->stream>>>(h->bc, h->dm, h->bb, h->bb.fac, Tk, x, P, active);
+    k_box_window<true><<<grid, kTeamBlock, 0, h->stream>>>(h->bc, h->dm, h->bb, h->bb.fac, Tk, x, P, active, nullptr);
+  h->launches++;
+  CK(cudaGetLastError());
+  if (len) *len = Tk + 1 < N ? Tk + 1 : N;
+  return DEKF_OK;
+}
+
+int dekf_get_window_cross_cov(dekf_handle *h, double *P, double *C, int32_t *len) {
+  if (!h) return DEKF_EINVAL;
+  if (!C) return fail(h, DEKF_EINVAL, "dekf_get_window_cross_cov: null C");
+  if (h->cfg.est_type != 0) return fail(h, DEKF_EINVAL, "dekf_get_window_cross_cov: est_type 1 (KF) has no window");
+  if (h->next_T < 2) return fail(h, DEKF_ESTATE, "dekf_get_window_cross_cov: needs a completed update(T >= 1)");
+  CK(cudaSetDevice(h->cfg.device));
+  const int Tk = h->next_T - 1, N = h->dm.N;
+  // dekf_run joins its internal streams into h->stream before returning, so these launches are ordered after every tick
+  if (h->bc.enable) {  // state-constrained: the factor the last active-set solve left (box_window.cuh)
+    const int warps = (h->dm.n + kTeamsPerWarp - 1) / kTeamsPerWarp, wpb = kTeamBlock / 32;
+    const dim3 grid((warps + wpb - 1) / wpb);
+    if (h->box_team)
+      k_box_window<false, true><<<grid, kTeamBlock, 0, h->stream>>>(h->bc, h->dm, h->bb, h->tb.fac, Tk, nullptr, P, nullptr, C);
+    else
+      k_box_window<true, true><<<grid, kTeamBlock, 0, h->stream>>>(h->bc, h->dm, h->bb, h->bb.fac, Tk, nullptr, P, nullptr, C);
+  } else if (h->cfg.leg_odom_type == 1) {  // foot states: the ring of dekf_get_foot_window, rewritten by every call
+    if (!h->foot_win_ring) {
+      const int W = h->nl == 4 ? FootWin<4>::W : (h->nl == 2 ? FootWin<2>::W : FootWin<1>::W);
+      const size_t bytes = (size_t)(N > 1 ? N - 1 : 1) * h->dm.ns * W * sizeof(double);
+      CK(cudaMalloc((void **)&h->foot_win_ring, bytes));
+      h->extra_bytes += bytes;
+    }
+    if (h->nl == 4)
+      launch_foot_window<4>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, nullptr, P, C, h->stream);
+    else if (h->nl == 2)
+      launch_foot_window<2>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, nullptr, P, C, h->stream);
+    else
+      launch_foot_window<1>(h->fc, h->dm, h->b64, h->fb, h->foot_win_ring, Tk, nullptr, P, C, h->stream);
+  } else {  // 9-state: the RTS covariance pass reads P_{k+1}^s back from its output, so without P it runs on a two-block ring
+    void *scr = nullptr;
+    if (h->mc64.window_solve == 0) {  // the scratch ring of dekf_get_window
+      if (!h->win_scr) {
+        const size_t bytes = (size_t)N * 54 * h->dm.ns * (h->f32 ? sizeof(float) : sizeof(double));
+        CK(cudaMalloc(&h->win_scr, bytes));
+        h->extra_bytes += bytes;
+      }
+      scr = h->win_scr;
+    }
+    int pslots = N;
+    if (!P) {
+      if (!h->cross_ring) {
+        const size_t bytes = 2 * 81 * (size_t)h->dm.n * sizeof(double);
+        CK(cudaMalloc((void **)&h->cross_ring, bytes));
+        h->extra_bytes += bytes;
+      }
+      P = h->cross_ring;
+      pslots = 2;
+    }
+    const dim3 grid((h->dm.n + kCovBlock - 1) / kCovBlock);
+    if (h->f32 && scr)
+      k_window_cov<float, true, true><<<grid, kCovBlock, 0, h->stream>>>(h->mc32, h->mc64, h->dm, h->b32, (float *)scr, Tk, P, C, pslots);
+    else if (h->f32)
+      k_window_cov<float, false, true><<<grid, kCovBlock, 0, h->stream>>>(h->mc32, h->mc64, h->dm, h->b32, nullptr, Tk, P, C, pslots);
+    else if (scr)
+      k_window_cov<double, true, true><<<grid, kCovBlock, 0, h->stream>>>(h->mc64, h->mc64, h->dm, h->b64, (double *)scr, Tk, P, C, pslots);
+    else
+      k_window_cov<double, false, true><<<grid, kCovBlock, 0, h->stream>>>(h->mc64, h->mc64, h->dm, h->b64, nullptr, Tk, P, C, pslots);
+  }
   h->launches++;
   CK(cudaGetLastError());
   if (len) *len = Tk + 1 < N ? Tk + 1 : N;
@@ -2459,10 +2535,11 @@ int dekf_get_host(dekf_handle *h, int32_t what, void *host_out) {
   const size_t n = (size_t)h->dm.n;
   const size_t dsz = (size_t)h->ds;
   // DEKF_GET_BOX_WINDOW_ACTIVE: [N][n] uint32, half a double row each
-  const size_t rows[16] = {9, 3, dsz * dsz, dsz, 16, 1, dsz * dsz, dsz, 0, 9 * (size_t)h->dm.N, 81 * (size_t)h->dm.N,
+  // DEKF_GET_WINDOW_C: [(N-1) * ds * ds][n], the lag-one blocks only
+  const size_t rows[17] = {9, 3, dsz * dsz, dsz, 16, 1, dsz * dsz, dsz, 0, 9 * (size_t)h->dm.N, 81 * (size_t)h->dm.N,
                            dsz * (size_t)h->dm.N, dsz * dsz * (size_t)h->dm.N, 9 * (size_t)h->dm.N, 81 * (size_t)h->dm.N,
-                           ((size_t)h->dm.N + 1) / 2};
-  if (what < 0 || what > DEKF_GET_BOX_WINDOW_ACTIVE) return fail(h, DEKF_EINVAL, "dekf_get_host: unknown selector");
+                           ((size_t)h->dm.N + 1) / 2, dsz * dsz * (size_t)(h->dm.N > 1 ? h->dm.N - 1 : 1)};
+  if (what < 0 || what > DEKF_GET_WINDOW_C) return fail(h, DEKF_EINVAL, "dekf_get_host: unknown selector");
   // one scratch for the life of the handle (the 200 Hz node shells call this every tick)
   size_t need = (dsz * dsz + dsz + 6 * (size_t)h->nl) * n * sizeof(double);
   if (what == DEKF_GET_WINDOW_X && need < rows[DEKF_GET_WINDOW_X] * n * sizeof(double)) need = rows[DEKF_GET_WINDOW_X] * n * sizeof(double);
@@ -2552,6 +2629,12 @@ int dekf_get_host(dekf_handle *h, int32_t what, void *host_out) {
       int32_t K = 0;
       rc = dekf_get_constrained_window(h, nullptr, d, nullptr, &K);
       bytes = (size_t)K * 81 * n * sizeof(double);
+      break;
+    }
+    case DEKF_GET_WINDOW_C: {
+      int32_t K = 0;
+      rc = dekf_get_window_cross_cov(h, nullptr, d, &K);
+      bytes = (size_t)(K - 1) * dsz * dsz * n * sizeof(double);
       break;
     }
     case DEKF_GET_BOX_WINDOW_ACTIVE: {

@@ -2557,9 +2557,11 @@ DEKF_HD constexpr int cov_slot(int r, int c) {
 // One backward covariance stage: reads P_{k+1}^s at pnext, writes P_k^s at pout (both [81] row-major at stride n_out).  `ck`,
 // `rec` as in window_back_stage.  `sh`: per-thread work area of 126 doubles at stride ss, G (row-major, [81]) then
 // Sigma - P_{k+1}^s (sym9, [45]).  P'_k is parked in the upper triangle of pout between the first and the last phase.
-template <typename D, typename T>
+// CROSS: also the lag-one cross-covariance Cov^s(x_k, x_{k+1}) = G P_{k+1}^s into cout ([81] row-major at stride n_out, rows
+// over x_k): the smoothed x_k given x_{k+1} is x'_k + G (x_{k+1} - mu), so its covariance with x_{k+1} is G P_{k+1}^s.
+template <typename D, typename T, bool CROSS = false>
 DEKF_HD void window_cov_stage(const MheConst<D> &c, const T *ck, const T *rec, size_t ns, const double *pnext, double *pout,
-                              size_t n_out, double *sh, size_t ss) {
+                              size_t n_out, double *sh, size_t ss, double *cout = nullptr) {
   const bool vo = rec[REC_FLAG * ns] != T(0);
   const D dt = c.dt, h = D(0.5) * c.dt * c.dt;
   double *Gs = sh, *Ds = sh + 81 * ss;
@@ -2739,45 +2741,66 @@ DEKF_HD void window_cov_stage(const MheConst<D> &c, const T *ck, const T *rec, s
       pout[(cc * 9 + r) * n_out] = (double)v;
     }
   }
+  if constexpr (CROSS) {
+    // phase 5: C_k = G P_{k+1}^s, one column of P_{k+1}^s in registers at a time, G re-read from the work area
+#pragma unroll 1
+    for (int cc = 0; cc < 9; ++cc) {
+      D p[9];
+#pragma unroll
+      for (int l = 0; l < 9; ++l) p[l] = (D)pnext[(l * 9 + cc) * n_out];
+#pragma unroll
+      for (int r = 0; r < 9; ++r) {
+        D v = (D)Gs[(r * 9) * ss] * p[0];
+#pragma unroll
+        for (int l = 1; l < 9; ++l) v = fm((D)Gs[(r * 9 + l) * ss], p[l], v);
+        cout[(r * 9 + cc) * n_out] = (double)v;
+      }
+    }
+  }
 }
 
 // Backward covariance pass over the filtered states of stages Tk-K+1 .. Tk in `ring` (as window_backward); pout [K][81][n_out].
-template <typename T>
+// CROSS: also the lag-one blocks, cout [K-1][81][n_out] (block j = Cov(x_{Tk-K+1+j}, x_{Tk-K+2+j})), and block j of pout sits
+// at slot j % pslots (pslots >= K: the whole window; 2: a two-block ring for a caller that wants the cross blocks only).
+template <typename T, bool CROSS = false>
 DEKF_HD void window_cov_backward(const MheConst<double> &c64, const Dims &dm, const Buffers<T> &b, const T *ring, int slots, int Tk,
-                                 int i, double *pout, size_t n_out, double *sh, size_t ss) {
+                                 int i, double *pout, size_t n_out, double *sh, size_t ss, double *cout = nullptr, int pslots = 0) {
   const int N = dm.N, K = Tk + 1 < N ? Tk + 1 : N, k0 = Tk - K + 1;
   const size_t ns = (size_t)dm.ns;
+  auto pblk = [&](int j) { return pout + (size_t)(CROSS ? j % pslots : j) * 81 * n_out + i; };
   {
     Cov9<double> P;  // P_T^s = P_T, widened
     Vec9<double> x;
     load_state_as(ring + (size_t)(Tk % slots) * 54 * ns + i, ns, P, x);
-    double *o = pout + (size_t)(Tk - k0) * 81 * n_out + i;
+    double *o = pblk(Tk - k0);
 #pragma unroll
     for (int r = 0; r < 9; ++r)
 #pragma unroll
       for (int cc = 0; cc < 9; ++cc) o[(r * 9 + cc) * n_out] = cov_at(P, r, cc);
   }
   for (int k = Tk - 1; k >= k0; --k) {
-    double *o = pout + (size_t)(k - k0) * 81 * n_out + i;
-    window_cov_stage<double, T>(c64, ring + (size_t)(k % slots) * 54 * ns + i, b.win + (size_t)(k % dm.NW) * REC_SIZE * ns + i, ns,
-                                o + 81 * n_out, o, n_out, sh, ss);
+    double *o = pblk(k - k0);
+    window_cov_stage<double, T, CROSS>(c64, ring + (size_t)(k % slots) * 54 * ns + i,
+                                       b.win + (size_t)(k % dm.NW) * REC_SIZE * ns + i, ns, pblk(k - k0 + 1), o, n_out, sh, ss,
+                                       CROSS ? cout + (size_t)(k - k0) * 81 * n_out + i : nullptr);
   }
 }
 
 // Smoothed covariances of update(Tk) (Tk >= 1) for instance i: pout [K][81][n_out], block j = stage Tk-K+1+j, row-major over
-// (p_s, v_s, accel bias).  Sources of the filtered states as in mhe_window_smooth; sh / ss: see window_cov_stage.
-template <typename T>
+// (p_s, v_s, accel bias).  Sources of the filtered states as in mhe_window_smooth; sh / ss: see window_cov_stage; CROSS,
+// cout, pslots: see window_cov_backward.
+template <typename T, bool CROSS = false>
 DEKF_HD void mhe_window_cov(const MheConst<T> &c, const MheConst<double> &c64, const Dims &dm, const Buffers<T> &b, T *scr, int Tk,
-                            int i, double *pout, size_t n_out, double *sh, size_t ss) {
+                            int i, double *pout, size_t n_out, double *sh, size_t ss, double *cout = nullptr, int pslots = 0) {
   if (scr == nullptr) {
-    window_cov_backward<T>(c64, dm, b, b.ckpt, dm.NW, Tk, i, pout, n_out, sh, ss);
+    window_cov_backward<T, CROSS>(c64, dm, b, b.ckpt, dm.NW, Tk, i, pout, n_out, sh, ss, cout, pslots);
     return;
   }
   window_forward<T>(c, dm, b, Tk, i, scr);
 #if defined(__CUDA_ARCH__)
   asm volatile("" ::: "memory");
 #endif
-  window_cov_backward<T>(c64, dm, b, scr, dm.N, Tk, i, pout, n_out, sh, ss);
+  window_cov_backward<T, CROSS>(c64, dm, b, scr, dm.N, Tk, i, pout, n_out, sh, ss, cout, pslots);
 }
 
 }  // namespace dekf

@@ -4,8 +4,9 @@
 //      step, each stage writing its factors L, Y, y (FootWin<L> layout, footstate.cuh) into a device ring
 //      [N-1][ns][W] -- instance-major within a stage, so that the warp's stores and loads of one stage are coalesced;
 //   2. backward mean pass  x_k = L^-T (y - Y x_{k+1});
-//   3. backward covariance pass  P_k = L^-T (I + Y P_{k+1} Y') L^-1  (only when P is requested), starting from
-//      P_T = L_T^-T L_T^-1 with the factor of M_T that solve() leaves in registers.
+//   3. backward covariance pass  P_k = L^-T (I + Y P_{k+1} Y') L^-1  (only when P or C is requested), starting from
+//      P_T = L_T^-T L_T^-1 with the factor of M_T that solve() leaves in registers; with WC, lane j first forms column j of
+//      the lag-one block C_k = -L^-T Y P_{k+1} (fw_cross_col) from P_{k+1} before the stage overwrites it.
 // Per stage the warp copies the record into shared memory; the backward passes then read it with warp-uniform addresses
 // (broadcasts) or, for row j of Y, consecutive ones.  The mean pass runs redundantly in every lane (no shuffles); in the
 // covariance pass lane j forms column j of G = L^-T (I + Y P Y'), G goes through shared memory to transpose, and lane c
@@ -48,9 +49,11 @@ __device__ __forceinline__ void foot_win_cov_team(const double *srec, double *sP
   __syncwarp();
 }
 
-template <int L, bool WX, bool WP>
+// WX / WP: store the window / its covariances; WC: store the lag-one cross-covariances [K-1][DS * DS] at Cout (the covariance
+// pass then runs whether or not WP is set)
+template <int L, bool WX, bool WP, bool WC = false>
 __device__ void foot_window_team(const FootConst &fc, const Dims &dm, const Buffers<double> &b, const FootBuffers &fb, double *ring,
-                                 int Tk, int i, int lane, double *sh, double *xout, double *Pout) {
+                                 int Tk, int i, int lane, double *sh, double *xout, double *Pout, double *Cout = nullptr) {
   using FW = FootWin<L>;
   constexpr int DS = FW::DS, W = FW::W, SP = DS | 1;
   double *srec = sh, *sP = sh + W, *sG = sP + DS * SP, *sX = sG + DS * SP;
@@ -82,7 +85,7 @@ __device__ void foot_window_team(const FootConst &fc, const Dims &dm, const Buff
       xout[((size_t)(K - 1) * DS + lane) * n + i] = xr;
     }
   }
-  if constexpr (WP) {
+  if constexpr (WP || WC) {
     if (st) {
 #pragma unroll
       for (int c = 0; c < DS; ++c)
@@ -90,7 +93,7 @@ __device__ void foot_window_team(const FootConst &fc, const Dims &dm, const Buff
     }
     __syncwarp();
     foot_win_cov_team<L>(srec, sP, true, sG, lane);
-    if (st) {
+    if (WP && st) {
 #pragma unroll
       for (int c = 0; c < DS; ++c) Pout[(((size_t)(K - 1) * DS + lane) * DS + c) * n + i] = sP[lane * SP + c];
     }
@@ -114,9 +117,17 @@ __device__ void foot_window_team(const FootConst &fc, const Dims &dm, const Buff
         xout[((size_t)j * DS + lane) * n + i] = mine;
       }
     }
-    if constexpr (WP) {
-      foot_win_cov_team<L>(srec, sP, false, sG, lane);
+    if constexpr (WC) {
+      double cg[DS];
+      fw_cross_col<double, L>(srec, sP, SP, st ? lane : DS - 1, cg);  // column `lane` of C_j, from P_{j+1}
       if (st) {
+#pragma unroll
+        for (int r = 0; r < DS; ++r) Cout[(((size_t)j * DS + r) * DS + lane) * n + i] = cg[r];
+      }
+    }
+    if constexpr (WP || WC) {
+      foot_win_cov_team<L>(srec, sP, false, sG, lane);
+      if (WP && st) {
 #pragma unroll
         for (int c = 0; c < DS; ++c) Pout[(((size_t)j * DS + lane) * DS + c) * n + i] = sP[lane * SP + c];
       }

@@ -159,6 +159,24 @@ DEKF_HD void fw_cov_col(const S *rec, const S *P, int sp, int j, S *g) {
   fw_back<S, L>(rec, g);
 }
 
+// column j of the lag-one cross-covariance C_k = Cov(x_k, x_{k+1}) = -L^-T Y P_{k+1} (x_k = L^-T (y - Y x_{k+1})), rows over
+// x_k; P = P_{k+1} (full, row stride sp)
+template <typename S, int L>
+DEKF_HD void fw_cross_col(const S *rec, const S *P, int sp, int j, S *g) {
+  using FW = FootWin<L>;
+  constexpr int DS = FW::DS;
+#pragma unroll
+  for (int r = 0; r < DS; ++r) {  // Y P e_j
+    S t = rec[FW::yi(r, 0)] * P[j];
+#pragma unroll
+    for (int c = 1; c < fw_ce(r); ++c) t += rec[FW::yi(r, c)] * P[c * sp + j];
+    g[r] = t;
+  }
+  fw_back<S, L>(rec, g);
+#pragma unroll
+  for (int r = 0; r < DS; ++r) g[r] = -g[r];
+}
+
 // serial backward covariance stage: Pk = L^-T (I + Y Pn Y') L^-1 = L^-T G' (Pn null: L^-T L^-1), DS x DS row-major; Pk is
 // written from its lower triangle, so every block is exactly symmetric
 template <typename S, int L>
@@ -405,10 +423,10 @@ DEKF_HD int foot_solve(const FootConst &fc, const Dims &dm, const Buffers<T> &b,
 // Tk-K+1 .. Tk.  The forward sweep of foot_solve from the arrival cost written by that update (the prior of x_{Tk-N+1};
 // Prior_0 while Tk < N) records every stage into rec ([K][FootWin<L>::W], the last slot takes L_T); then the backward
 // mean and covariance passes.  x: [K][DS] and P: [K][DS * DS] at element stride os (either may be null).  Row K-1 of x is
-// foot_solve's x_T bit for bit.
+// foot_solve's x_T bit for bit.  C (may be null): the lag-one cross-covariances [K-1][DS * DS] at stride os (fw_cross_col).
 template <typename T, int L>
 DEKF_HD void foot_window_smooth(const FootConst &fc, const Dims &dm, const Buffers<T> &b, const FootBuffers &fb, int Tk, int i,
-                                double *rec, double *x, double *P, size_t os) {
+                                double *rec, double *x, double *P, size_t os, double *C = nullptr) {
   using FW = FootWin<L>;
   constexpr int DS = FW::DS, W = FW::W;
   const size_t ns = (size_t)dm.ns;
@@ -440,9 +458,10 @@ DEKF_HD void foot_window_smooth(const FootConst &fc, const Dims &dm, const Buffe
   double Pn[DS * DS], Pk[DS * DS];
   if (x != nullptr)
     for (int c = 0; c < DS; ++c) x[((size_t)(K - 1) * DS + c) * os] = xv[c];
-  if (P != nullptr) {
+  if (P != nullptr || C != nullptr) {
     fw_cov_stage<double, L>(rT, nullptr, Pn);
-    for (int e = 0; e < DS * DS; ++e) P[((size_t)(K - 1) * DS * DS + e) * os] = Pn[e];
+    if (P != nullptr)
+      for (int e = 0; e < DS * DS; ++e) P[((size_t)(K - 1) * DS * DS + e) * os] = Pn[e];
   }
   for (int j = K - 2; j >= 0; --j) {
     const double *rj = rec + (size_t)j * W;
@@ -451,10 +470,16 @@ DEKF_HD void foot_window_smooth(const FootConst &fc, const Dims &dm, const Buffe
       fw_mean_stage<double, L>(rj, xn, xv);
       for (int c = 0; c < DS; ++c) x[((size_t)j * DS + c) * os] = xv[c];
     }
-    if (P != nullptr) {
+    if (C != nullptr)
+      for (int c = 0; c < DS; ++c) {
+        double cg[DS];
+        fw_cross_col<double, L>(rj, Pn, DS, c, cg);
+        for (int r = 0; r < DS; ++r) C[((size_t)j * DS * DS + r * DS + c) * os] = cg[r];
+      }
+    if (P != nullptr || C != nullptr) {
       fw_cov_stage<double, L>(rj, Pn, Pk);
       for (int e = 0; e < DS * DS; ++e) {
-        P[((size_t)j * DS * DS + e) * os] = Pk[e];
+        if (P != nullptr) P[((size_t)j * DS * DS + e) * os] = Pk[e];
         Pn[e] = Pk[e];
       }
     }

@@ -12,6 +12,8 @@ Reference (C++; /root/reference/src)                          here (Python over 
   (leg_odom_type 1: the same with 9 + 3L rows per state block)    the same methods, through dekf_get_foot_window
   (state-constrained handles: the same, with the active bounds)   the same methods, through dekf_get_constrained_window;
                                                                   BatchedEstimator.window_active(), mhe_qp_.active_window()
+  (lag-one cross-covariances of that window; not in the reference)  DecentralizedEstimation.mhe_qp_.P_window_cross(),
+                                                                  BatchedEstimator.window_cross_cov()
 
 torch is used for device memory and streams only; all arithmetic happens in libdekf_b200.so
 (sm_100a kernels).  Nothing here falls back to PyTorch or the CPU: a missing library or device raises.
@@ -211,6 +213,19 @@ def _window(h):
     return w[:K.value]
 
 
+def _window_cross_cov(h, return_cov):
+    """Lag-one cross-covariances of the window of the last update(T), any est_type 0 handle: [K-1][ds][ds][n] float64 on the
+    device, block j = Cov(x_{T-K+1+j}, x_{T-K+2+j}), rows over the earlier state; with return_cov also the [K][ds][ds][n]
+    diagonal blocks from the same pass, as (P, C) (dekf_get_window_cross_cov)."""
+    N, ds = int(h.cfg.N), h.ds
+    P = torch.empty(N, ds, ds, h.n, dtype=torch.float64, device=h.device) if return_cov else None
+    Cc = torch.empty(max(N - 1, 1), ds, ds, h.n, dtype=torch.float64, device=h.device)
+    K = C.c_int32()
+    h.check(h.L.dekf_get_window_cross_cov(h.h, _ptr(P), _ptr(Cc), C.byref(K)), "dekf_get_window_cross_cov")
+    k = K.value
+    return (P[:k], Cc[:k - 1]) if return_cov else Cc[:k - 1]
+
+
 def _window_cov(h):
     """Smoothed covariances of the last update(T): [K][9][9][n] float64 on the device (dekf_get_window_cov); foot-state
     handles (leg_odom_type 1): [K][ds][ds][n] (dekf_get_foot_window)."""
@@ -264,6 +279,11 @@ class _MheQpView:
         """Active bounds of every state of the same window of a state-constrained handle: [K][n] int64, bit a = lower bound of
         row a active, bit 9 + a = upper bound (dekf_get_constrained_window)."""
         return _box_window(self._o._hd, False, False, True)[2]
+
+    def P_window_cross(self, return_cov=False):
+        """Lag-one cross-covariances of the same window: [K-1][ds][ds][n], block j = Cov(x_{T-K+1+j}, x_{T-K+2+j}), rows over
+        the earlier state, not symmetric; return_cov=True returns (P_window(), C) from one pass (dekf_get_window_cross_cov)."""
+        return _window_cross_cov(self._o._hd, return_cov)
 
 
 class DecentralizedEstimation:
@@ -463,6 +483,13 @@ class BatchedEstimator:
         """Smoothed covariances of the same window: [K][9][9][n] float64 on the device, block j = stage T-K+1+j, row-major
         over (p_s, v_s, accel bias), exactly symmetric; block K-1 is the filtered covariance of x_T.  Stream-ordered."""
         return _window_cov(self._hd)
+
+    def window_cross_cov(self, return_cov=False):
+        """Lag-one cross-covariances of the same window, any est_type 0 handle: [K-1][ds][ds][n] float64 on the device, block
+        j = Cov(x_{T-K+1+j}, x_{T-K+2+j}) with rows over the earlier state (not symmetric); return_cov=True returns
+        (window_cov(), C) from one pass.  With the diagonal blocks they determine the window's whole joint posterior,
+        Cov(x_i, x_j) = C_i P_{i+1}^-1 C_{i+1} ... P_{j-1}^-1 C_{j-1}.  Stream-ordered."""
+        return _window_cross_cov(self._hd, return_cov)
 
     def window_active(self):
         """Active bounds of every state of the same window of a state-constrained handle (v_box_enable, x_box_mask,

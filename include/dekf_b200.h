@@ -30,6 +30,7 @@
  *   dekf_get_window_cov         posterior covariance of each state of MHEproblem::solution (not exported by the reference)
  *   dekf_get_foot_window        MHEproblem::solution and its covariances for leg_odom_type 1 (9 + 3 num_legs rows per state)
  *   dekf_get_constrained_window MHEproblem::solution, its covariances and active bounds with addConstraints rows (MheSrb.cpp:58-68)
+ *   dekf_get_window_cross_cov   lag-one cross-covariances of the states of MHEproblem::solution (not exported by the reference)
  *   dekf_get_p_vo               DecentralizedEstimation::p_vo_accmulate_   DecentralEst.hpp:280
  *   dekf_reset                  DecentralizedEstimation::reset()   DecentralEst.hpp:103
  *
@@ -288,6 +289,20 @@ int dekf_get_foot_window(dekf_handle *h, double *x, double *P, int32_t *len);
  * *len (host, may be NULL) receives K.  DEKF_EINVAL for all-null outputs and for handles without state constraints (those
  * use dekf_get_window / dekf_get_window_cov); DEKF_ESTATE before the first update(T >= 1) and after dekf_reset. */
 int dekf_get_constrained_window(dekf_handle *h, double *x, double *P, uint32_t *active, int32_t *len);
+/* Lag-one cross-covariances of the window of the last update(T) (T >= 1), for every est_type 0 handle (9-state, foot states,
+ * state-constrained).  C receives [K-1][ds*ds][n]: block j is Cov(x_{T-K+1+j}, x_{T-K+2+j}), row-major, with rows over the
+ * components of the EARLIER state and columns over the later one.  Blocks are not symmetric.  ds = 9, or dekf_state_dim(h)
+ * on leg_odom_type 1 handles.  P (may be NULL) receives in the same pass the [K][ds*ds][n] diagonal blocks, bit for bit what
+ * the handle kind's covariance getter returns.  K = min(T+1, N); *len (host, may be NULL) receives K.  The scaling is that of
+ * the covariance getters.  Device pointers, stream-ordered.  State-constrained handles: the bounds active at the optimum are
+ * equalities, so the rows of components fixed at the earlier stage and the columns of those fixed at the later one are 0
+ * (rows handles: a_i C = 0 for a row active at the earlier stage, C a_i' = 0 for one active at the later); an instance whose
+ * last solve hit the iteration cap gets all-NaN blocks.  With the diagonal blocks these determine the whole joint posterior
+ * of the window (it is Gauss-Markov): Cov(x_i, x_j) = C_i P_{i+1}^-1 C_{i+1} ... P_{j-1}^-1 C_{j-1}.  Scratch as in the
+ * kind's getter; a 9-state handle called without P also allocates a [2][81][n] ring on first use, counted in
+ * dekf_device_bytes.  DEKF_EINVAL for a null C and for est_type 1 handles; DEKF_ESTATE before the first update(T >= 1) and
+ * after dekf_reset. */
+int dekf_get_window_cross_cov(dekf_handle *h, double *P, double *C, int32_t *len);
 /* Host-pointer getter for callers without a CUDA runtime of their own (the C++ facade, a ROS node): `what` selects one
  * of the arrays above, `host_out` receives it (same [rows][n] layout, double; int32 for DEKF_GET_VO_COUNT).
  * Synchronises the handle's stream. */
@@ -308,7 +323,9 @@ enum {
   DEKF_GET_FOOT_WINDOW_P = 12, /* [K * ds * ds][n] its covariances (dekf_get_foot_window); room for N * ds * ds rows */
   DEKF_GET_BOX_WINDOW_X = 13,  /* [K * 9][n] window of a state-constrained handle (dekf_get_constrained_window); room for N * 9 rows */
   DEKF_GET_BOX_WINDOW_P = 14,  /* [K * 81][n] its covariances (dekf_get_constrained_window); room for N * 81 rows */
-  DEKF_GET_BOX_WINDOW_ACTIVE = 15 /* [K][n] uint32 its active sets (dekf_get_constrained_window); room for N rows */
+  DEKF_GET_BOX_WINDOW_ACTIVE = 15, /* [K][n] uint32 its active sets (dekf_get_constrained_window); room for N rows */
+  DEKF_GET_WINDOW_C = 16  /* [(K-1) * ds * ds][n] lag-one cross-covariances, any est_type 0 handle (dekf_get_window_cross_cov);
+                           * room for (N-1) * ds * ds rows */
 };
 int dekf_get_host(dekf_handle *h, int32_t what, void *host_out);
 /* debug taps of the last step (only when cfg.debug_taps != 0): copied into caller DEVICE buffers, any may be NULL.

@@ -13,6 +13,8 @@
 //   (both for leg_odom_type 1: 9 + 3 num_legs rows per state block)                 the same, through dekf_get_foot_window
 //   (both with state constraints, and the active bounds)                            the same and mhe_qp_.active_window(),
 //                                                                                   through dekf_get_constrained_window
+//   (lag-one cross-covariances of the state blocks, not in the reference)          mhe_qp_.P_window_cross(),
+//                                                                                   through dekf_get_window_cross_cov
 //
 // The reference estimates ONE robot and stores Eigen vectors; this facade steps `n_instances` robots per call and stores
 // flat SoA arrays `[rows][n_instances]` (instance fastest).  With n_instances == 1 every array has exactly the layout of the
@@ -378,6 +380,16 @@ class DecentralizedEstimation {
       const int K = o->last_T_ + 1 < o->N_ ? o->last_T_ + 1 : o->N_;
       P.resize((size_t)K * ds * ds * o->n_);
       return P;
+    }
+    // lag-one cross-covariances of that window, any est_type 0 handle (dekf_get_window_cross_cov): [(K-1) * ds * ds][n],
+    // block j = Cov(x_{T-K+1+j}, x_{T-K+2+j}), row-major with rows over the earlier state (not symmetric)
+    std::vector<double> P_window_cross() const {
+      const size_t ds = (size_t)o->ds_;
+      std::vector<double> C((size_t)(o->N_ > 1 ? o->N_ - 1 : 1) * ds * ds * o->n_);
+      detail::check(dekf_get_host(o->h_, DEKF_GET_WINDOW_C, C.data()), o->h_, "dekf_get_host");
+      const int K = o->last_T_ + 1 < o->N_ ? o->last_T_ + 1 : o->N_;
+      C.resize((size_t)(K - 1) * ds * ds * o->n_);
+      return C;
     }
     // active bounds of each state of that window (handles with state constraints, dekf_get_constrained_window): [K][n], bit a =
     // lower bound of row a active, bit 9 + a = upper bound

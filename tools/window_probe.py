@@ -1,7 +1,8 @@
 """Cost of the smoothed-window getters (dekf_get_window, and dekf_get_window_cov in the cov_* fields) on a large batch;
 with --foot, of dekf_get_foot_window on Go1 foot-state handles (x-only, P-only, x+P and one step, at each --foot-n); with --box,
 of dekf_get_constrained_window on state-constrained handles (PogoX config 4 and Go1 with a velocity box on the team layout, general
-rows on the serial layout).
+rows on the serial layout); with --cross, of dekf_get_window_cross_cov against the covariance getter of each handle kind (P only,
+C only, P + C on the same handle, alternated in the same process).
 
 Go1, N = 20, 65,536 instances, fp64 and fp32 handles, ragged and lock-step VO arrival, both window_solve modes.  Per setup:
 64 warm-up ticks (dekf_run), then the getter timed with CUDA events over --calls calls, then a tick with and without the
@@ -12,6 +13,7 @@ dekf_measure_copy_bw / dekf_measure_fma_peak of the same device, as in bench.py.
 usage: python tools/window_probe.py --out profiles/window_probe_b200.json [--n 65536] [--calls 200] [--ticks 40]
        python tools/window_probe.py --foot --out profiles/foot_window_probe_b200.json [--foot-n 16384 65536] [--calls 20]
        python tools/window_probe.py --box --out profiles/box_window_probe_b200.json [--calls 50] [--ticks 20]
+       python tools/window_probe.py --cross --out profiles/window_cross_probe_b200.json [--calls 20]
 """
 import argparse
 import ctypes as C
@@ -30,6 +32,10 @@ FLOPS = {"window_back": 1165, "window_back_vo": 2331, "window_fwd": 1100, "windo
 # one backward stage of the covariance getter (dekf_get_window_cov, double arithmetic) without / with a VO row
 # (tests/hostsim/window_cov_flopcount.cpp; tests/test_window_covariance.py keeps them equal)
 FLOPS_COV = {"window_cov": 4786, "window_cov_vo": 6543}
+# what the lag-one cross block of dekf_get_window_cross_cov adds per stage (double): the 9-state pass; the constrained pass and
+# its V C V' on rows handles (tests/hostsim/window_cross_flopcount.cpp, with foot_stage_flops(L)["cross"]; kept equal by
+# tests/test_window_cross_cov.py)
+FLOPS_CROSS = {"window_cross": 1377, "box_cross": 2187, "box_rows_vcvt": 2916}
 
 
 def algorithmic_bytes(N, K, esize, full):
@@ -73,7 +79,9 @@ def foot_stage_flops(L):
     ds = 9 + 3 * L
     ny = 9 * ds + sum(ds - (9 + 3 * ((c - 9) // 3)) for c in range(9, ds))   # nonzeros of Y
     back = ds * ds
-    return {"mean": 2 * ny + back, "cov": ds * (ds * (2 * ds - 1) + 2 * ny + back) + ds * back, "cov_T": 2 * ds * back}
+    # cross: the lag-one block C_k = -L^-T Y P_{k+1} of dekf_get_window_cross_cov, ds columns of Y (P e_c) and a back substitution
+    return {"mean": 2 * ny + back, "cov": ds * (ds * (2 * ds - 1) + 2 * ny + back) + ds * back, "cov_T": 2 * ds * back,
+            "cross": ds * (2 * ny - ds + back)}
 
 
 def foot_words(L):
@@ -247,6 +255,91 @@ def box_main(a, torch, estimator, synth, peaks):
     return res
 
 
+def cross_main(a, torch, estimator, synth, peaks):
+    """dekf_get_window_cross_cov against the P-only getter of each handle kind, N = 20, warm-up to K = N: P only (the kind's
+    covariance getter), C only and P + C, alternated over --rounds rounds of --calls calls each (median per call reported).
+    Bytes and flops: those of the P-only call plus the [K-1][ds*ds] output and the tally's cross flops; the C-only call of a
+    9-state handle still writes its P blocks, to a two-block ring, and is counted as P + C."""
+    N, warm = 20, 40
+    vbox = dict(v_box_enable=1, v_box_lo=(-0.45, -0.03, -0.015), v_box_hi=(0.55, 0.03, 0.015))
+    setups = [(f"go1_{p}_{'incr' if m else 'full'}", "go1", a.n, dict(window_solve=m), p) for p in ("fp64", "fp32") for m in (1, 0)]
+    setups += [(f"go1_foot_{n}", "go1", n, dict(leg_odom_type=1), "fp64") for n in a.foot_n]
+    setups += [("pogox_vbox_team", "pogox", 16384, vbox, "fp64"), ("go1_vbox", "go1", a.n, vbox, "fp64")]
+    res = dict(card=card(), torch_device=torch.cuda.get_device_name(0), N=N, warmup_ticks=warm, calls=a.calls, rounds=a.rounds,
+               peaks=peaks, cov_flops_per_stage=FLOPS_COV, cross_flops_per_stage=FLOPS_CROSS, foot_stage_flops=foot_stage_flops(4),
+               box_stage_flops=BOX_STAGE_FLOPS,
+               runs=[])
+    for name, robot, n, kw, prec in setups:
+        d = synth.make_stream(n, warm, robot=robot, vo_jitter=True, device="cuda")
+        vo = [bool(d["vo_flag"][s].any()) for s in range(warm)]
+        est = estimator.BatchedEstimator(estimator.robot_params(robot, ekf_rate=200, N=N, **kw), n, precision=prec)
+        est.run(0, warm, d, vo)
+        h = est._hd
+        ds = h.ds
+        P = torch.empty(N, ds * ds, n, dtype=torch.float64, device="cuda")
+        Cc = torch.empty(N - 1, ds * ds, n, dtype=torch.float64, device="cuda")
+        K = torch.zeros(1, dtype=torch.int32)
+        kp = C.cast(K.data_ptr(), C.POINTER(C.c_int32))
+        pp, cp = C.c_void_p(P.data_ptr()), C.c_void_p(Cc.data_ptr())
+        if kw.get("v_box_enable"):
+            p_only = lambda: h.check(h.L.dekf_get_constrained_window(h.h, None, pp, None, kp), "dekf_get_constrained_window")
+        elif kw.get("leg_odom_type") == 1:
+            p_only = lambda: h.check(h.L.dekf_get_foot_window(h.h, None, pp, kp), "dekf_get_foot_window")
+        else:
+            p_only = lambda: h.check(h.L.dekf_get_window_cov(h.h, pp, kp), "dekf_get_window_cov")
+        calls = {"P": p_only,
+                 "C": lambda: h.check(h.L.dekf_get_window_cross_cov(h.h, None, cp, kp), "dekf_get_window_cross_cov"),
+                 "PC": lambda: h.check(h.L.dekf_get_window_cross_cov(h.h, pp, cp, kp), "dekf_get_window_cross_cov")}
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        times = {k: [] for k in calls}
+        for f in calls.values():
+            for _ in range(3):
+                f()
+        torch.cuda.synchronize()
+        for _ in range(a.rounds):
+            for k, f in calls.items():
+                e0.record()
+                for _ in range(a.calls):
+                    f()
+                e1.record()
+                torch.cuda.synchronize()
+                times[k].append(e0.elapsed_time(e1) / a.calls)
+        Kv = int(K.item())
+        if kw.get("v_box_enable"):
+            by, fl = box_algorithmic(Kv, False, True, False, 4)
+            fl_c = (Kv - 1) * FLOPS_CROSS["box_cross"]
+        elif kw.get("leg_odom_type") == 1:
+            by, fl = foot_algorithmic(4, Kv, False, True)
+            fl_c = (Kv - 1) * foot_stage_flops(4)["cross"]
+        else:
+            cnt = torch.empty(n, dtype=torch.int32, device="cuda")
+            h.check(h.L.dekf_get_window_vo_count(h.h, C.c_void_p(cnt.data_ptr())), "dekf_get_window_vo_count")
+            n_vo = float(cnt.double().mean())
+            full, esize = kw["window_solve"] == 0, 8 if prec == "fp64" else 4
+            by = cov_algorithmic_bytes(N, Kv, esize, full)
+            f64, fh = cov_algorithmic_flops(Kv, n_vo, full)
+            fl = f64 + fh
+            fl_c = (Kv - 1) * FLOPS_CROSS["window_cross"]
+        r = dict(setup=name, robot=robot, n=n, precision=prec, ds=ds, K=Kv)
+        for k in calls:
+            b = by + (8 * (Kv - 1) * ds * ds if k != "P" else 0)
+            f = fl + (fl_c if k != "P" else 0)
+            ms = sorted(times[k])[len(times[k]) // 2]
+            t_bw = b * n / (peaks["copy_gbs"] * 1e9) * 1e3
+            t_fl = f * n / (peaks["fp64_tflops"] * 1e12) * 1e3
+            r[k] = dict(ms_per_call=ms, ms_all_rounds=times[k], bytes_per_instance=b, flops_per_instance=f, hbm_bound_ms=t_bw,
+                        flop_bound_ms=t_fl, bound="hbm" if t_bw >= t_fl else "fma", roof_fraction=max(t_bw, t_fl) / ms)
+        r["PC_over_P"] = r["PC"]["ms_per_call"] / r["P"]["ms_per_call"]
+        r["C_over_P"] = r["C"]["ms_per_call"] / r["P"]["ms_per_call"]
+        print(json.dumps({k: (v if not isinstance(v, dict) else v["ms_per_call"]) for k, v in r.items()}), flush=True)
+        res["runs"].append(r)
+        est.close()
+        del est, P, Cc, d
+        torch.cuda.empty_cache()
+    res["card_after"] = card()
+    return res
+
+
 def card():
     try:
         q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
@@ -265,6 +358,8 @@ def main():
     ap.add_argument("--foot", action="store_true", help="foot-state handles (dekf_get_foot_window) instead of the 9-state getters")
     ap.add_argument("--foot-n", type=int, nargs="+", default=[16384, 65536])
     ap.add_argument("--box", action="store_true", help="state-constrained handles (dekf_get_constrained_window)")
+    ap.add_argument("--cross", action="store_true", help="dekf_get_window_cross_cov against each kind's covariance getter")
+    ap.add_argument("--rounds", type=int, default=5)
     a = ap.parse_args()
     import torch
     from decentralized_ekf_mhe_b200 import build, estimator, synth
@@ -272,8 +367,8 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("window_probe needs a CUDA device")
     peaks = estimator.measure_peaks(0)
-    if a.foot or a.box:
-        res = (box_main if a.box else foot_main)(a, torch, estimator, synth, peaks)
+    if a.foot or a.box or a.cross:
+        res = (cross_main if a.cross else box_main if a.box else foot_main)(a, torch, estimator, synth, peaks)
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
         with open(a.out, "w") as f:
             json.dump(res, f, indent=1)
